@@ -2,6 +2,7 @@
 """bench.py -- keras_nerf hot path on B200: train rays/s (coarse+fine), one JSON line.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--precision auto|fp32|bf16] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one NeRF.train_step (BASELINE.json config[3]: 32,768 rays per GPU from 400x400 synthetic views,
 64 coarse + 128 fine samples, coarse+fine forward, backward, Adam) -- weak scaling: every rank trains on its
@@ -13,6 +14,11 @@ HOST buffers (H2D of images+rays and D2H of the metrics inside the timed region)
 offline, so this is the CPU oracle (torch-CPU restatement, `oracle/`) on all host cores.  It runs ONE step of the
 same 32,768-ray workload (BASELINE config[0]'s size: one coarse+fine train step, then one 128x128 render), once --
 about a minute of CPU work -- whatever --steps / --warmup say; the line reports steps = 1, warmup = 0.
+
+--dump-outputs DIR writes what the timed device steps hand their caller, as float32 DIR/<name>.npy (4.8 MB): the
+coarse and fine weights after the last step's Adam update and the two loss accumulators (coarse, fine; summed over the
+timed steps).  Inputs, initial weights and sample draws are seeded, so two builds run with the same arguments can be
+compared array for array.
 """
 import argparse
 import json
@@ -187,7 +193,13 @@ def main():
     ap.add_argument("--ray-chunks", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-render", action="store_true", help="skip the secondary 800x800 render metric")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the weights and loss accumulators after the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 arm")
     # stdout carries exactly ONE JSON line: libraries that print there (NCCL's version banner at communicator
     # creation) are sent to stderr until the line is written
     real_stdout = os.dup(1)
@@ -267,6 +279,11 @@ def main():
     sync()
     launches = int(lib.knerf_launch_count() - l0)
     ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, x in (("coarse_params", model.coarse.params), ("fine_params", model.fine.params),
+                        ("losses", model._losses)):
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), x.detach().float().cpu().numpy())
     loss_dev = [v / args.steps for v in model._losses.tolist()]
     model._losses.zero_()
 
