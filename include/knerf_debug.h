@@ -26,6 +26,10 @@ int knerf_selftest_umma2(const void* a_blob, const void* b_blob, int N, int K, f
  * library was built with -DKNERF_TC_TIMING (release builds carry no instrumentation). */
 int knerf_debug_tc_timing(unsigned long long* host_out, int n);
 
+/* The same for the BF16 weight-gradient kernel (12 uint64 per CTA; slots documented in csrc/mlp_tc_bwd.cu kWProf):
+ * wait cycles of its producer, issuers and flush warps, items and tiles per CTA, %globaltimer at CTA start and end. */
+int knerf_debug_wgrad_timing(unsigned long long* host_out, int n);
+
 #ifdef __cplusplus
 }
 #endif

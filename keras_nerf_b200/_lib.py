@@ -77,6 +77,7 @@ SIGNATURES = {
     "knerf_train_chunk_dp": (_I, [_CFG, _P, _P, _P, _P, _P, _P, _P, _P, _L, _P, _U64, _I, _I, _I, _F,
                                   _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _I]),
     "knerf_debug_tc_timing": (_I, [_P, _I]),
+    "knerf_debug_wgrad_timing": (_I, [_P, _I]),
     "knerf_selftest_umma": (_I, [_I, _P, _P, _I, _I, _P, _P]),
     "knerf_selftest_umma2": (_I, [_P, _P, _I, _I, _P, _P]),
 }

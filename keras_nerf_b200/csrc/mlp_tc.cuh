@@ -19,5 +19,6 @@ int tc_backward(const Model& m, const float* params, const void* packed, const f
                 float* grads, char* ws, int64_t ws_bytes, int parts, bool rec8, cudaStream_t st);
 
 int tc_debug_timing(unsigned long long* host_out, int n);
+int tc_debug_wgrad_timing(unsigned long long* host_out, int n);
 
 }  // namespace knerf

@@ -8,13 +8,15 @@
 //     No gradient flows into the xyz / direction encodings (mlp.py inputs are constants: nerf.py:361-369).
 //  2. tc_wgrad_kernel -- dW_l = X_l^T dZ_l with the reduction over SAMPLES: the saved activation / gradient
 //     blobs are consumed as MN-major UMMA operands (same bytes, other axis; see tc_ptx.cuh), fp32 partial
-//     sums stay in TMEM across all tiles of a work item and are flushed once with red.global.add.f32; idle warps
+//     sums stay in TMEM across all tiles of a work item and are flushed once with red.global.add.v4.f32; idle warps
 //     take the bias gradients (column sums of the dZ units in shared memory).
 //  3. tc_finish_kernel -- every gradient that contains d(rgb_features) = d(rgb_pre) Wc^T (rank 3): features,
 //     rgb_features and rgb kernels / biases from Y = h7^T d(rgb_pre), Yd = PE(dir)^T d(rgb_pre), sum d(rgb_pre).
 #include "mlp_tc.cuh"
 
+#include <algorithm>
 #include <cstdlib>
+#include <vector>
 #include "tc_roles2.cuh"
 
 namespace knerf {
@@ -278,23 +280,18 @@ constexpr int kWUnitBytes = 32768;     // 16 chunks x 128 samples x 16 B: 128 fe
 constexpr int kWSlots = 7;            // 7 x 32 KB in flight per CTA (224 KB of the 227 KB)
 constexpr int kWThreads = 224;         // warp 0 producer, warps 1 and 6 MMA issuers, warps 2-5 flush
 constexpr int kNumTasks = 10;
-// Item share of the heads task (a `big` task is 128).  It moves only 76 KB per tile but issues 24 N = 16 MMAs, each of
-// which holds its issuing thread as long as a wide one: measured 2.08 / 1.76 / 1.65 / 1.65 / 1.63 ns per sample for
-// the whole kernel at 50 / 80 / 110 / 140 / 178; 178 gives 217 + 36 + 43 = 296 items = exactly two per CTA.
+// Per-tile cost of the heads task (a `big` task is 128).  It moves only 76 KB per tile but issues 24 N = 16 MMAs, each
+// of which holds its issuing thread as long as a wide one (measured with a static item schedule: 2.08 / 1.76 / 1.65 /
+// 1.65 / 1.63 ns per sample for the whole kernel at 50 / 80 / 110 / 140 / 178).
 constexpr int kHeadsCost = 178;
-// fp8 records (build_task_table8): 64 KB and 16 MMAs per tile for a `big` task (cost 128), 40 KB / 8 MMAs for the two
-// encoding tasks, 38 KB / 12 narrow MMAs for the heads; 66 slabs -> 462 + 2 x 41 + 48 = 592 items = four per CTA
-// (swept on the GPU, profiles/r02_fp8_records.md: the item count must be a multiple of the 148 CTAs -- a partly filled
-// extra round costs 4-35 % -- and four per CTA beat two by 1.5-2 %)
-#ifndef KNERF_WG8_X   // (scratch builds for the balance measurements pass the three numbers as macros)
-#define KNERF_WG8_X 80
-#define KNERF_WG8_H 94
-#define KNERF_WG8_S 66
-#endif
-constexpr int kXpartCost8 = KNERF_WG8_X;
-constexpr int kHeadsCost8 = KNERF_WG8_H;
-constexpr int kSlabs8 = KNERF_WG8_S;
+// fp8 records (build_task_table8): 64 KB per tile for a `big` task (cost 128), 40 KB / 8 MMAs for the two encoding
+// tasks, 38 KB / 12 narrow MMAs for the heads (swept on the GPU with 16 N = 128 MMAs per `big` tile,
+// profiles/r02_fp8_records.md; those tiles now take 8 N = 256 MMAs)
+constexpr int kXpartCost8 = 80;
+constexpr int kHeadsCost8 = 94;
 constexpr int kWMaxUnits = 6;
+constexpr int kWQueue = 2;            // item ids in flight between the producer and the other roles
+constexpr int kWBlocks = 4;           // TMEM accumulator blocks of 128 columns: flushed and handed back one at a time
 
 // one ring slot: `bytes` from the forward (src 0) or dz (src 1) record at offset 0 and, optionally, `bytes2` from the
 // dz record at slot offset 8192 (two small operands share a slot); bias_layer >= 0: column sums of this dZ unit
@@ -302,14 +299,21 @@ constexpr int kWMaxUnits = 6;
 struct WUnit { int src, off, bytes, bias_layer, bias_col0, off2, bytes2; };
 // accumulator group: A = unit a (+ a_sub bytes), B = unit b (+ b_sub bytes)
 struct WGroup { int a, b, col, N, layer, row_base, row_limit, col_base, mode, free_a, free_b, a_sub, b_sub, issuer; };
-// last_grp[x][k]: the last group of issuer x that reads unit k (the one after which x releases the slot), -1 = none
-struct WTask { int n_units; WUnit u[kWMaxUnits]; int n_groups; WGroup g[kWMaxUnits]; int cost; int8_t last_grp[2][kWMaxUnits]; };
+// last_grp[x][k]: the last group of issuer x that reads unit k (the one after which x releases the slot), -1 = none;
+// last_in_blk[x][b]: the last group of issuer x in TMEM block b (its last tile's MMAs end the block's accumulation);
+// a group covers the blocks blk_first(g) .. blk_last(g)
+struct WTask {
+  int n_units; WUnit u[kWMaxUnits]; int n_groups; WGroup g[kWMaxUnits]; int cost;
+  int8_t last_grp[2][kWMaxUnits]; int8_t last_in_blk[2][kWBlocks];
+};
 // mode 0: dW[layer][(row_base+row), col_base+col]
 //      1: A = h7, B = the packed d_pre operand: column 3 = the sigma kernel's gradient, columns 0..2 = Y = h7^T d(rgb_pre)
 //         into the fp32 scratch
 //      4: A = PE(dir): columns 0..2 = Yd = PE(dir)^T d(rgb_pre) into the scratch     (tc_finish_kernel uses Y, Yd)
 
 struct WTaskTable { WTask t[kNumTasks]; };
+__host__ __device__ inline int blk_first(const WGroup& g) { return g.col >> 7; }
+__host__ __device__ inline int blk_last(const WGroup& g) { return (g.col + (g.N < 32 ? 32 : g.N) - 1) >> 7; }
 
 // Fit the task table of the chain's fixed program to the model embedded in it (api.cu tc_chain_map).  Identity layers
 // (w_off < 0) keep their tasks, so that the item layout does not depend on the model, but flush nothing: row_limit 0,
@@ -335,6 +339,30 @@ static void fit_tasks_to_model(WTaskTable& T, const TcParams& P) {
     }
     for (int u = 0; u < t.n_units; ++u)
       if (t.u[u].bias_layer >= 0 && P.b_off[t.u[u].bias_layer] < 0) t.u[u].bias_layer = -1;
+  }
+}
+
+// Two MMA-issuing threads (tcgen05.mma holds its issuer for ~160 cycles per N = 128 MMA whose pipe time is 64):
+// every accumulator group belongs to ONE issuer, so the fp32 accumulation order of each gradient element -- and
+// with it every bit -- is that of a single issuer.  Default split: groups alternate (the heads task, the last one,
+// sets its own).
+static void finish_task_table(WTaskTable& T, int n) {
+  for (int k = 0; k < n; ++k) {
+    WTask& t = T.t[k];
+    if (k != n - 1)
+      for (int gi = 0; gi < t.n_groups; ++gi) t.g[gi].issuer = gi & 1;
+    for (int x = 0; x < 2; ++x) {
+      for (int u = 0; u < kWMaxUnits; ++u) {
+        t.last_grp[x][u] = -1;
+        for (int gi = 0; gi < t.n_groups; ++gi)
+          if (t.g[gi].issuer == x && (t.g[gi].a == u || t.g[gi].b == u)) t.last_grp[x][u] = (int8_t)gi;
+      }
+      for (int b = 0; b < kWBlocks; ++b) {
+        t.last_in_blk[x][b] = -1;
+        for (int gi = 0; gi < t.n_groups; ++gi)
+          if (t.g[gi].issuer == x && blk_first(t.g[gi]) <= b && b <= blk_last(t.g[gi])) t.last_in_blk[x][b] = (int8_t)gi;
+      }
+    }
   }
 }
 
@@ -392,25 +420,12 @@ static WTaskTable build_task_table(int dx, int dd) {
     t.g[0].issuer = 0; t.g[1].issuer = 1; t.g[2].issuer = 0;
     t.cost = kHeadsCost;
   }
-  // Two MMA-issuing threads (tcgen05.mma holds its issuer for ~160 cycles per N = 128 MMA whose pipe time is 64):
-  // every accumulator group belongs to ONE issuer, so the fp32 accumulation order of each gradient element -- and
-  // with it every bit -- is that of a single issuer.  Default split: groups alternate.
-  for (int k = 0; k < n; ++k) {
-    WTask& t = T.t[k];
-    if (k != n - 1)
-      for (int gi = 0; gi < t.n_groups; ++gi) t.g[gi].issuer = gi & 1;
-    for (int x = 0; x < 2; ++x)
-      for (int u = 0; u < kWMaxUnits; ++u) {
-        t.last_grp[x][u] = -1;
-        for (int gi = 0; gi < t.n_groups; ++gi)
-          if (t.g[gi].issuer == x && (t.g[gi].a == u || t.g[gi].b == u)) t.last_grp[x][u] = (int8_t)gi;
-      }
-  }
+  finish_task_table(T, n);
   return T;
 }
 
-// fp8 records: a unit is a WHOLE 32 KB record (256 features x 128 samples); the 128 x 128 accumulator groups address
-// its halves through a_sub / b_sub.  64 KB per tile and `big` task instead of 128.
+// fp8 records: a unit is a WHOLE 32 KB record (256 features x 128 samples); the accumulator groups address its halves
+// through a_sub / b_sub.  64 KB per tile and `big` task instead of 128.
 static WTaskTable build_task_table8(int dx, int dd) {
   WTaskTable T{};
   int n = 0;
@@ -419,11 +434,12 @@ static WTaskTable build_task_table8(int dx, int dd) {
     WTask& t = T.t[n++];
     t.n_units = 2;
     t.u[0] = {0, a_off, kH8Bytes, -1, 0, 0, 0}; t.u[1] = {1, b_off, kH8Bytes, layer, 0, 0, 0};
-    t.n_groups = 4;
-    t.g[0] = {0, 1, 0, 128, layer, row_base, 128, 0, 0, 0, 0, 0, 0};
-    t.g[1] = {0, 1, 128, 128, layer, row_base, 128, 128, 0, 0, 0, 0, kHalf};
-    t.g[2] = {0, 1, 256, 128, layer, row_base + 128, 128, 0, 0, 0, 0, kHalf, 0};
-    t.g[3] = {0, 1, 384, 128, layer, row_base + 128, 128, 128, 0, 0, 0, kHalf, kHalf};
+    // one N = 256 group per 128 input features: B is the whole record (its 16-column chunks are SBO apart, so both
+    // halves of the outputs are one operand), and each issuer issues half as many MMAs as with 128 x 128 groups -- the
+    // kernel is bound by MMA issue (profiles/r03_wgrad.md)
+    t.n_groups = 2;
+    t.g[0] = {0, 1, 0, 256, layer, row_base, 128, 0, 0, 0, 0, 0, 0};
+    t.g[1] = {0, 1, 256, 256, layer, row_base + 128, 128, 0, 0, 0, 0, kHalf, 0};
     t.cost = 128;
   };
   auto xpart = [&](int layer, int b_off, int row_base) {
@@ -451,68 +467,110 @@ static WTaskTable build_task_table8(int dx, int dd) {
     t.g[0].issuer = 0; t.g[1].issuer = 1; t.g[2].issuer = 0;
     t.cost = kHeadsCost8;
   }
-  for (int k = 0; k < n; ++k) {
-    WTask& t = T.t[k];
-    if (k != n - 1)
-      for (int gi = 0; gi < t.n_groups; ++gi) t.g[gi].issuer = gi & 1;
-    for (int x = 0; x < 2; ++x)
-      for (int u = 0; u < kWMaxUnits; ++u) {
-        t.last_grp[x][u] = -1;
-        for (int gi = 0; gi < t.n_groups; ++gi)
-          if (t.g[gi].issuer == x && (t.g[gi].a == u || t.g[gi].b == u)) t.last_grp[x][u] = (int8_t)gi;
-      }
-  }
+  finish_task_table(T, n);
   return T;
 }
 
+// ---- optional in-kernel counters (-DKNERF_TC_TIMING builds; knerf_debug_wgrad_timing reads them out) ----------------
+// per CTA: 0 producer waits for a free slot (cycles) | 1, 2 issuer 0 / 1 waits for a loaded slot | 3, 4 issuer 0 / 1 waits
+// for the previous item's flush | 5 flush warp 2: cycles from acc_done to its acc_free arrive | 6 flush warp 2 waits for
+// acc_done | 7 items | 8 tiles | 9, 10 %globaltimer (ns) at the CTA's start / end | 11 CTA cycles start to end
+#ifdef KNERF_TC_TIMING
+constexpr int kWProf = 12;
+static __device__ unsigned long long g_wg_prof[160][kWProf];
+__device__ __forceinline__ unsigned long long globaltimer_ns() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+#define KN_WG_DECL() unsigned long long kn_wg[kWProf] = {}
+#define KN_WG_WAIT(slot, bar, par) do { const long long kn_t0 = clock64(); mbar_wait(bar, par); \
+                                        kn_wg[slot] += (unsigned long long)(clock64() - kn_t0); } while (0)
+#define KN_WG_ADD(slot, v) kn_wg[slot] += (unsigned long long)(v)
+#define KN_WG_CLOCK(var) const long long var = clock64()
+#define KN_WG_FLUSH() for (int kn_i = 0; kn_i < kWProf; ++kn_i) if (kn_wg[kn_i]) atomicAdd(&g_wg_prof[blockIdx.x][kn_i], kn_wg[kn_i])
+#else
+#define KN_WG_DECL()
+#define KN_WG_WAIT(slot, bar, par) mbar_wait(bar, par)
+#define KN_WG_ADD(slot, v)
+#define KN_WG_CLOCK(var)
+#define KN_WG_FLUSH()
+#endif
+
 struct WSmem {
   uint8_t slot[kWSlots][kWUnitBytes];
-  uint64_t full[kWSlots], empty[kWSlots], acc_done, acc_free;
+  uint64_t full[kWSlots], empty[kWSlots], acc_done[kWBlocks], acc_free[kWBlocks], q_full[kWQueue], q_empty[kWQueue];
+  int q_item[kWQueue];
   uint32_t tmem_base;
 };
 
-struct WItem { int task; int64_t tile_lo, tile_hi; };
+// Work items: (task, tiles [lo, hi)), claimed one at a time from a counter in the fp32 scratch (kXOffQueue) in the
+// order of the list.  Boundaries depend only on n_tiles and the task costs, so every item's partial sums are the same
+// bits from run to run; only the order of the cross-CTA red.global.add flushes varies, as it did with a static schedule.
+constexpr int kWMaxItems = 1024;
+struct WItemList { int2 range[kWMaxItems]; int8_t task[kWMaxItems]; };
 
-__device__ __forceinline__ WItem decode_item(const WTaskTable& T, int item, int slabs_per_cost_x128, int64_t n_tiles) {
-  // item ids are laid out task after task; task k owns max(1, cost_k * slabs / 128) slabs
-  WItem it{-1, 0, 0};
-  int base = 0;
+// Guided sizes: an item takes 1/(kWGuide * 148) of the cost still unassigned, but no less than 1/kWMinShare of a CTA's
+// share and no less than kWMinTiles `big` tiles (each item ends with a flush of up to 256 KB of partial sums), so items
+// shrink towards the end of the list and the CTAs finish within about one small item of each other.  Items never span
+// two tasks; the list is sorted longest first.
+constexpr int kWGuide = 2;
+constexpr int kWMinShare = 16;
+constexpr int kWMinTiles = 4;
+static int build_items(const WTaskTable& T, int64_t n_tiles, WItemList& L) {
+  double total = 0.0;
+  for (int k = 0; k < kNumTasks; ++k) total += (double)T.t[k].cost * (double)n_tiles;
+  const double min_cost = std::max(total / kNumSMs / kWMinShare, 128.0 * kWMinTiles);
+  struct It { double cost; int task; int64_t lo, hi; };
+  std::vector<It> v;
+  double left = total;
   for (int k = 0; k < kNumTasks; ++k) {
-    const int ns = max(1, T.t[k].cost * slabs_per_cost_x128 / 128);
-    if (item < base + ns) {
-      const int s = item - base;
-      it.task = k;
-      it.tile_lo = n_tiles * s / ns;
-      it.tile_hi = n_tiles * (s + 1) / ns;
-      return it;
+    const double c = T.t[k].cost;
+    for (int64_t lo = 0; lo < n_tiles;) {
+      const double want = std::max(min_cost, left / (kWGuide * kNumSMs));
+      int64_t n = std::max<int64_t>(1, (int64_t)(want / c + 0.5));
+      if (n_tiles - lo - n < (n + 1) / 2) n = n_tiles - lo;   // no runt at the end of a task
+      v.push_back({c * (double)n, k, lo, lo + n});
+      left -= c * (double)n;
+      lo += n;
     }
-    base += ns;
   }
-  return it;
+  std::stable_sort(v.begin(), v.end(), [](const It& a, const It& b) { return a.cost > b.cost; });
+  if ((int64_t)v.size() > kWMaxItems) return -1;
+  for (size_t i = 0; i < v.size(); ++i) {
+    L.range[i] = make_int2((int)v[i].lo, (int)v[i].hi);
+    L.task[i] = (int8_t)v[i].task;
+  }
+  return (int)v.size();
 }
 
-static int count_items(const WTaskTable& T, int slabs_per_cost_x128) {
-  int n = 0;
-  for (int k = 0; k < kNumTasks; ++k) n += std::max(1, T.t[k].cost * slabs_per_cost_x128 / 128);
-  return n;
-}
-
+// Roles: warp 0 lane 0 claims items and loads their operand units into the ring; warps 1 and 6 (lane 0) issue the MMAs
+// of their accumulator groups; warps 2-5 take the bias gradients while an item runs and flush its accumulators after it.
+// The item ids reach the other roles through a kWQueue-deep shared-memory queue (the producer runs ahead into the next
+// item while the current one is being computed).  TMEM block b (128 columns) of the next item is written only after the
+// flush warps have drained block b of the previous one (acc_free[b]); they drain block 0 first.
 template <bool REC8>
 __global__ void __launch_bounds__(kWThreads, 1)
-tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz, int64_t n_tiles,
-                float* __restrict__ grads, float* __restrict__ xbuf, TcParams P, const __grid_constant__ WTaskTable T,
-                int n_items, int slabs) {
+tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz, float* __restrict__ grads,
+                float* __restrict__ xbuf, TcParams P, const __grid_constant__ WTaskTable T,
+                const __grid_constant__ WItemList L, int n_items) {
   constexpr int kRB = REC8 ? kRec8Bytes : kRecBytes, kDB = REC8 ? kDz8Bytes : kDzBytes;
   constexpr int kSub2 = REC8 ? 4096 : 8192;   // slot offset of a unit's second part (the packed d_pre operand)
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   WSmem& sm = *reinterpret_cast<WSmem*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  KN_WG_DECL();
+  KN_WG_CLOCK(kn_start);
+#ifdef KNERF_TC_TIMING
+  if (tid == 0) g_wg_prof[blockIdx.x][9] = globaltimer_ns();
+#endif
   if (tid == 0) {
     // a slot is free again when the MMAs that read it have completed AND the flush warps are done with it
     // (one release per issuer + one from the flush warps)
     for (int i = 0; i < kWSlots; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.empty[i], 3); }
-    mbar_init(&sm.acc_done, 2);
-    mbar_init(&sm.acc_free, 128);
+    for (int b = 0; b < kWBlocks; ++b) { mbar_init(&sm.acc_done[b], 2); mbar_init(&sm.acc_free[b], 128); }
+    // a queue entry is read by the two issuers and the four flush warps
+    for (int i = 0; i < kWQueue; ++i) { mbar_init(&sm.q_full[i], 1); mbar_init(&sm.q_empty[i], 6); }
     fence_mbar_init();
   }
   if (warp == 1) tmem_alloc<512>(&sm.tmem_base);
@@ -520,18 +578,29 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = sm.tmem_base;
+  // the j-th item of this CTA (-1: none left)
+  auto take_item = [&](int j) -> int {
+    mbar_wait(&sm.q_full[j % kWQueue], (j / kWQueue) & 1);
+    return *reinterpret_cast<volatile int*>(&sm.q_item[j % kWQueue]);
+  };
 
   if (warp == 0) {
     if (lane == 0) {
+      unsigned int* counter = reinterpret_cast<unsigned int*>(xbuf + kXOffQueue);
       uint32_t it = 0;
-      for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-        const WItem w = decode_item(T, item, slabs, n_tiles);
-        const WTask& t = T.t[w.task];
-        for (int64_t tile = w.tile_lo; tile < w.tile_hi; ++tile) {
+      for (int j = 0;; ++j) {
+        const int claimed = (int)atomicAdd(counter, 1u);
+        const int item = claimed < n_items ? claimed : -1;
+        mbar_wait(&sm.q_empty[j % kWQueue], ((j / kWQueue) & 1) ^ 1);
+        sm.q_item[j % kWQueue] = item;
+        mbar_arrive(&sm.q_full[j % kWQueue]);
+        if (item < 0) break;
+        const WTask& t = T.t[L.task[item]];
+        for (int64_t tile = L.range[item].x; tile < L.range[item].y; ++tile) {
           for (int k = 0; k < t.n_units; ++k, ++it) {
             const uint32_t slot = it % kWSlots, ph = (it / kWSlots) & 1;
             const uint8_t* src = (t.u[k].src == 0 ? rec + tile * kRB : dz + tile * kDB) + t.u[k].off;
-            mbar_wait(&sm.empty[slot], ph ^ 1);
+            KN_WG_WAIT(0, &sm.empty[slot], ph ^ 1);
             mbar_arrive_expect_tx(&sm.full[slot], t.u[k].bytes + t.u[k].bytes2);
             tma_load_1d(sm.slot[slot], src, t.u[k].bytes, &sm.full[slot]);
             if (t.u[k].bytes2)
@@ -543,26 +612,35 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
   } else if (warp == 1 || warp == 6) {
     if (lane == 0) {
       const int me = (warp == 1) ? 0 : 1;
-      uint32_t it = 0, free_par = 0;
-      bool first_item = true;
-      for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-        const WItem w = decode_item(T, item, slabs, n_tiles);
-        const WTask& t = T.t[w.task];
-        if (w.tile_lo >= w.tile_hi) continue;
-        if (!first_item) {   // the previous item's accumulators must have been flushed
-          mbar_wait(&sm.acc_free, free_par);
-          free_par ^= 1;
-          tc_fence_after();
-        }
-        first_item = false;
-        for (int64_t tile = w.tile_lo; tile < w.tile_hi; ++tile, it += t.n_units) {
+      uint32_t it = 0;
+      for (int j = 0;; ++j) {
+        const int item = take_item(j);
+        mbar_arrive(&sm.q_empty[j % kWQueue]);
+        if (item < 0) break;
+        const WTask& t = T.t[L.task[item]];
+        const int64_t lo = L.range[item].x, hi = L.range[item].y;
+        // Block b of this item may be written once the flush warps have drained it for the previous item.  Every item
+        // waits for all blocks (those it does not write at its end, before its acc_done arrival), so that neither
+        // barrier of a block can get a phase ahead of its reader.
+        uint32_t freed = (j == 0) ? 0xFu : 0u, done = 0u;
+        auto wait_free = [&](int b) {
+          if (!((freed >> b) & 1u)) {
+            KN_WG_WAIT(3 + me, &sm.acc_free[b], (j - 1) & 1);
+            tc_fence_after();
+            freed |= 1u << b;
+          }
+        };
+        for (int64_t tile = lo; tile < hi; ++tile, it += t.n_units) {
           for (int gi = 0; gi < t.n_groups; ++gi) {
             const WGroup& g = t.g[gi];
             if (g.issuer != me) continue;
+            const int b0 = blk_first(g), b1 = blk_last(g);
+            if (tile == lo)
+              for (int b = b0; b <= b1; ++b) wait_free(b);
             const uint32_t ia = it + g.a, ib = it + g.b;
             const uint32_t sa = ia % kWSlots, sb = ib % kWSlots;
-            mbar_wait(&sm.full[sa], (ia / kWSlots) & 1);
-            mbar_wait(&sm.full[sb], (ib / kWSlots) & 1);
+            KN_WG_WAIT(1 + me, &sm.full[sa], (ia / kWSlots) & 1);
+            KN_WG_WAIT(1 + me, &sm.full[sb], (ib / kWSlots) & 1);
             tc_fence_after();
             const uint32_t a_base = smem_u32(sm.slot[sa]) + g.a_sub, b_base = smem_u32(sm.slot[sb]) + g.b_sub;
             if (REC8) {   // e4m3 activations x e5m2 gradients, 32 samples per MMA (512 B further along every chunk)
@@ -571,7 +649,7 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
               for (int k = 0; k < 4; ++k) {
                 const uint64_t da = umma_smem_desc(a_base + k * 512, 128, kChunkA);
                 const uint64_t db = umma_smem_desc(b_base + k * 512, 128, kChunkA);
-                umma_f8(tmem + g.col, da, db, idesc, (tile > w.tile_lo || k > 0) ? 1u : 0u);
+                umma_f8(tmem + g.col, da, db, idesc, (tile > lo || k > 0) ? 1u : 0u);
               }
             } else {
               const uint32_t idesc = umma_idesc_bf16(128, g.N, 1, 1);
@@ -579,11 +657,18 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
               for (int k = 0; k < 8; ++k) {   // K = 128 samples per tile, 16 per MMA; MN-major: LBO = 128 B, SBO = 2 KB
                 const uint64_t da = umma_smem_desc(a_base + k * 256, 128, kChunkA);
                 const uint64_t db = umma_smem_desc(b_base + k * 256, 128, kChunkA);
-                umma_bf16(tmem + g.col, da, db, idesc, (tile > w.tile_lo || k > 0) ? 1u : 0u);
+                umma_bf16(tmem + g.col, da, db, idesc, (tile > lo || k > 0) ? 1u : 0u);
               }
             }
             if (t.last_grp[me][g.a] == gi) umma_commit(&sm.empty[sa]);
             if (g.b != g.a && t.last_grp[me][g.b] == gi) umma_commit(&sm.empty[sb]);
+            if (tile + 1 == hi) {
+              for (int b = b0; b <= b1; ++b) {
+                if (t.last_in_blk[me][b] != gi) continue;   // this issuer's part of block b is complete
+                umma_commit(&sm.acc_done[b]);
+                done |= 1u << b;
+              }
+            }
           }
           // units this issuer never reads: release them too (after their load has landed, so that the arrival
           // counts for this use of the slot and not for the previous one)
@@ -594,7 +679,11 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
             mbar_arrive(&sm.empty[iu % kWSlots]);
           }
         }
-        umma_commit(&sm.acc_done);
+        for (int b = 0; b < kWBlocks; ++b) {
+          if ((done >> b) & 1u) continue;
+          wait_free(b);
+          umma_commit(&sm.acc_done[b]);
+        }
       }
     }
   } else {
@@ -602,23 +691,27 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
     const int q = warp & 3, row = q * 32 + lane;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     const int ftid = tid - 64, fc = ftid >> 3, fsub = ftid & 7;
-    uint32_t done_par = 0, uit = 0;
-    for (int item = blockIdx.x; item < n_items; item += gridDim.x) {
-      const WItem w = decode_item(T, item, slabs, n_tiles);
-      const WTask& t = T.t[w.task];
-      if (w.tile_lo >= w.tile_hi) continue;
+    const float inv_scale = REC8 ? dz8_scale(__ldg(reinterpret_cast<const uint32_t*>(xbuf) + kXOffAmax), true) : 1.f;
+    uint32_t uit = 0;
+    for (int j = 0;; ++j) {
+      const int item = take_item(j);
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&sm.q_empty[j % kWQueue]);
+      if (item < 0) break;
+      const int task = L.task[item];
+      const WTask& t = T.t[task];
+      const int64_t lo = L.range[item].x, hi = L.range[item].y;
       // While the tensor core works through the item, these warps take the bias gradients: column sums (over
       // samples) of every dZ unit passing through shared memory.  Thread (fc, fsub) owns 8 columns of chunk fc
       // and every 8th sample; partial sums stay in registers for the whole item.
       // (fp8 records: a task has ONE dZ unit of 16 chunks x 16 columns; bacc[0] / bacc[1] = columns 0..7 / 8..15 of chunk fc)
-      const float inv_scale = REC8 ? dz8_scale(__ldg(reinterpret_cast<const uint32_t*>(xbuf) + kXOffAmax), true) : 1.f;
       float bacc[2][8];
 #pragma unroll
       for (int u = 0; u < 2; ++u)
 #pragma unroll
         for (int e = 0; e < 8; ++e) bacc[u][e] = 0.f;
       float pacc[3] = {0.f, 0.f, 0.f};          // this thread's row of the packed d_pre operand, summed over the tiles
-      for (int64_t tile = w.tile_lo; tile < w.tile_hi; ++tile) {
+      for (int64_t tile = lo; tile < hi; ++tile) {
         int nb = 0;
         for (int k = 0; k < t.n_units; ++k, ++uit) {
           const uint32_t slot = uit % kWSlots;
@@ -631,10 +724,10 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
                 const uint4 v = *reinterpret_cast<const uint4*>(base + i * 128);
                 const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                  const float2 lo = e5m2x2_lo(wv[j]), hi = e5m2x2_hi(wv[j]);
-                  float* a = bacc[j >> 1] + (j & 1) * 4;
-                  a[0] += lo.x; a[1] += lo.y; a[2] += hi.x; a[3] += hi.y;
+                for (int jj = 0; jj < 4; ++jj) {
+                  const float2 lo2 = e5m2x2_lo(wv[jj]), hi2 = e5m2x2_hi(wv[jj]);
+                  float* a = bacc[jj >> 1] + (jj & 1) * 4;
+                  a[0] += lo2.x; a[1] += lo2.y; a[2] += hi2.x; a[3] += hi2.y;
                 }
               }
             } else {
@@ -681,51 +774,69 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
           ++nb;
         }
       }
-      if (!REC8 && w.task == kNumTasks - 1) {   // heads task: sum d(rgb_pre) of this call for tc_finish_kernel
+      if (!REC8 && task == kNumTasks - 1) {   // heads task: sum d(rgb_pre) of this call for tc_finish_kernel
 #pragma unroll
         for (int e = 0; e < 3; ++e) {
           const float sres = warp_sum(pacc[e]);
           if (lane == 0) atomicAdd(xbuf + kXOffS + e, sres);
         }
       }
-      mbar_wait(&sm.acc_done, done_par);
-      done_par ^= 1;
-      tc_fence_after();
-      for (int gi = 0; gi < t.n_groups; ++gi) {
-        const WGroup& g = t.g[gi];
-        const int ncol = g.N < 32 ? 32 : g.N;
-        for (int c0 = 0; c0 < ncol; c0 += 32) {
-          float v[32];
-          tmem_ld32(tmem + lane_base + g.col + c0, v);   // warp-collective: outside the row guard
-          if (REC8) {
+      KN_WG_ADD(7, 1);
+      KN_WG_ADD(8, hi - lo);
+      for (int b = 0; b < kWBlocks; ++b) {
+        KN_WG_WAIT(6, &sm.acc_done[b], j & 1);
+        KN_WG_CLOCK(kn_flush);
+        tc_fence_after();
+        for (int gi = 0; gi < t.n_groups; ++gi) {
+          const WGroup& g = t.g[gi];
+          const int ncol = g.N < 32 ? 32 : g.N;
+          for (int c0 = 0; c0 < ncol; c0 += 32) {
+            if (((g.col + c0) >> 7) != b) continue;
+            float v[32];
+            tmem_ld32(tmem + lane_base + g.col + c0, v);   // warp-collective: outside the row guard
+            if (REC8) {
 #pragma unroll
-            for (int i = 0; i < 32; ++i) v[i] *= inv_scale;
-          }
-          if (row < g.row_limit) {
-            if (g.mode == 0) {   // kernel [fan_in, U] of a hidden layer: columns >= U belong to the padding
-              float* dst = grads + P.w_off[g.layer] + (int64_t)(g.row_base + row) * P.U + g.col_base + c0;
-              const int nv = P.U - (g.col_base + c0);
+              for (int i = 0; i < 32; ++i) v[i] *= inv_scale;
+            }
+            if (row < g.row_limit) {
+              if (g.mode == 0) {   // kernel [fan_in, U] of a hidden layer: columns >= U belong to the padding
+                float* dst = grads + P.w_off[g.layer] + (int64_t)(g.row_base + row) * P.U + g.col_base + c0;
+                const int nv = P.U - (g.col_base + c0);
+                if (nv >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
 #pragma unroll
-              for (int i = 0; i < 32; ++i)
-                if (i < nv) atomicAdd(dst + i, v[i]);
-            } else if (g.mode == 1) {
-              atomicAdd(grads + P.w_off[8] + g.row_base + row, v[3]);
-              float* dst = xbuf + kXOffY + (g.row_base + row) * 4;
-              atomicAdd(dst, v[0]); atomicAdd(dst + 1, v[1]); atomicAdd(dst + 2, v[2]);
-            } else {
-              float* dst = xbuf + kXOffYd + row * 4;
-              atomicAdd(dst, v[0]); atomicAdd(dst + 1, v[1]); atomicAdd(dst + 2, v[2]);
+                  for (int i = 0; i < 32; i += 4) red_add_v4(dst + i, v[i], v[i + 1], v[i + 2], v[i + 3]);
+                } else {   // a narrower model's last columns, or a row that does not start 16-byte aligned
+#pragma unroll
+                  for (int i = 0; i < 32; ++i)
+                    if (i < nv) atomicAdd(dst + i, v[i]);
+                }
+              } else if (g.mode == 1) {
+                atomicAdd(grads + P.w_off[8] + g.row_base + row, v[3]);
+                float* dst = xbuf + kXOffY + (g.row_base + row) * 4;
+                atomicAdd(dst, v[0]); atomicAdd(dst + 1, v[1]); atomicAdd(dst + 2, v[2]);
+              } else {
+                float* dst = xbuf + kXOffYd + row * 4;
+                atomicAdd(dst, v[0]); atomicAdd(dst + 1, v[1]); atomicAdd(dst + 2, v[2]);
+              }
             }
           }
         }
+        tc_fence_before();
+        mbar_arrive(&sm.acc_free[b]);
+        KN_WG_ADD(5, clock64() - kn_flush);
       }
-      tc_fence_before();
-      mbar_arrive(&sm.acc_free);
     }
   }
   tc_fence_before();
   __syncthreads();
   if (warp == 1) tmem_dealloc<512>(tmem);
+#ifdef KNERF_TC_TIMING
+  if (tid == 0) {
+    KN_WG_ADD(11, clock64() - kn_start);
+    g_wg_prof[blockIdx.x][10] = globaltimer_ns();
+  }
+  if (tid == 0 || tid == 32 || tid == 64 || tid == 192) KN_WG_FLUSH();
+#endif
 }
 
 // =============================================================================================================
@@ -826,6 +937,20 @@ __global__ void __launch_bounds__(256) tc_finish_kernel(const float* __restrict_
 
 }  // namespace
 
+// diagnostic (-DKNERF_TC_TIMING builds only): copy and clear the weight-gradient kernel's per-CTA counters
+int tc_debug_wgrad_timing(unsigned long long* host_out, int n) {
+#ifdef KNERF_TC_TIMING
+  static unsigned long long zeros[160 * kWProf];
+  if (n > 160 * kWProf) n = 160 * kWProf;
+  if (cudaMemcpyFromSymbol(host_out, g_wg_prof, (size_t)n * 8) != cudaSuccess) return -1;
+  if (cudaMemcpyToSymbol(g_wg_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
+  return n;
+#else
+  (void)host_out; (void)n;
+  return 0;
+#endif
+}
+
 // parts: which of the backward kernels to launch (bit 0 dgrad, bit 1 wgrad + finish; KNERF_BWD_*_ONLY)
 int tc_backward(const Model& m, const float* params, const void* packed, const float* d_pre, int64_t R, int S,
                 float* grads, char* ws, int64_t ws_bytes, int parts, bool rec8, cudaStream_t st) {
@@ -872,20 +997,20 @@ int tc_backward(const Model& m, const float* params, const void* packed, const f
     KN_LAUNCH_CHECK();
   }
   if (parts & 2) {
-    // ~3 KB, passed by value as a __grid_constant__
+    // the task table (~3 KB) and the item list (~9 KB) are passed by value as __grid_constant__ parameters
     WTaskTable h_table = rec8 ? build_task_table8(m.dx, m.dd) : build_task_table(m.dx, m.dd);
     fit_tasks_to_model(h_table, P);
-    // items = 2 x 148: 7 tasks of cost 128, 2 of cost 76, 1 of cost 178 -> 217 + 36 + 43 = 296 items for 31 slabs
-    const int slabs = (int)std::max<int64_t>(1, std::min<int64_t>(rec8 ? kSlabs8 : 31, n_tiles / 4));
-    const int n_items = count_items(h_table, slabs);
-    const int grid = std::min(n_items, kNumSMs);
+    KN_CHECK_ARG(n_tiles < (int64_t)1 << 30, "tc_backward: %lld rows are too many for one call", (long long)M);
+    WItemList h_items;
+    const int n_items = build_items(h_table, n_tiles, h_items);
+    if (n_items < 0) return fail(KNERF_ERR_UNSUPPORTED, "tc_backward: more than %d weight-gradient items", kWMaxItems);
     const size_t smem = sizeof(WSmem);
     if (rec8) {
       KN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      tc_wgrad_kernel<true><<<grid, kWThreads, smem, st>>>(rec, dz, n_tiles, grads, xbuf, P, h_table, n_items, slabs);
+      tc_wgrad_kernel<true><<<kNumSMs, kWThreads, smem, st>>>(rec, dz, grads, xbuf, P, h_table, h_items, n_items);
     } else {
       KN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      tc_wgrad_kernel<false><<<grid, kWThreads, smem, st>>>(rec, dz, n_tiles, grads, xbuf, P, h_table, n_items, slabs);
+      tc_wgrad_kernel<false><<<kNumSMs, kWThreads, smem, st>>>(rec, dz, grads, xbuf, P, h_table, h_items, n_items);
     }
     KN_LAUNCH_CHECK();
     tc_finish_prep_kernel<<<6, 256, 0, st>>>(params, P, xbuf);

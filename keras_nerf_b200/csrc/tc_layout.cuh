@@ -163,10 +163,12 @@ constexpr int kDz8P = 8 * kH8Bytes;                // (d rgb_pre[3], d sigma_pre
 constexpr int kDz8Bytes = kDz8P + 2048;            // 258 KB per 128 samples
 constexpr int kDz8Top = 6;                         // max|d_pre| * scale lies in [2^(kDz8Top-1), 2^kDz8Top)
 
-// fp32 scratch at the head of the training workspace (zeroed by every backward call): Y = h7^T d(rgb_pre) [256 x 4],
-// Yd = PE(dir)^T d(rgb_pre) [32 x 4] and sum d(rgb_pre) [4] -- the rank-3 factors of every gradient that contains
-// d(rgb_features) (tc_finish_kernel)
-constexpr int kXOffY = 0;
+// fp32 scratch at the head of the training workspace (zeroed by every backward call): the weight-gradient kernel's
+// work-item counter (a uint32), Y = h7^T d(rgb_pre) [256 x 4], Yd = PE(dir)^T d(rgb_pre) [32 x 4] and sum d(rgb_pre) [4]
+// -- the rank-3 factors of every gradient that contains d(rgb_features) (tc_finish_kernel).  The counter lies below
+// kXOffS: a weight-gradient-only call over fp8 records zeroes only [0, kXOffS).
+constexpr int kXOffQueue = 0;
+constexpr int kXOffY = 4;
 constexpr int kXOffYd = kXOffY + 256 * 4;
 constexpr int kXOffS = kXOffYd + 32 * 4;
 constexpr int kXOffT = kXOffS + 4;           // T[j][c] = sum_n W_g[j][n] W_c[n][c]                      [256 x 4]

@@ -211,6 +211,11 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
                : "memory");
 }
 
+// p[0..3] += (a, b, c, d) in global memory as ONE 16-byte reduction (REDG.E.ADD.F32x4); p must be 16-byte aligned
+__device__ __forceinline__ void red_add_v4(float* p, float a, float b, float c, float d) {
+  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
+}
+
 // ---- small numeric helpers -------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
