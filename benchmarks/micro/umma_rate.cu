@@ -1,5 +1,8 @@
 // Microbenchmark: raw issue/execute rate of tcgen05.mma from shared-memory operands in the library's chunk-major
 // (SWIZZLE_NONE) layout, 1-CTA (M=128) and cta_group::2 (M=256), with and without a tcgen05.commit per K=32 stage.
+// rate_f8_kernel: kind::f8f6f4 (e4m3 x e5m2) at the weight-gradient kernel's shapes -- M 128, K 32, N 256 / 128, both
+// operands MN-major with LBO 128 B / SBO 2 KB exactly as tc_wgrad_kernel builds them (or the same bytes K-major), issued
+// by one thread or by two threads into disjoint accumulators.
 // build: nvcc -O3 -std=c++17 -gencode arch=compute_100a,code=sm_100a -I keras_nerf_b200/csrc -o benchmarks/micro/umma_rate benchmarks/micro/umma_rate.cu
 #include <cstdio>
 #include <cstdlib>
@@ -95,6 +98,83 @@ void run(int grid, int n_stages, int N, int commit_every) {
   cudaFree(d);
 }
 
+// fp8: A = [8 chunks][128 k][16] (16 KB), B = [N/16 chunks][128 k][16] (N = 256: 32 KB) -- one weight-gradient tile of
+// 128 samples, 4 MMAs of K = 32.  K-major: the same 48 KB as [8 k-chunks][rows][16].  LAYOUT: 0 both MN-major, 1 both
+// K-major, 2 A MN-major / B K-major, 3 A K-major / B MN-major.  mode bit 0: tcgen05.commit per
+// 4 MMAs; bit 1: mbarrier.try_wait (on an already completed phase) per 4 MMAs -- the issuer loop of tc_wgrad_kernel.
+template <int LAYOUT>
+__global__ void __launch_bounds__(64) rate_f8_kernel(int n_mma, int N, int issuers, int mode, long long* out) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  __shared__ __align__(8) uint64_t bar_done[2], bar_full, bar_stage[2];
+  __shared__ uint32_t tmem_base_s;
+  const int tid = threadIdx.x, warp = tid >> 5;
+  for (int i = tid; i < 49152 / 4; i += 64) reinterpret_cast<uint32_t*>(smem)[i] = 0x38383838u ^ (i & 0x07070707u);
+  if (tid == 0) {
+    for (int i = 0; i < 2; ++i) { mbar_init(&bar_done[i], 1); mbar_init(&bar_stage[i], 1); }
+    mbar_init(&bar_full, 1);
+    fence_mbar_init();
+  }
+  if (warp == 0) tmem_alloc<512>(&tmem_base_s);
+  fence_async_smem();
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = tmem_base_s;
+  const int me = warp;
+  if ((tid & 31) == 0 && me < issuers) {
+    constexpr bool KA = LAYOUT == 1 || LAYOUT == 3, KB = LAYOUT == 1 || LAYOUT == 2;
+    const uint32_t idesc = umma_idesc_f8(128, N, kE4M3, kE5M2, KA ? 0 : 1, KB ? 0 : 1);
+    const uint32_t a_base = smem_u32(smem), b_base = smem_u32(smem) + 16384;
+    const long long t0 = clock64();
+    for (int s = 0; s < n_mma; s += 4) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        const uint64_t da = KA ? umma_smem_desc(a_base + k * 2 * 2048, 2048, 128) : umma_smem_desc(a_base + k * 512, 128, 2048);
+        const uint64_t db = KB ? umma_smem_desc(b_base + k * 2 * N * 16, N * 16, 128) : umma_smem_desc(b_base + k * 512, 128, 2048);
+        umma_f8(tmem + me * 256, da, db, idesc, (s > 0 || k > 0) ? 1u : 0u);
+      }
+      if (mode & 2) mbar_wait(&bar_full, 1);
+      if (mode & 1) umma_commit(&bar_stage[me]);
+    }
+    const long long t1 = clock64();
+    umma_commit(&bar_done[me]);
+    mbar_wait(&bar_done[me], 0);
+    const long long t2 = clock64();
+    out[(blockIdx.x * 2 + me) * 2] = t1 - t0;
+    out[(blockIdx.x * 2 + me) * 2 + 1] = t2 - t0;
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 0) tmem_dealloc<512>(tmem);
+}
+
+template <int LAYOUT>
+void run_f8(int n_mma, int N, int issuers, int mode) {
+  constexpr int grid = 148;
+  long long* d;
+  cudaMalloc(&d, grid * 4 * sizeof(long long));
+  cudaMemset(d, 0, grid * 4 * sizeof(long long));
+  cudaFuncSetAttribute(rate_f8_kernel<LAYOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 49152);
+  for (int rep = 0; rep < 2; ++rep) {
+    rate_f8_kernel<LAYOUT><<<grid, 64, 49152>>>(n_mma, N, issuers, mode, d);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess || (e = cudaDeviceSynchronize()) != cudaSuccess) { printf("error: %s\n", cudaGetErrorString(e)); exit(1); }
+  }
+  long long h[grid * 4];
+  cudaMemcpy(h, d, sizeof(h), cudaMemcpyDeviceToHost);
+  double issue = 0, total = 0;
+  for (int b = 0; b < grid; ++b) {
+    double t = 0;
+    for (int x = 0; x < issuers; ++x) { issue += h[(b * 2 + x) * 2]; t = h[(b * 2 + x) * 2 + 1] > t ? h[(b * 2 + x) * 2 + 1] : t; }
+    total += t;
+  }
+  // issue: cycles one issuer spends per MMA it issues; complete: SM time per MMA, all issuers' MMAs counted
+  printf("f8 e4m3 x e5m2 %s M=128 N %3d K 32, %d issuer(s), commit %d wait %d: issue %.1f cyc/MMA, complete %.1f cyc/MMA"
+         " (floor %d)\n", LAYOUT == 0 ? "A, B MN-major" : LAYOUT == 1 ? "A, B K-major " : LAYOUT == 2 ? "A MN, B K    " : "A K, B MN    ", N, issuers, mode & 1, (mode >> 1) & 1,
+         issue / grid / issuers / n_mma, total / grid / ((double)issuers * n_mma), N / 2);
+  cudaFree(d);
+}
+
 int main() {
   for (int mode : {0, 1, 2, 4, 3, 7, 8, 14}) {
     run<false>(148, 4096, 256, mode);
@@ -105,5 +185,14 @@ int main() {
   run<false>(148, 4096, 128, 0);
   run<false, true>(148, 4096, 128, 0);
   run<false, true>(148, 4096, 256, 0);
+  // kind::f8f6f4 at the shapes of tc_wgrad_kernel (fp8 records)
+  for (int N : {256, 128})
+    for (int issuers : {1, 2})
+      for (int mode : {0, 3}) {
+        run_f8<0>(8192, N, issuers, mode);
+        run_f8<1>(8192, N, issuers, mode);
+      }
+  run_f8<2>(8192, 256, 1, 0);
+  run_f8<3>(8192, 256, 1, 0);
   return 0;
 }

@@ -7,7 +7,9 @@
 
 Each shape runs forward, dgrad-only, then wgrad-only calls; the counters of the last wgrad-only call are read (the
 others are cleared).  Times are CTA means (kcycles) unless marked; `end min/max` = earliest over latest CTA end time,
-both measured from the earliest CTA start (%globaltimer)."""
+both measured from the earliest CTA start (%globaltimer).  `busy` = cycles inside the MMA / commit sequences, the
+issuer's waits excluded; `releases, last = X` = ring-slot releases whose last arrival came from X (mlp_tc_bwd.cu
+kWProf)."""
 import ctypes as C
 import os
 import sys
@@ -19,7 +21,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
-N_PROF = 12
+N_PROF = 24
 
 
 def run_shape(R, S, records):
@@ -76,6 +78,13 @@ def run_shape(R, S, records):
         "issuer0 wait acc_free": m[3] / 1e3, "issuer1 wait acc_free": m[4] / 1e3,
         "flush wait acc_done": m[6] / 1e3, "flush total": m[5] / 1e3,
         "flush per item": m[5] / max(m[7], 1) / 1e3, "items per CTA": m[7], "tiles per CTA": m[8],
+        "issuer0 busy (MMA + commit)": m[12] / 1e3, "issuer1 busy (MMA + commit)": m[13] / 1e3,
+        "issuer0 cycles per tile": m[12] / max(m[8], 1), "issuer1 cycles per tile": m[13] / max(m[8], 1),
+        "flush bias sums": m[14] / 1e3, "flush bias cycles per dZ unit": m[14] / max(m[15], 1),
+        "flush wait full": m[16] / 1e3, "flush wait release barrier": m[17] / 1e3,
+        "releases, last = issuer0": m[18], "releases, last = issuer1": m[19], "releases, last = flush": m[20],
+        "releases, flush first": m[21],
+        "issuer0 between groups": m[22] / 1e3, "issuer1 between groups": m[23] / 1e3,
         "items min/max": f"{a[:, 7].min():.0f}/{a[:, 7].max():.0f}",
         "end min/max": end.min() / end.max(),
     }

@@ -312,6 +312,11 @@ struct WTask {
 //      4: A = PE(dir): columns 0..2 = Yd = PE(dir)^T d(rgb_pre) into the scratch     (tc_finish_kernel uses Y, Yd)
 
 struct WTaskTable { WTask t[kNumTasks]; };
+// One accumulator group as its issuer runs it, built once per work item: units a / b, rel = release unit a (bit 0) /
+// unit b (bit 1) after this group, cover / last = TMEM blocks the group writes / whose accumulation it ends for this
+// issuer, slot-0 operand descriptors (with a_sub / b_sub), accumulator address, instruction descriptor.
+struct IssueGroup { int a, b; uint32_t rel, cover, last; uint64_t da, db; uint32_t tcol, idesc; };
+constexpr int kWMaxMine = 2;          // groups per issuer and task
 __host__ __device__ inline int blk_first(const WGroup& g) { return g.col >> 7; }
 __host__ __device__ inline int blk_last(const WGroup& g) { return (g.col + (g.N < 32 ? 32 : g.N) - 1) >> 7; }
 
@@ -351,6 +356,11 @@ static void finish_task_table(WTaskTable& T, int n) {
     WTask& t = T.t[k];
     if (k != n - 1)
       for (int gi = 0; gi < t.n_groups; ++gi) t.g[gi].issuer = gi & 1;
+    for (int x = 0; x < 2; ++x) {
+      int mine = 0;
+      for (int gi = 0; gi < t.n_groups; ++gi) mine += t.g[gi].issuer == x;
+      if (mine > kWMaxMine) std::abort();   // the issuer keeps at most kWMaxMine groups in registers
+    }
     for (int x = 0; x < 2; ++x) {
       for (int u = 0; u < kWMaxUnits; ++u) {
         t.last_grp[x][u] = -1;
@@ -475,8 +485,15 @@ static WTaskTable build_task_table8(int dx, int dd) {
 // per CTA: 0 producer waits for a free slot (cycles) | 1, 2 issuer 0 / 1 waits for a loaded slot | 3, 4 issuer 0 / 1 waits
 // for the previous item's flush | 5 flush warp 2: cycles from acc_done to its acc_free arrive | 6 flush warp 2 waits for
 // acc_done | 7 items | 8 tiles | 9, 10 %globaltimer (ns) at the CTA's start / end | 11 CTA cycles start to end
+// | 12, 13 issuer 0 / 1 cycles inside its MMA + commit sequences (its waits excluded) | 14 flush warp 2: cycles of the
+// bias column sums | 15 dZ units column-summed | 16 flush warp 2 waits for a loaded slot | 17 flush warp 2 waits at the
+// slot-release barrier of the four flush warps | 18, 19, 20 slot releases whose last arrival came from issuer 0 /
+// issuer 1 / the flush warps | 21 releases where the flush warps arrived first | 22, 23 issuer 0 / 1 cycles from the end
+// of one MMA + commit sequence to the start of the next group's waits (the loop's own instructions)
+// (18-20: the flush warps' place is exact -- the pending count of the barrier state their arrive returns; between the
+// two issuers the one that committed later counts as the later, since the MMAs of one SM complete in issue order)
 #ifdef KNERF_TC_TIMING
-constexpr int kWProf = 12;
+constexpr int kWProf = 24;
 static __device__ unsigned long long g_wg_prof[160][kWProf];
 __device__ __forceinline__ unsigned long long globaltimer_ns() {
   unsigned long long t;
@@ -489,6 +506,15 @@ __device__ __forceinline__ unsigned long long globaltimer_ns() {
 #define KN_WG_ADD(slot, v) kn_wg[slot] += (unsigned long long)(v)
 #define KN_WG_CLOCK(var) const long long var = clock64()
 #define KN_WG_FLUSH() for (int kn_i = 0; kn_i < kWProf; ++kn_i) if (kn_wg[kn_i]) atomicAdd(&g_wg_prof[blockIdx.x][kn_i], kn_wg[kn_i])
+// mbarrier arrive that returns how many arrivals the phase still expected before this one (1: this one completed it)
+__device__ __forceinline__ uint32_t mbar_arrive_pending(uint64_t* bar) {
+  uint32_t n;
+  asm volatile("{\n\t.reg .b64 st;\n\t"
+               "mbarrier.arrive.shared::cta.b64 st, [%1];\n\t"
+               "mbarrier.pending_count.b64 %0, st;\n\t}"
+               : "=r"(n) : "r"(smem_u32(bar)) : "memory");
+  return n;
+}
 #else
 #define KN_WG_DECL()
 #define KN_WG_WAIT(slot, bar, par) mbar_wait(bar, par)
@@ -502,6 +528,11 @@ struct WSmem {
   uint64_t full[kWSlots], empty[kWSlots], acc_done[kWBlocks], acc_free[kWBlocks], q_full[kWQueue], q_empty[kWQueue];
   int q_item[kWQueue];
   uint32_t tmem_base;
+  WUnit pu[kWMaxUnits];                // the producer's copy of the current task's units
+#ifdef KNERF_TC_TIMING
+  long long kn_commit_t[kWSlots][2];   // clock64 of each issuer's last release of the slot's current use
+  int kn_flush_tag[kWSlots];           // (use << 1) | 1 if the flush warps' arrival completed the release
+#endif
 };
 
 // Work items: (task, tiles [lo, hi)), claimed one at a time from a counter in the fp32 scratch (kXOffQueue) in the
@@ -571,6 +602,9 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
     for (int b = 0; b < kWBlocks; ++b) { mbar_init(&sm.acc_done[b], 2); mbar_init(&sm.acc_free[b], 128); }
     // a queue entry is read by the two issuers and the four flush warps
     for (int i = 0; i < kWQueue; ++i) { mbar_init(&sm.q_full[i], 1); mbar_init(&sm.q_empty[i], 6); }
+#ifdef KNERF_TC_TIMING
+    for (int i = 0; i < kWSlots; ++i) sm.kn_flush_tag[i] = -2;
+#endif
     fence_mbar_init();
   }
   if (warp == 1) tmem_alloc<512>(&sm.tmem_base);
@@ -596,15 +630,26 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
         mbar_arrive(&sm.q_full[j % kWQueue]);
         if (item < 0) break;
         const WTask& t = T.t[L.task[item]];
+        const int n_units = t.n_units;
+        for (int k = 0; k < n_units; ++k) sm.pu[k] = t.u[k];   // (indexed constant-bank reads are slow: once per item)
         for (int64_t tile = L.range[item].x; tile < L.range[item].y; ++tile) {
-          for (int k = 0; k < t.n_units; ++k, ++it) {
+          for (int k = 0; k < n_units; ++k, ++it) {
+            const WUnit u = sm.pu[k];
             const uint32_t slot = it % kWSlots, ph = (it / kWSlots) & 1;
-            const uint8_t* src = (t.u[k].src == 0 ? rec + tile * kRB : dz + tile * kDB) + t.u[k].off;
+            const uint8_t* src = (u.src == 0 ? rec + tile * kRB : dz + tile * kDB) + u.off;
             KN_WG_WAIT(0, &sm.empty[slot], ph ^ 1);
-            mbar_arrive_expect_tx(&sm.full[slot], t.u[k].bytes + t.u[k].bytes2);
-            tma_load_1d(sm.slot[slot], src, t.u[k].bytes, &sm.full[slot]);
-            if (t.u[k].bytes2)
-              tma_load_1d(sm.slot[slot] + kSub2, dz + tile * kDB + t.u[k].off2, t.u[k].bytes2, &sm.full[slot]);
+#ifdef KNERF_TC_TIMING
+            if (it >= (uint32_t)kWSlots) {   // who released use it / kWSlots - 1 of this slot last
+              const int tag = *reinterpret_cast<volatile int*>(&sm.kn_flush_tag[slot]);
+              const volatile long long* ct = sm.kn_commit_t[slot];
+              // a tag not yet written for this use: the flush warps' arrival was the one that just completed it
+              if ((tag >> 1) != (int)(it / kWSlots - 1) || (tag & 1)) KN_WG_ADD(20, 1);
+              else KN_WG_ADD(ct[0] > ct[1] ? 18 : 19, 1);
+            }
+#endif
+            mbar_arrive_expect_tx(&sm.full[slot], u.bytes + u.bytes2);
+            tma_load_1d(sm.slot[slot], src, u.bytes, &sm.full[slot]);
+            if (u.bytes2) tma_load_1d(sm.slot[slot] + kSub2, dz + tile * kDB + u.off2, u.bytes2, &sm.full[slot]);
           }
         }
       }
@@ -612,13 +657,44 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
   } else if (warp == 1 || warp == 6) {
     if (lane == 0) {
       const int me = (warp == 1) ? 0 : 1;
+      const uint32_t slot0 = smem_u32(sm.slot[0]);
       uint32_t it = 0;
+#ifdef KNERF_TC_TIMING
+      long long kn_mark = clock64();
+#endif
       for (int j = 0;; ++j) {
         const int item = take_item(j);
         mbar_arrive(&sm.q_empty[j % kWQueue]);
         if (item < 0) break;
         const WTask& t = T.t[L.task[item]];
         const int64_t lo = L.range[item].x, hi = L.range[item].y;
+        // This issuer's part of the task, read from the table once per item: the table lives in the constant bank,
+        // and the indexed reads of it in the tile loop held the issuer ~1,150 cycles per tile
+        // (profiles/r04_wgrad_limiter.md).
+        IssueGroup mine[kWMaxMine];
+        int n_mine = 0;
+        uint32_t skip = 0;   // units this issuer never reads
+        for (int k = 0; k < t.n_units; ++k)
+          if (t.last_grp[me][k] < 0) skip |= 1u << k;
+        for (int gi = 0; gi < t.n_groups; ++gi) {
+          const WGroup& g = t.g[gi];
+          if (g.issuer != me) continue;
+          IssueGroup m;
+          m.a = g.a; m.b = g.b;
+          m.rel = (t.last_grp[me][g.a] == gi ? 1u : 0u) | (g.b != g.a && t.last_grp[me][g.b] == gi ? 2u : 0u);
+          m.cover = 0u; m.last = 0u;
+          for (int b = blk_first(g); b <= blk_last(g); ++b) {
+            m.cover |= 1u << b;
+            if (t.last_in_blk[me][b] == gi) m.last |= 1u << b;   // this group ends this issuer's part of block b
+          }
+          m.da = umma_smem_desc(slot0 + g.a_sub, 128, kChunkA);
+          m.db = umma_smem_desc(slot0 + g.b_sub, 128, kChunkA);
+          m.tcol = tmem + g.col;
+          m.idesc = REC8 ? umma_idesc_f8(128, g.N, kE4M3, kE5M2, 1, 1) : umma_idesc_bf16(128, g.N, 1, 1);
+          if (n_mine == 0) mine[0] = m; else mine[1] = m;   // constant indices keep `mine` in registers
+          ++n_mine;
+        }
+        const int n_units = t.n_units;
         // Block b of this item may be written once the flush warps have drained it for the previous item.  Every item
         // waits for all blocks (those it does not write at its end, before its acc_done arrival), so that neither
         // barrier of a block can get a phase ahead of its reader.
@@ -630,52 +706,58 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
             freed |= 1u << b;
           }
         };
-        for (int64_t tile = lo; tile < hi; ++tile, it += t.n_units) {
-          for (int gi = 0; gi < t.n_groups; ++gi) {
-            const WGroup& g = t.g[gi];
-            if (g.issuer != me) continue;
-            const int b0 = blk_first(g), b1 = blk_last(g);
-            if (tile == lo)
-              for (int b = b0; b <= b1; ++b) wait_free(b);
-            const uint32_t ia = it + g.a, ib = it + g.b;
-            const uint32_t sa = ia % kWSlots, sb = ib % kWSlots;
-            KN_WG_WAIT(1 + me, &sm.full[sa], (ia / kWSlots) & 1);
-            KN_WG_WAIT(1 + me, &sm.full[sb], (ib / kWSlots) & 1);
-            tc_fence_after();
-            const uint32_t a_base = smem_u32(sm.slot[sa]) + g.a_sub, b_base = smem_u32(sm.slot[sb]) + g.b_sub;
-            if (REC8) {   // e4m3 activations x e5m2 gradients, 32 samples per MMA (512 B further along every chunk)
-              const uint32_t idesc = umma_idesc_f8(128, g.N, kE4M3, kE5M2, 1, 1);
+        auto issue = [&](const IssueGroup& m, int64_t tile) {
+#ifdef KNERF_TC_TIMING
+          KN_WG_ADD(22 + me, clock64() - kn_mark);
+#endif
+          if (tile == lo)
+            for (int b = 0; b < kWBlocks; ++b)
+              if ((m.cover >> b) & 1u) wait_free(b);
+          const uint32_t ia = it + m.a, ib = it + m.b;
+          const uint32_t sa = ia % kWSlots, sb = ib % kWSlots;
+          KN_WG_WAIT(1 + me, &sm.full[sa], (ia / kWSlots) & 1);
+          KN_WG_WAIT(1 + me, &sm.full[sb], (ib / kWSlots) & 1);
+          KN_WG_CLOCK(kn_issue);
+          tc_fence_after();
+          // the descriptors' start-address field is addr >> 4 (< 2^14 for any shared-memory address): slot and k
+          // offsets add to the precomputed slot-0 descriptors
+          const uint64_t da = m.da + (uint64_t)(sa * (kWUnitBytes >> 4)), db = m.db + (uint64_t)(sb * (kWUnitBytes >> 4));
+          if (REC8) {   // e4m3 activations x e5m2 gradients, 32 samples per MMA (512 B further along every chunk)
 #pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint64_t da = umma_smem_desc(a_base + k * 512, 128, kChunkA);
-                const uint64_t db = umma_smem_desc(b_base + k * 512, 128, kChunkA);
-                umma_f8(tmem + g.col, da, db, idesc, (tile > lo || k > 0) ? 1u : 0u);
-              }
-            } else {
-              const uint32_t idesc = umma_idesc_bf16(128, g.N, 1, 1);
+            for (int k = 0; k < 4; ++k)
+              umma_f8(m.tcol, da + k * 32, db + k * 32, m.idesc, (tile > lo || k > 0) ? 1u : 0u);
+          } else {
 #pragma unroll
-              for (int k = 0; k < 8; ++k) {   // K = 128 samples per tile, 16 per MMA; MN-major: LBO = 128 B, SBO = 2 KB
-                const uint64_t da = umma_smem_desc(a_base + k * 256, 128, kChunkA);
-                const uint64_t db = umma_smem_desc(b_base + k * 256, 128, kChunkA);
-                umma_bf16(tmem + g.col, da, db, idesc, (tile > lo || k > 0) ? 1u : 0u);
-              }
-            }
-            if (t.last_grp[me][g.a] == gi) umma_commit(&sm.empty[sa]);
-            if (g.b != g.a && t.last_grp[me][g.b] == gi) umma_commit(&sm.empty[sb]);
-            if (tile + 1 == hi) {
-              for (int b = b0; b <= b1; ++b) {
-                if (t.last_in_blk[me][b] != gi) continue;   // this issuer's part of block b is complete
-                umma_commit(&sm.acc_done[b]);
-                done |= 1u << b;
-              }
-            }
+            for (int k = 0; k < 8; ++k)   // K = 128 samples per tile, 16 per MMA; MN-major: LBO = 128 B, SBO = 2 KB
+              umma_bf16(m.tcol, da + k * 16, db + k * 16, m.idesc, (tile > lo || k > 0) ? 1u : 0u);
           }
+#ifdef KNERF_TC_TIMING
+          if (m.rel & 1u) sm.kn_commit_t[sa][me] = clock64();
+          if (m.rel & 2u) sm.kn_commit_t[sb][me] = clock64();
+#endif
+          if (m.rel & 1u) umma_commit(&sm.empty[sa]);
+          if (m.rel & 2u) umma_commit(&sm.empty[sb]);
+          if (tile + 1 == hi && m.last) {
+            for (int b = 0; b < kWBlocks; ++b)
+              if ((m.last >> b) & 1u) umma_commit(&sm.acc_done[b]);
+            done |= m.last;
+          }
+          KN_WG_ADD(12 + me, clock64() - kn_issue);
+#ifdef KNERF_TC_TIMING
+          kn_mark = clock64();
+#endif
+        };
+        for (int64_t tile = lo; tile < hi; ++tile, it += n_units) {
+          if (n_mine > 0) issue(mine[0], tile);
+          if (n_mine > 1) issue(mine[1], tile);
           // units this issuer never reads: release them too (after their load has landed, so that the arrival
           // counts for this use of the slot and not for the previous one)
-          for (int k = 0; k < t.n_units; ++k) {
-            if (t.last_grp[me][k] >= 0) continue;
-            const uint32_t iu = it + k;
+          for (uint32_t sk = skip; sk != 0u; sk &= sk - 1u) {
+            const uint32_t iu = it + (uint32_t)(__ffs(sk) - 1);
             mbar_wait(&sm.full[iu % kWSlots], (iu / kWSlots) & 1);
+#ifdef KNERF_TC_TIMING
+            sm.kn_commit_t[iu % kWSlots][me] = clock64();
+#endif
             mbar_arrive(&sm.empty[iu % kWSlots]);
           }
         }
@@ -715,8 +797,10 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
         int nb = 0;
         for (int k = 0; k < t.n_units; ++k, ++uit) {
           const uint32_t slot = uit % kWSlots;
-          mbar_wait(&sm.full[slot], (uit / kWSlots) & 1);
+          KN_WG_WAIT(16, &sm.full[slot], (uit / kWSlots) & 1);
+          KN_WG_CLOCK(kn_bias);
           if (t.u[k].bias_layer >= 0) {
+            KN_WG_ADD(15, 1);
             const uint8_t* base = sm.slot[slot] + fc * kChunkA + fsub * 16;
             if (REC8) {
 #pragma unroll 4
@@ -724,11 +808,7 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
                 const uint4 v = *reinterpret_cast<const uint4*>(base + i * 128);
                 const uint32_t wv[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
-                for (int jj = 0; jj < 4; ++jj) {
-                  const float2 lo2 = e5m2x2_lo(wv[jj]), hi2 = e5m2x2_hi(wv[jj]);
-                  float* a = bacc[jj >> 1] + (jj & 1) * 4;
-                  a[0] += lo2.x; a[1] += lo2.y; a[2] += hi2.x; a[3] += hi2.y;
-                }
+                for (int jj = 0; jj < 4; ++jj) add_e5m2x4(bacc[jj >> 1] + (jj & 1) * 4, wv[jj]);
               }
             } else {
               float* a = bacc[nb & 1];
@@ -745,8 +825,20 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
             const uint2 v = *reinterpret_cast<const uint2*>(sm.slot[slot] + 8192 + ftid * 16);   // one row per thread: this
             pacc[0] += bf16_lo(v.x); pacc[1] += bf16_hi(v.x); pacc[2] += bf16_lo(v.y);           // sits on the slot-release path
           }
+#ifdef KNERF_TC_TIMING
+          const long long kn_sum_end = clock64();
+          KN_WG_ADD(14, kn_sum_end - kn_bias);
+          named_bar_sync(2, 128);
+          KN_WG_ADD(17, clock64() - kn_sum_end);
+          if (ftid == 0) {
+            const uint32_t pending = mbar_arrive_pending(&sm.empty[slot]);
+            sm.kn_flush_tag[slot] = (int)((uit / kWSlots) << 1) | (pending == 1 ? 1 : 0);
+            if (pending == 3) KN_WG_ADD(21, 1);
+          }
+#else
           named_bar_sync(2, 128);               // all 128 readers are done with the slot
           if (ftid == 0) mbar_arrive(&sm.empty[slot]);
+#endif
         }
       }
       {

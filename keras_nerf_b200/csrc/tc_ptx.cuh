@@ -255,14 +255,18 @@ __device__ __forceinline__ uint32_t pack_e5m2x4(float a, float b, float c, float
       : "=r"(r) : "f"(a), "f"(b), "f"(c), "f"(d));
   return r;
 }
-// an e5m2 byte is the upper byte of the fp16 with the same value: bytes (0, 1) / (2, 3) of a word -> two fp32
-__device__ __forceinline__ float2 e5m2x2_lo(uint32_t w) {
-  const uint32_t h = __byte_perm(w, 0u, 0x1404);
-  return __half22float2(*reinterpret_cast<const __half2*>(&h));
+// acc += an fp16 value: one instruction (FHADD, which reads either half of a register), exact fp16 -> fp32 and one fp32
+// rounding -- the same bits as a conversion followed by an fp32 add
+__device__ __forceinline__ float add_f16(float acc, unsigned short h) {
+  asm("add.rn.f32.f16 %0, %1, %0;" : "+f"(acc) : "h"(h));
+  return acc;
 }
-__device__ __forceinline__ float2 e5m2x2_hi(uint32_t w) {
-  const uint32_t h = __byte_perm(w, 0u, 0x3424);
-  return __half22float2(*reinterpret_cast<const __half2*>(&h));
+// a[0..3] += the four e5m2 bytes of w.  An e5m2 byte is the upper byte of the fp16 with the same value, so one prmt
+// makes two fp16 of two bytes.
+__device__ __forceinline__ void add_e5m2x4(float* a, uint32_t w) {
+  const uint32_t lo = __byte_perm(w, 0u, 0x1404), hi = __byte_perm(w, 0u, 0x3424);
+  a[0] = add_f16(a[0], (unsigned short)(lo & 0xffffu)); a[1] = add_f16(a[1], (unsigned short)(lo >> 16));
+  a[2] = add_f16(a[2], (unsigned short)(hi & 0xffffu)); a[3] = add_f16(a[3], (unsigned short)(hi >> 16));
 }
 // prmt.b32 in its default mode: a selector nibble with bit 3 set yields the SIGN of the selected byte replicated over
 // the byte (0x00 / 0xff) -- one instruction turns flag bits parked in byte msbs into byte / half-word masks
