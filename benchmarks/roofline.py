@@ -12,10 +12,11 @@ if ROOT not in sys.path:
 
 # SURVEY §8(d): algorithmic work per sample (unpadded shapes)
 FLOP_FWD_PER_SAMPLE = 1_186_816            # 593,408 MAC
-# bf16 INFERENCE executes fewer: `features` is folded into `rgb_features` (no activation in between, mlp.py:42-46)
-# and sigma becomes output column 128 of that step: 593,408 - 256*256 + 288*16 MAC.  Throughput figures keep the
-# unfolded count (SURVEY §8d) and carry the executed one next to it.
-FLOP_FWD_INFER_EXECUTED = 2 * (593_408 - 256 * 256 + 288 * 16)
+# bf16 INFERENCE executes fewer: `features`, `rgb_features` and the rgb head are folded into one N = 16 step from h7 and
+# PE(dir) (no activation before the sigmoid, mlp.py:42-48) whose column 3 is sigma: 593,408 - 256*256 (features)
+# - 283*128 (rgb_features) - 128*3 (rgb) - 256 (sigma) + 288*16 MAC.  Throughput figures keep the unfolded count
+# (SURVEY §8d) and carry the executed one next to it.
+FLOP_FWD_INFER_EXECUTED = 2 * (593_408 - 256 * 256 - 283 * 128 - 128 * 3 - 256 + 288 * 16)
 FLOP_TRAIN_PER_SAMPLE = 3_489_024          # fwd + dgrad + wgrad
 FLOP_WGRAD_PER_SAMPLE = 1_186_816          # every weight once more
 FLOP_DGRAD_PER_SAMPLE = FLOP_TRAIN_PER_SAMPLE - FLOP_FWD_PER_SAMPLE - FLOP_WGRAD_PER_SAMPLE
@@ -186,5 +187,5 @@ def render_ms_per_frame(precision, dev, strategy=None, wh=800, frames=2):
     if model.precision == "bf16":
         out["tflops_executed"] = FLOP_FWD_INFER_EXECUTED * samples / (ms * 1e-3) / 1e12
         out["note"] = ("tflops counts the unfolded 593,408 MAC/sample; the inference kernel folds features into "
-                       "rgb_features and executes 532,480 MAC/sample (tflops_executed)")
+                       "rgb_features and the heads and executes 495,616 MAC/sample (tflops_executed)")
     return out

@@ -26,6 +26,9 @@ int knerf_selftest_umma2(const void* a_blob, const void* b_blob, int N, int K, f
  * library was built with -DKNERF_TC_TIMING (release builds carry no instrumentation). */
 int knerf_debug_tc_timing(unsigned long long* host_out, int n);
 
+/* The same for the BF16 dgrad kernel (same 40 slots; slot 15 + 16 tl: its per-tile prologue). */
+int knerf_debug_dgrad_timing(unsigned long long* host_out, int n);
+
 /* The same for the BF16 weight-gradient kernel (24 uint64 per CTA; slots documented in csrc/mlp_tc_bwd.cu kWProf):
  * wait and busy cycles of its producer, issuers and flush warps, which arrival released each ring slot last, items
  * and tiles per CTA, %globaltimer at CTA start and end. */

@@ -78,6 +78,7 @@ SIGNATURES = {
                                   _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _I]),
     "knerf_debug_tc_timing": (_I, [_P, _I]),
     "knerf_debug_wgrad_timing": (_I, [_P, _I]),
+    "knerf_debug_dgrad_timing": (_I, [_P, _I]),
     "knerf_selftest_umma": (_I, [_I, _P, _P, _I, _I, _P, _P]),
     "knerf_selftest_umma2": (_I, [_P, _P, _I, _I, _P, _P]),
 }

@@ -112,6 +112,7 @@ extern "C" int knerf_device_supports_bf16(void) {
 
 extern "C" int knerf_debug_tc_timing(unsigned long long* host_out, int n) { return tc_debug_timing(host_out, n); }
 extern "C" int knerf_debug_wgrad_timing(unsigned long long* host_out, int n) { return tc_debug_wgrad_timing(host_out, n); }
+extern "C" int knerf_debug_dgrad_timing(unsigned long long* host_out, int n) { return tc_debug_dgrad_timing(host_out, n); }
 
 extern "C" int64_t knerf_param_count(const knerf_config* cfg) {
   Model m;

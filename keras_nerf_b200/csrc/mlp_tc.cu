@@ -8,11 +8,11 @@
 //
 // Forward kernel (persistent CTA pairs, 384 threads per CTA; roles in tc_roles.cuh / tc_roles2.cuh):
 //   warp 0      TMA producer: streams this CTA's half of the pre-packed bf16 weight blob, K = 64 stages, 4-slot ring
-//   warps 1,11  MMA issuers (leader CTA): tcgen05.mma.cta_group::2 (M = 256, N = 256|144, K = 16), alternate items
+//   warps 1,11  MMA issuers (leader CTA): tcgen05.mma.cta_group::2 (M = 256, N = 256|16, K = 16), alternate items
 //   warps 2-9   compute:      PE prologue, TMEM -> register epilogues (ReLU, bf16 pack) that write the next layer's
-//                             A operand straight into shared memory, rgb head, output.
-//                             Biases ride in the GEMM (constant-1 column, tc_layout.cuh); sigma is column 128 of
-//                             the last step.
+//                             A operand straight into shared memory, output (sigmoid / ReLU of the head columns).
+//                             Biases ride in the GEMM (constant-1 column, tc_layout.cuh); the last step's N = 16
+//                             columns are the folded heads' pre-activations (rgb, sigma).
 //   warp 10     record store (training): bulk copies of the operand tiles to HBM
 // Each CTA keeps TWO 128-sample tiles in flight (accumulators in TMEM columns [0,256) and [256,512)): while
 // the tensor core runs tile 1's layer, the compute warps drain tile 0's accumulator and build its next A
@@ -48,50 +48,78 @@ __device__ __forceinline__ float fwd_weight(const float* __restrict__ params, co
   }
   return params[P.w_off[L] + (int64_t)row * U + n];
 }
-// W' = W_f W_g[:256] [256,128] and its bias b_f W_g[:256] + b_g [128] in fp32 (tc_layout.cuh), one thread per element
-__global__ void __launch_bounds__(128) fold_kernel(const float* __restrict__ params, TcParams P, float* __restrict__ fold) {
+// W' = W_f W_g[:256] [256,128] and its bias b_f W_g[:256] + b_g [128] in fp32 (tc_layout.cuh), one thread per element,
+// and the folded heads (kHeadOff): head row k = (row k of [W'; D; b'] times W_c, then + b_c for the bias row; sigma's
+// kernel / bias in column 3).  Block k: k < 256 row k of W', 256 + i row i of W_g[U:] (i < dd), 288 the bias row.
+// The products over n run through one fixed reduction tree: the same bits run after run, and zero-padded rows and
+// columns (a narrower model embedded in the 256-wide chain) only add exact zeros.
+__global__ void __launch_bounds__(128) fold_kernel(const float* __restrict__ params, TcParams P, float* __restrict__ fold,
+                                                   float* __restrict__ head) {
   const int U = P.U, H = P.U / 2;
   const float* Wf = params + P.w_off[9];    // features      [U, U]
   const float* Wg = params + P.w_off[10];   // rgb_features  [U + dd, U/2]
-  const int n = threadIdx.x, k = blockIdx.x;   // k = 256: the bias row
+  const float* Wc = params + P.w_off[11];   // rgb           [U/2, 3]
+  const int n = threadIdx.x, k = blockIdx.x;
   float acc = 0.f;
-  if (n < H && (k < U || k == 256)) {
-    const float* row = k < 256 ? Wf + (int64_t)k * U : params + P.b_off[9];
-    acc = k < 256 ? 0.f : params[P.b_off[10] + n];
+  if (k < 256 || k == 288) {
+    if (n < H && (k < U || k == 288)) {
+      const float* row = k < 256 ? Wf + (int64_t)k * U : params + P.b_off[9];
+      acc = k < 256 ? 0.f : params[P.b_off[10] + n];
 #pragma unroll 8
-    for (int j = 0; j < U; ++j) acc = fmaf(row[j], Wg[j * H + n], acc);
+      for (int j = 0; j < U; ++j) acc = fmaf(row[j], Wg[j * H + n], acc);
+    }
+    fold[(k < 256 ? k : 256) * 128 + n] = acc;
+  } else if (n < H && k - 256 < P.dd) {
+    acc = Wg[(int64_t)(U + k - 256) * H + n];
   }
-  fold[k * 128 + n] = acc;
-}
-// last forward step: reduction index k (h7, then the direction encoding), output column n
-__device__ __forceinline__ float fold_weight(const float* __restrict__ params, const TcParams& P,
-                                             const float* __restrict__ fold, int k, int n) {
-  if (n < 128) {
-    if (k >= 256) return (k - 256 < P.dd && n < P.U / 2) ? params[P.w_off[10] + (int64_t)(P.U + k - 256) * (P.U / 2) + n] : 0.f;
-    return fold[k * 128 + n];
+  __shared__ float red[4][3];
+  float c3[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    c3[c] = n < H ? acc * Wc[n * 3 + c] : 0.f;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) c3[c] += __shfl_xor_sync(0xffffffffu, c3[c], o);
+    if ((n & 31) == 0) red[n >> 5][c] = c3[c];
   }
-  return (n == 128 && k < P.U) ? params[P.w_off[8] + k] : 0.f;   // sigma kernel [U, 1]
+  __syncthreads();
+  if (n < 3) {
+    float v = (red[0][n] + red[1][n]) + (red[2][n] + red[3][n]);
+    if (k == 288) v += params[P.b_off[11] + n];
+    head[k * 4 + n] = v;
+  } else if (n == 3) {
+    head[k * 4 + 3] = k < U ? params[P.w_off[8] + k] : (k == 288 ? params[P.b_off[8]] : 0.f);   // sigma [U, 1], b_s
+  }
 }
-__device__ __forceinline__ float fold_bias(const float* __restrict__ params, const TcParams& P,
-                                           const float* __restrict__ fold, int n) {
-  return n < 128 ? fold[256 * 128 + n] : (n == 128 ? params[P.b_off[8]] : 0.f);
+// last forward step: reduction index k (h7, then the direction encoding), output column n.  Column c < 4 takes the bf16
+// rounding of head value c, column 4 + c the bf16 rounding of what that leaves: the epilogue adds the two accumulators,
+// so the folded weights enter with ~2^-17 relative error instead of one bf16 rounding of the whole product W' W_c
+// (which on trained weights, where the terms of W' W_c add up coherently, doubled the fine pass's pixel error).
+__device__ __forceinline__ float fold_split(float v, int n) {
+  const float hi = bf16_lo(pack_bf16x2(v, 0.f));
+  return n < 4 ? hi : v - hi;
+}
+__device__ __forceinline__ float fold_weight(const float* __restrict__ head, int k, int n) {
+  return n < 8 ? fold_split(head[k * 4 + (n & 3)], n) : 0.f;
+}
+__device__ __forceinline__ float fold_bias(const float* __restrict__ head, int n) {
+  return n < 8 ? fold_split(head[288 * 4 + (n & 3)], n) : 0.f;
 }
 // B operand element of dgrad step b: output n = input feature of the layer (< 256), reduction index k = its output
-// feature.  b = 0 goes from d(rgb_features) straight to d(h7): W'[n][k]
+// feature.  b = 0 goes from (d rgb_pre, d sigma_pre) straight to d(h7): [W''' | w_s][n][k]
 __device__ __forceinline__ float bwd_weight(const float* __restrict__ params, const TcParams& P,
-                                            const float* __restrict__ fold, int b, int k, int n) {
-  if (b == 0) return fold[n * 128 + k];
+                                            const float* __restrict__ head, int b, int k, int n) {
+  if (b == 0) return k < 4 ? head[n * 4 + k] : 0.f;
   if (P.w_off[BwdProg::layer(b)] < 0) return n == k ? 1.f : 0.f;   // identity layer of the embedding
   return (n < P.U && k < P.U) ? params[P.w_off[BwdProg::layer(b)] + (int64_t)n * P.U + k] : 0.f;
 }
 
 template <class Prog, bool FWD>
 __device__ __forceinline__ void pack_pair(const float* __restrict__ params, const TcParams& P,
-                                          const float* __restrict__ fold, uint8_t* __restrict__ blob, int gtid, int gsz) {
+                                          const float* __restrict__ head, uint8_t* __restrict__ blob, int gtid, int gsz) {
   using PL = PairLayout<Prog>;
   auto weight = [&](int s, int k, int n) -> float {
-    if (!FWD) return bwd_weight(params, P, fold, s, k, n);
-    return s == 8 ? fold_weight(params, P, fold, k, n) : fwd_weight(params, P, s, k, n);
+    if (!FWD) return bwd_weight(params, P, head, s, k, n);
+    return s == 8 ? fold_weight(head, k, n) : fwd_weight(params, P, s, k, n);
   };
   for (int v = gtid; v < PL::kBytes / 16; v += gsz) {
     const int byte = v * 16;
@@ -114,7 +142,7 @@ __device__ __forceinline__ void pack_pair(const float* __restrict__ params, cons
       const int cta = rem / pb, r2 = rem - cta * pb;
       const int cb = r2 / (half * 16), nl = (r2 - cb * half * 16) / 16;
       if (cb == 1)
-        w[3] = pack_bf16x2(0.f, s == 8 ? fold_bias(params, P, fold, cta * half + nl)
+        w[3] = pack_bf16x2(0.f, s == 8 ? fold_bias(head, cta * half + nl)
                                        : ((P.b_off[s] < 0 || cta * half + nl >= P.U) ? 0.f : params[P.b_off[s] + cta * half + nl]));
     }
     *reinterpret_cast<uint4*>(blob + byte) = make_uint4(w[0], w[1], w[2], w[3]);
@@ -124,24 +152,9 @@ __device__ __forceinline__ void pack_pair(const float* __restrict__ params, cons
 __global__ void __launch_bounds__(256) pack_kernel(const float* __restrict__ params, TcParams P,
                                                    uint8_t* __restrict__ packed) {
   const int gtid = blockIdx.x * blockDim.x + threadIdx.x, gsz = gridDim.x * blockDim.x;
-  const float* fold = reinterpret_cast<const float*>(packed + kFoldOff);   // written by fold_kernel
-  pack_pair<FwdProg, true>(params, P, fold, packed + kFwdPairOff, gtid, gsz);
-  pack_pair<BwdProg, false>(params, P, fold, packed + kBwdPairOff, gtid, gsz);
-  float* aux = reinterpret_cast<float*>(packed + kAuxOff);
-  for (int i = gtid; i < kAuxFloats; i += gsz) {
-    const int blk = i >> 8, j = i & 255;
-    float v = 0.f;
-    if (blk < 12) {
-      const int fo = (blk == 8) ? 1 : (blk == 10) ? P.U / 2 : (blk == 11) ? 3 : P.U;
-      if (j < fo && P.b_off[blk] >= 0) v = params[P.b_off[blk] + j];
-    } else if (blk == 12) {
-      if (j < P.U) v = params[P.w_off[8] + j];          // sigma kernel [U,1]
-    } else {
-      const int k = i - 13 * 256;
-      if (k < (P.U / 2) * 3) v = params[P.w_off[11] + k];   // rgb kernel [U/2,3]
-    }
-    aux[i] = v;
-  }
+  const float* head = reinterpret_cast<const float*>(packed + kHeadOff);   // written by fold_kernel
+  pack_pair<FwdProg, true>(params, P, head, packed + kFwdPairOff, gtid, gsz);
+  pack_pair<BwdProg, false>(params, P, head, packed + kBwdPairOff, gtid, gsz);
 }
 
 // ---- positional encoding into an A operand -----------------------------------------------------------------
@@ -282,10 +295,6 @@ __device__ __noinline__ void pe_dir(uint8_t* xs, uint8_t* rec, int r, int h, flo
   store_cols<REC8>(xs, rec, r, 2 * h, v, 2);
 }
 
-// fp32 head weights staged in the dead half of a tile's encoding buffer: [0,256) sigma kernel, [256,640) rgb
-// kernel [128,3], [640,644) b_sigma, b_rgb
-__device__ __forceinline__ float* head_smem(uint8_t* xs) { return reinterpret_cast<float*>(xs + 4 * kChunkA); }
-
 // ---- epilogue of a hidden step: accumulator -> bf16 A operand of the next step ---------------------------------
 // Thread (row r, half h) converts 128 of the 256 columns, 32 at a time.  The bias is already in the accumulator
 // (folded into the GEMM), ReLU (mlp.py:33-34) is fused into the bf16 conversion.  mask_out (training): the ReLU'
@@ -393,8 +402,6 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
     const int q = warp & 3, h = (warp - 2) >> 2;
     const int r = q * 32 + lane;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    const int ctid = tid - 64;
-    const float* aux = reinterpret_cast<const float*>(packed + kAuxOff);
     uint32_t acc_par[2] = {0, 0};
 
     uint32_t st_pending = 0, st_par = 0;      // training: bit tl = hs[tl] is being stored / parity of st_done[tl]
@@ -448,14 +455,7 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
           if (s < kLast) {
             // hidden layers: 128 of the 256 columns per thread
             float dirv[3];
-            float4 headw = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (s == 5) {   // fetched now, used after the epilogue: the L2 latency hides behind it
-              load_dir(dirv, d, g, M, S);
-              // rgb head weights -> shared memory (see below): sigma kernel [256] + rgb kernel [128,3] are contiguous
-              if (ctid < 160) headw = __ldg(reinterpret_cast<const float4*>(aux + 12 * 256) + ctid);
-              else if (ctid == 160) headw = make_float4(__ldg(aux + 8 * 256), __ldg(aux + 11 * 256), __ldg(aux + 11 * 256 + 1),
-                                                        __ldg(aux + 11 * 256 + 2));
-            }
+            if (s == 5) load_dir(dirv, d, g, M, S);   // fetched now, used after the epilogue: the L2 latency hides behind it
             hs_writable(tl);
             epi_hidden<TRAIN, REC8>(tmem + lane_base + tl * 256, sm.hs[tl], h, r,
                                     save ? rec_t + kOffMask + s * kMaskLayerBytes : nullptr,
@@ -463,58 +463,22 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
             if (s == 5) {
               // xs[tl] is dead after layer 5 (skip concat consumed): it now carries PE(dir) for the last step
               pe_dir<REC8>(sm.xs[tl], save ? rec_t + kOffDS : nullptr, r, h, dirv[0], dirv[1], dirv[2]);
-              // Chunks 4..7 of xs[tl] are dead until the next tile's PE(xyz): they hold the fp32 weights of the
-              // CUDA-core rgb head for the last step.  (With 227 KB of shared memory the SM has no L1: every __ldg
-              // of them was an L2 round trip.)  Visibility to the other warps: every warp passes a_ready(5) ->
-              // MMA(6) -> acc_ready(6) before anyone reads them.
-              if (ctid <= 160) *(reinterpret_cast<float4*>(head_smem(sm.xs[tl])) + ctid) = headw;
             }
             a_ready_arrive(tl, true);
           } else {
-            // columns 0..127: rgb_features (bias included, linear; mlp.py:43-46), then the rgb head + sigmoid on CUDA
-            // cores (mlp.py:48); column 128: the sigma pre-activation (mlp.py:40)
+            // columns 0..2 (+ 4..6): the rgb pre-activations, 3 (+ 7): sigma's (heads folded into the step, biases
+            // included; mlp.py:40, 43-48).  One half-row thread per row finishes it; the other starts the next tile.
             const int64_t next = pair + stride;
             float nin[3] = {0.f, 0.f, 0.f};   // the next tile of this slot: fetch its sample now, encode it afterwards
             if (next < n_pairs) load_sample(nin, o, d, t, tile_of(next, tl) * kTileM + r, M, S);
-            const float* wrgb = head_smem(sm.xs[tl]) + 256;
-            float pr = 0.f, pg = 0.f, pb = 0.f;
-#pragma unroll 1
-            for (int gI = 0; gI < 2; ++gI) {
-              const int col0 = h * 64 + gI * 32;
-              uint32_t v[32];
-              tmem_ld32_issue(tmem + lane_base + tl * 256 + col0, v);
-              // rgb kernel rows col0..col0+31: 96 consecutive floats, 16-byte aligned (shared memory)
-              float4 wq[24];
-#pragma unroll
-              for (int i = 0; i < 24; ++i) wq[i] = *(reinterpret_cast<const float4*>(wrgb + col0 * 3) + i);
-              tmem_ld32_wait(v);
-              const float* wv = reinterpret_cast<const float*>(wq);
-#pragma unroll
-              for (int c8 = 0; c8 < 4; ++c8) {
-                const float* x = reinterpret_cast<const float*>(&v[c8 * 8]);
-#pragma unroll
-                for (int e = 0; e < 8; ++e) {
-                  const int j = (c8 * 8 + e) * 3;
-                  pr += x[e] * wv[j]; pg += x[e] * wv[j + 1]; pb += x[e] * wv[j + 2];
-                }
-              }
-            }
-            float sig_pre = 0.f;
             if (h == 0) {   // warp-uniform
-              float v16[32];
-              tmem_ld32(tmem + lane_base + tl * 256 + 128, v16);   // (columns 144.. are stale: only [0] is used)
-              sig_pre = v16[0];
+              float a[8];
+              tmem_ld8(tmem + lane_base + tl * 256, a);
+              const float z[4] = {a[0] + a[4], a[1] + a[5], a[2] + a[6], a[3] + a[7]};
+              if (valid)
+                rgbsigma[g] = make_float4(1.f / (1.f + expf(-z[0])), 1.f / (1.f + expf(-z[1])), 1.f / (1.f + expf(-z[2])),
+                                          fmaxf(z[3], 0.f));
             }
-            if (h == 1) *reinterpret_cast<float4*>(sm.part[r]) = make_float4(pr, pg, pb, 0.f);
-            named_bar_sync(1, kComputeThreads);
-            if (h == 0 && valid) {
-              const float4 hb = *(reinterpret_cast<const float4*>(head_smem(sm.xs[tl])) + 160);   // b_sigma, b_rgb
-              const float4 o4 = *reinterpret_cast<const float4*>(sm.part[r]);
-              const float zr = pr + o4.x + hb.y, zg = pg + o4.y + hb.z, zb = pb + o4.z + hb.w;
-              rgbsigma[g] = make_float4(1.f / (1.f + expf(-zr)), 1.f / (1.f + expf(-zg)), 1.f / (1.f + expf(-zb)),
-                                        fmaxf(sig_pre, 0.f));
-            }
-            named_bar_sync(1, kComputeThreads);
             tc_fence_before();
             // this tile is finished: start the next pair's tile in the same slot right away
             if (next < n_pairs) prologue(next, tl, nin);
@@ -574,7 +538,8 @@ TcParams tc_make_params(const Model& m) {
 int tc_pack_weights(const Model& m, const float* params, void* packed, cudaStream_t st) {
   if (!is_flagship(m)) return fail(KNERF_ERR_UNSUPPORTED, "KNERF_BF16 implements models of dense_units <= 256 (even), up to 8 layers, at most one skip concat (not into the heads), L_xyz <= 10, L_dir <= 4");
   KN_CHECK_ARG((reinterpret_cast<uintptr_t>(packed) & 15) == 0, "tc_pack_weights: packed must be 16-byte aligned");
-  fold_kernel<<<257, 128, 0, st>>>(params, tc_make_params(m), reinterpret_cast<float*>((uint8_t*)packed + kFoldOff));
+  fold_kernel<<<kHeadRows, 128, 0, st>>>(params, tc_make_params(m), reinterpret_cast<float*>((uint8_t*)packed + kFoldOff),
+                                         reinterpret_cast<float*>((uint8_t*)packed + kHeadOff));
   KN_LAUNCH_CHECK();
   pack_kernel<<<kNumSMs * 2, 256, 0, st>>>(params, tc_make_params(m), (uint8_t*)packed);
   KN_LAUNCH_CHECK();

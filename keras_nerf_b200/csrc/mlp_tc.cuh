@@ -20,5 +20,6 @@ int tc_backward(const Model& m, const float* params, const void* packed, const f
 
 int tc_debug_timing(unsigned long long* host_out, int n);
 int tc_debug_wgrad_timing(unsigned long long* host_out, int n);
+int tc_debug_dgrad_timing(unsigned long long* host_out, int n);
 
 }  // namespace knerf

@@ -1,8 +1,8 @@
 // a11 (KNERF_BF16 mode): backward of the NeRF MLP on tcgen05 tensor cores.
 //
 //  1. tc_mlp_dgrad_kernel -- the forward's chain structure run backwards (same CTA-pair roles): starting from the
-//     gradient w.r.t. the head pre-activations (from the fused compositing backward) it goes from d(rgb_features)
-//     straight to d(h7) through W'^T (tc_layout.cuh: `features` is folded away), then layer 7 .. layer 1, each step
+//     gradient w.r.t. the head pre-activations (from the fused compositing backward) it goes from (d rgb_pre, d sigma_pre)
+//     straight to d(h7) through [W''' | w_s]^T (tc_layout.cuh: the heads are folded), then layer 7 .. layer 1, each step
 //     one [128 x 256] x [256 x 256] GEMM followed by a ReLU' epilogue (1-bit masks written by the forward).
 //     Every pre-activation gradient tile dZ_l is written once to HBM in chunk-major bf16 for step 2.
 //     No gradient flows into the xyz / direction encodings (mlp.py inputs are constants: nerf.py:361-369).
@@ -31,27 +31,21 @@ namespace {
 // dgrad chain
 // =============================================================================================================
 // epilogue of one dgrad step: accumulator (dH = dZ_next W^T) -> pre-activation gradient tile, bf16.
-// KIND 1: dZ7 = (dG W'^T + d(sigma_pre) Ws^T) * ReLU'(h7) -- the sigma head hangs off h7 too;
-// 2: dZ_l = dH * ReLU'(h_l), l = 6..1;  3: dZ0, the last step: feeds no further GEMM, so it goes to HBM directly
+// KIND 2: dZ_l = dH * ReLU'(h_l), l = 7..1;  3: dZ0, the last step: feeds no further GEMM, so it goes to HBM directly
 // (dst = record or nullptr) and must NOT touch hs[tl], which the other half-row thread of this row may already be
 // rebuilding for the next tile.  KIND < 3: dst = hs[tl], the next A operand and (via warp 10) the dZ record.
 // mb = this thread's ReLU' bits (4 x 32 columns; bit 8 t + q = column 4 q + t of the group).
 // REC8 (fp8 records): the dZ record leaves from here as e5m2(dZ * scale), 16 columns per 16-byte vector (rec8, nullptr
 // for a padding tile); dst is only the next A operand then (unused for KIND 3).
 template <int KIND, bool REC8>
-__device__ __noinline__ void epi_dgrad(uint32_t tacc, uint8_t* __restrict__ dst, int h, int r, uint4 mbv, float dsig,
-                                       const float* __restrict__ wsig, uint8_t* __restrict__ rec8) {
+__device__ __noinline__ void epi_dgrad(uint32_t tacc, uint8_t* __restrict__ dst, int h, int r, uint4 mbv,
+                                       uint8_t* __restrict__ rec8) {
   const uint32_t mb[4] = {mbv.x, mbv.y, mbv.z, mbv.w};   // by value: no local memory (no L1 on this SM)
 #pragma unroll
   for (int gI = 0; gI < 4; ++gI) {
     const int col0 = h * 128 + gI * 32;
     uint32_t v[32];
     tmem_ld32_issue(tacc + col0, v);
-    float4 ws[8];
-    if (KIND == 1) {
-#pragma unroll
-      for (int i = 0; i < 8; ++i) ws[i] = *(reinterpret_cast<const float4*>(wsig + col0) + i);   // shared memory
-    }
     tmem_ld32_wait(v);
     uint32_t q8[8];
 #pragma unroll
@@ -59,11 +53,6 @@ __device__ __noinline__ void epi_dgrad(uint32_t tacc, uint8_t* __restrict__ dst,
       float x[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) x[e] = __uint_as_float(v[c8 * 8 + e]);
-      if (KIND == 1) {
-        const float4 w0 = ws[2 * c8], w1 = ws[2 * c8 + 1];
-        x[0] += dsig * w0.x; x[1] += dsig * w0.y; x[2] += dsig * w0.z; x[3] += dsig * w0.w;
-        x[4] += dsig * w1.x; x[5] += dsig * w1.y; x[6] += dsig * w1.z; x[7] += dsig * w1.w;
-      }
       uint4 pk = make_uint4(pack_bf16x2(x[0], x[1]), pack_bf16x2(x[2], x[3]), pack_bf16x2(x[4], x[5]),
                             pack_bf16x2(x[6], x[7]));
       // ReLU' of columns 4q .. 4q+3 (q = 2 c8, 2 c8 + 1): bit q of bytes 0..3 of mb (tc_layout.cuh kRecMask).  Shifted left
@@ -128,8 +117,8 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
     if (lane == 0 && cta == 0) mma2_role<BwdProg>(sm, tmem, 1u, true, n_pairs, first, stride);
   } else if (warp == 10) {
     // record store: the A operands dZ7..dZ1 of the chain (items 1..7) are also the dZ records of the weight-gradient
-    // kernel (tc_roles.cuh store_role); item 0 = dG only takes part in the hand-shake: nothing downstream reads it
-    // from HBM (its weight gradients factor through d(rgb_pre), see build_task_table)
+    // kernel (tc_roles.cuh store_role); item 0 = (d rgb_pre, d sigma_pre) only takes part in the hand-shake: the
+    // prologue writes its record (kDzP)
     if (!REC8 && lane == 0) {   // (fp8 records leave from the epilogue's registers)
       store_role(sm, 8, n_tiles, n_pairs, first, stride, tile_of,
                  [&](int item, int64_t tile) {
@@ -156,23 +145,14 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
     const int q = warp & 3, h = (warp - 2) >> 2;
     const int r = q * 32 + lane;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    // The fp32 kernels of the two CUDA-core heads (sigma [256], rgb [128,3]) live in shared memory for the whole
-    // kernel -- the dgrad chain has no encoding operand, so xs[] is free.  With 227 KB of shared memory the SM has
-    // no L1 left: reading them with __ldg cost an L2 round trip each (224 per thread and tile).
-    const float* aux = reinterpret_cast<const float*>(packed + kAuxOff);
-    float* head = reinterpret_cast<float*>(sm.xs[0]);
-    for (int i = tid - 64; i < 160; i += kComputeThreads)
-      *(reinterpret_cast<float4*>(head) + i) = __ldg(reinterpret_cast<const float4*>(aux + 12 * 256) + i);
-    named_bar_sync(1, kComputeThreads);
-    const float* wsig = head;
-    const float* wrgb = head + 256;
     uint32_t acc_par[2] = {0, 0};
-    float dsig_keep0 = 0.f, dsig_keep1 = 0.f;
     // fp8 records: one power-of-two scale per call, from max|d_pre| (written by dpre_amax_kernel before this launch)
     const float scale = REC8 ? dz8_scale(__ldg(reinterpret_cast<const uint32_t*>(xbuf) + kXOffAmax), false) : 1.f;
 
-    // tile start: dG = d(rgb_pre) Wc^T (K = 3, CUDA cores) becomes the first A operand
+    KN_PROF_DECL();
+    // tile start: (d rgb_pre, d sigma_pre, 0 ...) is the first A operand (K = 32, tc_layout.cuh BwdProg)
     auto prologue = [&](int64_t pair, int tl) {
+      KN_PROF_BEGIN(t_p);
       const int64_t tile = tile_of(pair, tl);
       const int64_t g = tile * kTileM + r;
       const bool active = tile < n_tiles;
@@ -181,13 +161,10 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
       // fp8 records: the whole chain runs on gradients times the record scale (a power of two: the same mantissas, so
       // every dZ is the same number times 2^k), and the e5m2 records need no multiply in the epilogues
       const float4 dq = REC8 ? make_float4(dp.x * scale, dp.y * scale, dp.z * scale, dp.w * scale) : dp;
-      if (tl == 0) dsig_keep0 = dq.w; else dsig_keep1 = dq.w;
       uint8_t* dz_t = dz + tile * kDB;
-      if (active && !REC8) {
-        const uint4 pk = (h == 0) ? make_uint4(pack_bf16x2(dp.x, dp.y), pack_bf16x2(dp.z, dp.w), 0u, 0u)
-                                  : make_uint4(0u, 0u, 0u, 0u);
-        *reinterpret_cast<uint4*>(dz_t + kDzP + h * kChunkA + r * 16) = pk;
-      }
+      const uint4 pk = (h == 0) ? make_uint4(pack_bf16x2(dq.x, dq.y), pack_bf16x2(dq.z, dq.w), 0u, 0u)
+                                : make_uint4(0u, 0u, 0u, 0u);
+      if (active && !REC8) *reinterpret_cast<uint4*>(dz_t + kDzP + h * kChunkA + r * 16) = pk;   // (dq = dp here)
       if (active && REC8 && h == 0)   // one 16-column chunk: (d rgb_pre, d sigma_pre) * scale, then zeros
         *reinterpret_cast<uint4*>(dz_t + kDz8P + r * 16) =
             make_uint4(pack_e5m2x4(dq.x, dq.y, dq.z, dq.w), 0u, 0u, 0u);
@@ -202,29 +179,15 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
         }
       }
       hs_writable(tl);
-#pragma unroll 2
-      for (int c8 = 0; c8 < 8; ++c8) {
-        const int col = h * 64 + c8 * 8;
-        float x[8];
-        // rgb kernel rows col..col+7: 24 consecutive floats, 16-byte aligned (shared memory, broadcast reads)
-        const float4* w4 = reinterpret_cast<const float4*>(wrgb + col * 3);
-        const float4 a0 = w4[0], a1 = w4[1], a2 = w4[2], a3 = w4[3], a4 = w4[4], a5 = w4[5];
-        x[0] = dq.x * a0.x + dq.y * a0.y + dq.z * a0.z;
-        x[1] = dq.x * a0.w + dq.y * a1.x + dq.z * a1.y;
-        x[2] = dq.x * a1.z + dq.y * a1.w + dq.z * a2.x;
-        x[3] = dq.x * a2.y + dq.y * a2.z + dq.z * a2.w;
-        x[4] = dq.x * a3.x + dq.y * a3.y + dq.z * a3.z;
-        x[5] = dq.x * a3.w + dq.y * a4.x + dq.z * a4.y;
-        x[6] = dq.x * a4.z + dq.y * a4.w + dq.z * a5.x;
-        x[7] = dq.x * a5.y + dq.y * a5.z + dq.z * a5.w;
-        const uint4 pk = make_uint4(pack_bf16x2(x[0], x[1]), pack_bf16x2(x[2], x[3]), pack_bf16x2(x[4], x[5]),
-                                    pack_bf16x2(x[6], x[7]));
-        const int off = (col >> 3) * kChunkA + r * 16;
-        *reinterpret_cast<uint4*>(sm.hs[tl] + off) = pk;   // first A operand and the dG record (warp 10 stores it)
-      }
+      // chunk 0 of the row (h = 0), zeros in chunk 1 (h = 0) and chunks 2, 3 (h = 1): the step reads K = 32, and a
+      // stale NaN pattern times a zero weight would not be zero
+      *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h) * kChunkA + r * 16) = pk;
+      *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h + 1) * kChunkA + r * 16) = make_uint4(0u, 0u, 0u, 0u);
       a_ready_arrive(tl);
+      KN_PROF_END(t_p, 15 + tl * 16);
     };
 
+    KN_PROF_BEGIN(t_c);
     if (first < n_pairs) {
 #pragma unroll 1
       for (int tl = 0; tl < 2; ++tl) prologue(first, tl);
@@ -238,7 +201,6 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
           const bool active = tile < n_tiles;
           uint8_t* out = REC8 ? dz + tile * kDB + kDz8Z0 + zi * kH8Bytes : dz + tile * kDB + kDzZ0 + zi * kHSBytes;
           const uint8_t* mask = rec + tile * kRB + kOffMask + zi * kMaskLayerBytes;
-          const float dsig = tl == 0 ? dsig_keep0 : dsig_keep1;
           // the ReLU' bits (written by the forward, 1 bit per activation) do not depend on the accumulator: fetch
           // this thread's 4 x 32 columns BEFORE waiting for the MMA so that the latency overlaps it
           uint32_t mb[4] = {0u, 0u, 0u, 0u};
@@ -246,22 +208,24 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
             const uint4 mv = __ldg(reinterpret_cast<const uint4*>(mask + h * 2048 + r * 16));
             mb[0] = mv.x; mb[1] = mv.y; mb[2] = mv.z; mb[3] = mv.w;
           }
+          KN_PROF_BEGIN(t_w);
           mbar_wait_cluster(&sm.acc_ready[tl], acc_par[tl]);
+          KN_PROF_END(t_w, 4);
+          KN_PROF_BEGIN(t_e);
           acc_par[tl] ^= 1;
           tc_fence_after();
           if (b + 1 < BwdProg::kSteps) hs_writable(tl);
-          // separately instantiated bodies (a merged loop gets if-converted: the d(sigma) term and its loads
-          // would run on every step)
           const uint32_t tacc = tmem + lane_base + tl * 256;
           const uint4 mbv = make_uint4(mb[0], mb[1], mb[2], mb[3]);
           uint8_t* out8 = (REC8 && active) ? out : nullptr;
-          if (b == 0) epi_dgrad<1, REC8>(tacc, sm.hs[tl], h, r, mbv, dsig, wsig, out8);
-          else if (b + 1 < BwdProg::kSteps) epi_dgrad<2, REC8>(tacc, sm.hs[tl], h, r, mbv, 0.f, nullptr, out8);
-          else epi_dgrad<3, REC8>(tacc, active ? out : nullptr, h, r, mbv, 0.f, nullptr, out8);
+          if (b + 1 < BwdProg::kSteps) epi_dgrad<2, REC8>(tacc, sm.hs[tl], h, r, mbv, out8);
+          else epi_dgrad<3, REC8>(tacc, active ? out : nullptr, h, r, mbv, out8);
           if (b + 1 < BwdProg::kSteps) {
             a_ready_arrive(tl);
+            KN_PROF_END(t_e, 6 + tl * 16 + b);
           } else {
             tc_fence_before();
+            KN_PROF_END(t_e, 6 + tl * 16 + b);
             // (bias gradients = column sums of the dZ tiles are taken by tc_wgrad_kernel, which has them in smem)
             const int64_t next = pair + stride;
             if (next < n_pairs) prologue(next, tl);
@@ -269,6 +233,8 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
         }
       }
     }
+    KN_PROF_END(t_c, 5);
+    if (tid == 64) { KN_PROF_FLUSH(); }
   }
   chain2_teardown(tmem, warp);
 }
@@ -1036,6 +1002,21 @@ int tc_debug_wgrad_timing(unsigned long long* host_out, int n) {
   if (n > 160 * kWProf) n = 160 * kWProf;
   if (cudaMemcpyFromSymbol(host_out, g_wg_prof, (size_t)n * 8) != cudaSuccess) return -1;
   if (cudaMemcpyToSymbol(g_wg_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
+  return n;
+#else
+  (void)host_out; (void)n;
+  return 0;
+#endif
+}
+
+// diagnostic (-DKNERF_TC_TIMING builds only): copy and clear the dgrad kernel's per-CTA cycle counters (the slots of
+// tc_roles.cuh; this translation unit has its own g_tc_prof, so the forward's counters do not mix in)
+int tc_debug_dgrad_timing(unsigned long long* host_out, int n) {
+#ifdef KNERF_TC_TIMING
+  static unsigned long long zeros[160 * 40];
+  if (n > 160 * 40) n = 160 * 40;
+  if (cudaMemcpyFromSymbol(host_out, g_tc_prof, (size_t)n * 8) != cudaSuccess) return -1;
+  if (cudaMemcpyToSymbol(g_tc_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
   return n;
 #else
   (void)host_out; (void)n;

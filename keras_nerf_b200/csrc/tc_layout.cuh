@@ -23,18 +23,22 @@ constexpr int kComputeThreads = 256;
 // ---- forward steps ---------------------------------------------------------------------------------------
 // mlp.py:42-46 applies NO activation between `features` and `rgb_features`, so
 //   G = [h7 W_f + b_f, dir] W_g + b_g = h7 (W_f W_g[:256]) + dir W_g[256:] + (b_f W_g[:256] + b_g)
-// is ONE step from h7 (the product W' = W_f W_g[:256] is formed in fp32 when the weights are packed), and
-// sigma = relu(h7 w_s + b_s) rides along as output column 128 of the same step (N = 144).  Saves the 256 x 256
-// `features` GEMM (11 % of the MACs), its 64 KB/tile activation record and the CUDA-core sigma dot product.
+// is ONE step from h7 (the product W' = W_f W_g[:256] is formed in fp32 when the weights are packed).  Saves the
+// 256 x 256 `features` GEMM (11 % of the MACs) and its 64 KB/tile activation record.  The rgb head after it is linear
+// too (mlp.py:47-48: sigmoid(G W_c + b_c)), so the last step goes from h7 straight to the head pre-activations:
+//   rgb_pre = h7 W''' + PE(dir) D + b'''      W''' = W' W_c [256 x 3],  D = W_g[256:] W_c [27 x 3],  b''' = b' W_c + b_c
+// (formed in fp32 at packing, fold_kernel), and sigma_pre = h7 w_s + b_s rides along as output column 3.  Columns 4..7
+// repeat the four with the bf16 residual of each weight (mlp_tc.cu fold_weight): N = 16, the epilogue adds column
+// pairs and applies the sigmoids and the ReLU.
 // The backward pass never needs the `features` activations either: with X = h7^T dG (one weight-gradient GEMM)
 //   dW_f = X W_g[:256]^T,   dW_g[:256] = W_f^T X + b_f (x) sum(dG),   db_f = sum(dG) W_g[:256]^T
 // (tc_finish_kernel, once per backward call), and the dgrad chain goes from dG to d(h7) through W'^T directly.
 // Reported FLOP counts always use the unfolded 593,408 MAC per sample (SURVEY §8d).
 // step:        0    1..4   5      6,7   8
-// layer:       L0   L1-4   L5     L6,7  [rgb_features o features | sigma]       (rgb head: CUDA cores)
+// layer:       L0   L1-4   L5     L6,7  [rgb o rgb_features o features | sigma]
 struct FwdProg {
   static constexpr int kSteps = 9;
-  static constexpr int kNLast = 144;                 // 128 rgb_features + sigma + 15 zero columns
+  static constexpr int kNLast = 16;                  // (rgb_pre[3], sigma_pre) x (bf16 part, residual), 8 zero columns
   __host__ __device__ static constexpr int layer(int s) { return s; }   // (s < 8; the last step is packed specially)
   __host__ __device__ static constexpr int nk_h(int s) { return s == 0 ? 0 : 8; }   // 32-wide K blocks fed by hs
   __host__ __device__ static constexpr int nk_x(int s) { return (s == 0 || s == 5) ? 2 : (s == 8 ? 1 : 0); }
@@ -49,13 +53,13 @@ struct FwdProg {
 };
 
 // ---- backward (dgrad) steps --------------------------------------------------------------------------------
-// step b:      0                                                  1 .. 7
-// computes:    dZ7 = (dG W'^T + dsigma Ws^T) * [h7>0]             dZ_{7-b} = (dZ_{8-b} W_{8-b}^T) * [h_{7-b}>0]
-// weights:     W' = W_f W_g[:256] (K = 128 rgb_features columns)  layer 7 .. layer 1   (rows < 256 of the Keras kernel)
+// step b:      0                                                          1 .. 7
+// computes:    dZ7 = (d(rgb_pre) W'''^T + dsigma Ws^T) * [h7>0]           dZ_{7-b} = (dZ_{8-b} W_{8-b}^T) * [h_{7-b}>0]
+// weights:     [W''' | Ws | 0] (K = 32: d rgb_pre[3], d sigma_pre, zeros)  layer 7 .. layer 1   (rows < 256 of the Keras kernel)
 struct BwdProg {
   static constexpr int kSteps = 8;
   __host__ __device__ static constexpr int layer(int b) { return 8 - b; }            // (b >= 1)
-  __host__ __device__ static constexpr int nk_h(int b) { return b == 0 ? 4 : 8; }
+  __host__ __device__ static constexpr int nk_h(int b) { return b == 0 ? 1 : 8; }
   __host__ __device__ static constexpr int nk_x(int) { return 0; }
   __host__ __device__ static constexpr int N(int) { return 256; }
   static constexpr bool kHasBias = false;
@@ -97,14 +101,13 @@ struct PairLayout {
 };
 
 // ---- packed weight buffer ------------------------------------------------------------------------------------
-// [fp32 side table][fp32 folded kernel W' + bias][forward blob][dgrad blob].  The side table holds 16-byte aligned copies (the Keras flat buffer
-// is not aligned: the 1-wide sigma bias shifts everything after it): bias[l] at l*256 (l = 0..11), sigma kernel
-// [256] at 12*256, rgb kernel [128,3] at 13*256.
-constexpr int kAuxOff = 0;
-constexpr int kAuxFloats = 12 * 256 + 256 + 512;
-constexpr int kFoldOff = kAuxOff + kAuxFloats * 4;           // fp32 W' = W_f W_g[:256] [256,128], then its bias [128]
-constexpr int kFoldFloats = 256 * 128 + 128;
-constexpr int kFwdPairOff = kFoldOff + kFoldFloats * 4;
+// [fp32 folded kernel W' + bias][fp32 folded heads][forward blob][dgrad blob].
+constexpr int kFoldOff = 0;                                  // fp32 W' = W_f W_g[:256] [256,128], then its bias [128]
+constexpr int kFoldFloats = 256 * 128 + 128;                 //   (tc_finish_kernel: the rgb kernel's gradient)
+constexpr int kHeadOff = kFoldOff + kFoldFloats * 4;         // fp32 [289][4]: row k < 256 (W'''[k], w_s[k]), 256 + i
+constexpr int kHeadRows = 289;                               //   (D[i], 0), 288 (b''', b_s) -- the B operands of forward
+constexpr int kHeadFloats = 320 * 4;                         //   step 8 and dgrad step 0 (padded: the blobs start
+constexpr int kFwdPairOff = kHeadOff + kHeadFloats * 4;      //   128-byte aligned)
 constexpr int kBwdPairOff = kFwdPairOff + PairLayout<FwdProg>::kBytes;
 constexpr int kPackedBytes = kBwdPairOff + PairLayout<BwdProg>::kBytes;
 
@@ -192,7 +195,6 @@ struct ChainSmem {
   uint8_t hs[2][kHSBytes];
   uint8_t xs[2][kXSBytes];
   uint8_t stage[kNumStages2][kStageBytes2];
-  float part[kTileM][4];
   uint64_t full[kNumStages2], empty[kNumStages2], a_ready[2], acc_ready[2], st_ready[2], st_done[2];
   uint32_t tmem_base;
   uint32_t items_issued;      // ordered mode: ring items whose MMAs have been issued (the two issuers take turns)

@@ -141,6 +141,17 @@ __device__ __forceinline__ void tmem_ld32_wait(uint32_t (&r)[32]) {
                :: "memory");
 }
 
+// 8 consecutive columns (the forward's last step: the head pre-activations as hi + lo parts)
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr));
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
   uint32_t r[32];
   asm volatile(

@@ -14,14 +14,16 @@ using namespace tc;
 // ---- optional in-kernel timing (build with -DKNERF_TC_TIMING; off by default, zero cost) ----------------------
 // per CTA, clock64() cycles: slot 0 producer waits for a free stage | 1 MMA thread waits for the A operand |
 // 2 MMA thread waits for a weight stage | 3 MMA thread total | 4 compute warp 2 waits for an accumulator |
-// 5 compute total | 6.. per-step epilogue cycles of compute warp 2 (16 + s for tile slot 1)
+// 5 compute total | 6.. per-step epilogue cycles of compute warp 2 (16 + s for tile slot 1) | 15, 31: the dgrad
+// kernel's tile prologue (tile slot 0, 1)
 #ifdef KNERF_TC_TIMING
 static __device__ unsigned long long g_tc_prof[160][40];
 // counters live in the thread's local memory (L1) and are flushed once at the end of the role
 #define KN_PROF_DECL() unsigned long long kn_prof[40]; for (int kn_i = 0; kn_i < 40; ++kn_i) kn_prof[kn_i] = 0ull
 #define KN_PROF_BEGIN(var) const long long var = clock64()
 #define KN_PROF_END(var, slot) kn_prof[slot] += (unsigned long long)(clock64() - var)
-#define KN_PROF_FLUSH() for (int kn_i = 0; kn_i < 40; ++kn_i) if (kn_prof[kn_i]) g_tc_prof[blockIdx.x][kn_i] += kn_prof[kn_i]
+// (atomic: both MMA issuers of a leader CTA flush into the same slots)
+#define KN_PROF_FLUSH() for (int kn_i = 0; kn_i < 40; ++kn_i) if (kn_prof[kn_i]) atomicAdd(&g_tc_prof[blockIdx.x][kn_i], kn_prof[kn_i])
 #else
 #define KN_PROF_DECL()
 #define KN_PROF_BEGIN(var)

@@ -120,8 +120,7 @@ __device__ __forceinline__ void mma2_role(ChainSmem& sm, uint32_t tmem, uint32_t
                                           int64_t first, int64_t stride) {
   using PL = PairLayout<Prog>;
   uint32_t it = 0, a_par = 0;   // bit tl of a_par = parity of a_ready[tl]
-  uint32_t step_no = 0;   // GEMM steps before the current one; every step has >= 2 items, so both issuers take
-                          // part in every (step, slot)
+  uint32_t step_no = 0;   // GEMM steps before the current one
   // descriptor templates: K-major SWIZZLE_NONE, SBO = 128 B, LBO = rows * 16 B; only the 14-bit start address varies
   const uint32_t stage0 = smem_u32(sm.stage[0]);
   KN_PROF_DECL();
@@ -143,17 +142,19 @@ __device__ __forceinline__ void mma2_role(ChainSmem& sm, uint32_t tmem, uint32_t
         const uint32_t d_tmem = tmem + tl * 256;
         volatile uint32_t* issued = &sm.items_issued;
         volatile uint32_t* fi = &sm.first_issued[tl];
+        // Both threads wait for the A operand even when a step has only one item (dgrad step 0) and this thread none
+        // of it: its acc_ready commit below must not arrive before the compute warps have taken the previous phase.
+        KN_PROF_BEGIN(t_a);
+        mbar_wait_cluster(&sm.a_ready[tl], (a_par >> tl) & 1);
+        KN_PROF_END(t_a, 1);
+        tc_fence_after();
         bool started = false;
 #pragma unroll 1
         for (int i = 0; i < ns; ++i, ++it) {
           if ((it & 1u) != p) continue;
           if (!started) {   // this thread's first item of the step
             started = true;
-            KN_PROF_BEGIN(t_a);
-            mbar_wait_cluster(&sm.a_ready[tl], (a_par >> tl) & 1);
             if (!ordered && i > 0) { while (*fi <= step_no) {} }   // item 0 (accumulate = 0) is the other thread's
-            KN_PROF_END(t_a, 1);
-            tc_fence_after();
           }
           const uint32_t slot = it % kNumStages2, ph = (it / kNumStages2) & 1;
           KN_PROF_BEGIN(t_f);

@@ -124,7 +124,8 @@ umma_selftest2_kernel(const uint8_t* __restrict__ a_blob, const uint8_t* __restr
     float v[32];
     tmem_ld32(tmem + ((uint32_t)(warp * 32) << 16) + c0, v);
 #pragma unroll
-    for (int i = 0; i < 32; ++i) d_out[(size_t)row * N + c0 + i] = v[i];
+    for (int i = 0; i < 32; ++i)
+      if (c0 + i < N) d_out[(size_t)row * N + c0 + i] = v[i];   // (N = 16: the load also returns 16 unused columns)
   }
   tc_fence_before();
   cluster_sync_all();
@@ -137,8 +138,8 @@ using namespace knerf;
 
 extern "C" int knerf_selftest_umma2(const void* a_blob, const void* b_blob, int N, int K, float* d_out, void* stream) {
   KN_CHECK_ARG(a_blob && b_blob && d_out, "knerf_selftest_umma2: null pointer");
-  KN_CHECK_ARG(N % 32 == 0 && N >= 32 && N <= 256 && K % 16 == 0 && K >= 16 && K <= 256,
-               "knerf_selftest_umma2: N in 32..256 step 32, K in 16..256 step 16");
+  KN_CHECK_ARG(N % 16 == 0 && N >= 16 && N <= 256 && K % 16 == 0 && K >= 16 && K <= 256,
+               "knerf_selftest_umma2: N in 16..256 step 16, K in 16..256 step 16");
   const size_t smem = (size_t)(128 + N / 2) * K * 2;
   KN_CUDA(cudaFuncSetAttribute(umma_selftest2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   umma_selftest2_kernel<<<2, 128, smem, (cudaStream_t)stream>>>((const uint8_t*)a_blob, (const uint8_t*)b_blob, N, K,
