@@ -270,6 +270,32 @@ int knerf_train_chunk_dp(const knerf_config* cfg, const float* params_coarse, co
                          float* image_c, float* image_f, void* workspace, int64_t workspace_bytes,
                          void* stream, knerf_comm* comm, void* comm_stream, int reduce);
 
+/* ---- mesh export: isosurface of a scalar grid (NeRF.extract_mesh; no counterpart in the reference) ---------------
+ * Marching tetrahedra on the Kuhn split: every cell of field[nx,ny,nz] (index (i*ny + j)*nz + k, x slowest) is cut into
+ * the 6 tets 0 -> e_a -> e_a+e_b -> (1,1,1), one per axis permutation (a,b,c) in the order 012, 021, 102, 120, 201, 210.
+ * The split is the same in every cell, so the surface is watertight; there are no ambiguous cases.
+ *  - a grid point is inside when f > iso (strict); the edge p -> p+delta (delta in 100, 010, 001, 110, 101, 011, 111, in
+ *    that order) carries a vertex when exactly one endpoint is inside, at t = (iso - f_p) / (f_q - f_p),
+ *    v = origin + spacing * (p + t*delta) (fp32), with the normal = -normalise(interpolated central-difference gradient,
+ *    one-sided on the grid faces), pointing towards decreasing f; a zero gradient gives a zero normal.
+ *  - a tet with 1 or 3 corners inside gives one triangle; 2 inside (a,b) and 2 outside (c,d) give the quad
+ *    ac, ad, bd, bc split along ac-bd.  Counter-clockwise seen from outside: the normal of the triangle through the
+ *    EDGE MIDPOINTS points from the inside corners' centroid towards the outside ones'.
+ *  - vertices in the order (grid point, delta); triangles in the order (cell, tet, triangle).  No atomics: two runs
+ *    give the same bytes.
+ * Usage: the count pass writes counts[2] = {V, T} (DEVICE int64); the caller reads them back, allocates, then calls the
+ * emit pass with the same field, iso and workspace (untouched in between).  vertices[V,3], normals[V,3] (may be NULL),
+ * triangles[T,3] int32; nothing is written at or beyond max_vertices / max_triangles.  max_vertices >= 2^31 is
+ * KNERF_ERR_UNSUPPORTED (int32 indices).  Workspace: knerf_isosurface_workspace_bytes, 256-byte aligned, about
+ * 5 bytes per grid point.  nx, ny, nz >= 2.                                                                        */
+int64_t knerf_isosurface_workspace_bytes(int nx, int ny, int nz);
+int knerf_isosurface_count(const float* field, int nx, int ny, int nz, float iso, int64_t* counts, void* workspace,
+                           int64_t workspace_bytes, void* stream);
+int knerf_isosurface_emit(const float* field, int nx, int ny, int nz, float iso, const float* origin_host,
+                          const float* spacing_host, float* vertices, float* normals, int32_t* triangles,
+                          int64_t max_vertices, int64_t max_triangles, void* workspace, int64_t workspace_bytes,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -76,6 +76,9 @@ SIGNATURES = {
     "knerf_allreduce_grads": (_I, [_P, _P, _L, _P]),
     "knerf_train_chunk_dp": (_I, [_CFG, _P, _P, _P, _P, _P, _P, _P, _P, _L, _P, _U64, _I, _I, _I, _F,
                                   _P, _P, _P, _P, _P, _P, _L, _P, _P, _P, _I]),
+    "knerf_isosurface_workspace_bytes": (_L, [_I, _I, _I]),
+    "knerf_isosurface_count": (_I, [_P, _I, _I, _I, _F, _P, _P, _L, _P]),
+    "knerf_isosurface_emit": (_I, [_P, _I, _I, _I, _F, _P, _P, _P, _P, _P, _L, _L, _P, _L, _P]),
     "knerf_debug_tc_timing": (_I, [_P, _I]),
     "knerf_debug_wgrad_timing": (_I, [_P, _I]),
     "knerf_debug_dgrad_timing": (_I, [_P, _I]),

@@ -391,6 +391,126 @@ class NeRF:
             fine['weights'] = st.gather_rows(fw, n, 0, sizes=sizes).reshape(B, H, W, S)
         return coarse, fine
 
+    # ---- mesh export (no counterpart in the reference) ------------------------------------------
+    def _network(self, network):
+        if not self._compiled:
+            raise RuntimeError("compile() the model first (the bf16 mode needs its packed weights)")
+        if network not in ("coarse", "fine"):
+            raise ValueError(f"network must be 'coarse' or 'fine', got {network!r}")
+        return (self.coarse if network == "coarse" else self.fine).params, self._packed_ptr(network)
+
+    def _query_rows(self, rows_wanted, S):
+        """rays per knerf_mlp_forward call: up to 2^22 samples, halved while the scratch exceeds 1 GiB (the fp32 modes
+        keep whole activation rows), at least one ray; -> (rays, workspace)"""
+        lib = _lib.load()
+        samples = 1 << 22
+        while samples > S and lib.knerf_workspace_bytes(C.byref(self.cfg), samples, self._prec_flags, 0) > (1 << 30):
+            samples //= 2
+        R = max(1, min(rows_wanted, samples // S))
+        need = lib.knerf_workspace_bytes(C.byref(self.cfg), R * S, self._prec_flags, 0)
+        if need < 0:
+            raise _lib.KnerfError("knerf_workspace_bytes: " + lib.knerf_last_error().decode())
+        return R, torch.empty(need, dtype=torch.uint8, device=self.device)
+
+    def _forward(self, params, packed, o, d, t, S, out, ws):
+        _lib.call("knerf_mlp_forward", C.byref(self.cfg), _lib.ptr(params), packed, _lib.ptr(o), _lib.ptr(d),
+                  _lib.ptr(t), o.shape[0], S, self._prec_flags, 0, _lib.ptr(out), ws.data_ptr(), ws.numel(),
+                  _lib.stream())
+
+    @staticmethod
+    def _grid_frame(resolution, bound):
+        """(n[3], origin[3], spacing[3]) of the lattice: `bound` a scalar b (the cube [-b, b]^3) or (min[3], max[3]);
+        `resolution` an int or three; point i of axis a at origin[a] + spacing[a] * i (fp32)"""
+        n = np.broadcast_to(np.asarray(resolution, dtype=np.int64), (3,)).copy()
+        if (n < 2).any():
+            raise ValueError(f"resolution must be >= 2 per axis, got {resolution!r}")
+        if np.ndim(bound) == 0:
+            lo, hi = np.full(3, -float(bound), np.float32), np.full(3, float(bound), np.float32)
+        else:
+            lo, hi = (np.broadcast_to(np.asarray(b, dtype=np.float32), (3,)).copy() for b in bound)
+        if not (np.isfinite(lo).all() and np.isfinite(hi).all() and (hi > lo).all()):
+            raise ValueError(f"bound must be finite with min < max per axis, got {bound!r}")
+        spacing = ((hi - lo) / (n - 1).astype(np.float32)).astype(np.float32)
+        return n, lo, spacing
+
+    def density_grid(self, resolution=256, bound=1.5, network="fine", samples_per_call=None):
+        """sigma of `network` on a regular lattice -> CUDA tensor [nx, ny, nz] (x slowest, z fastest).  The lattice is
+        evaluated as rays along +z through the fused forward in the model's precision: one ray per (x, y) column,
+        origin (x_i, y_j, z_0), direction (0, 0, 1), depths k * spacing_z.  The direction does not change sigma.
+        `samples_per_call` (default: up to 2^22 within 1 GiB of scratch) only bounds memory; it does not change a bit."""
+        params, packed = self._network(network)
+        n, lo, spacing = self._grid_frame(resolution, bound)
+        nx, ny, nz = (int(v) for v in n)
+        dev = self.device
+        f32 = lambda a: torch.as_tensor(a, dtype=torch.float32, device=dev)  # noqa: E731
+        axis = lambda a: f32(lo[a]) + torch.arange(int(n[a]), dtype=torch.float32, device=dev) * f32(spacing[a])  # noqa
+        xs, ys = axis(0), axis(1)
+        tz = torch.arange(nz, dtype=torch.float32, device=dev) * f32(spacing[2])
+        cols = nx * ny
+        R, ws = self._query_rows(cols, nz)
+        if samples_per_call is not None:
+            R = max(1, min(R, int(samples_per_call) // nz))
+        grid = torch.empty((nx, ny, nz), dtype=torch.float32, device=dev)
+        flat = grid.view(cols, nz)
+        d_all = torch.zeros((R, 3), dtype=torch.float32, device=dev)
+        d_all[:, 2] = 1.0
+        t_all = tz.expand(R, nz).contiguous()
+        out = torch.empty((R, nz, 4), dtype=torch.float32, device=dev)
+        with torch.cuda.device(dev):
+            for s in range(0, cols, R):
+                e = min(cols, s + R)
+                c = torch.arange(s, e, device=dev)
+                o = torch.stack([xs[c // ny], ys[c % ny], torch.full((e - s,), float(lo[2]), device=dev)], -1)
+                self._forward(params, packed, o, d_all[:e - s], t_all[:e - s], nz, out, ws)
+                flat[s:e] = out[:e - s, :, 3]
+        return grid
+
+    def vertex_colors(self, vertices, normals, network="fine"):
+        """rgb of `network` at every vertex, looking at the surface along its normal: o = v, d = -n (a zero normal
+        looks along -z), one sample at t = 0 -> CUDA tensor [V, 3]"""
+        params, packed = self._network(network)
+        v = _lib.dev(vertices, self.device).reshape(-1, 3)
+        d = -_lib.dev(normals, self.device).reshape(-1, 3)
+        d[(d == 0).all(-1)] = torch.tensor([0.0, 0.0, -1.0], device=self.device)
+        V = v.shape[0]
+        rgb = torch.empty((V, 3), dtype=torch.float32, device=self.device)
+        if V == 0:
+            return rgb
+        R, ws = self._query_rows(V, 1)
+        t = torch.zeros((R, 1), dtype=torch.float32, device=self.device)
+        out = torch.empty((R, 1, 4), dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.device):
+            for s in range(0, V, R):
+                e = min(V, s + R)
+                self._forward(params, packed, v[s:e], d[s:e].contiguous(), t[:e - s], 1, out, ws)
+                rgb[s:e] = out[:e - s, 0, :3]
+        return rgb
+
+    def extract_mesh(self, resolution=256, threshold=50.0, bound=1.5, network="fine", colors=True, close=True):
+        """Triangle mesh of the level set sigma = `threshold` of `network` on a `resolution` lattice over `bound` (see
+        density_grid), by marching tetrahedra (utils/mesh.py).  close=True pads the grid with one layer of zeros, so a
+        surface that leaves the box is capped on its faces and the mesh stays closed.  Returns a dict of CUDA tensors:
+        vertices [V,3], normals [V,3] (outward: towards decreasing sigma), colors [V,3] (or None), faces [T,3] int32,
+        and `seconds`: wall time of each stage (grid, isosurface, colors), each ended by a device synchronise."""
+        import time
+        from ...utils.mesh import marching_tetrahedra
+        t0 = time.perf_counter()
+        grid = self.density_grid(resolution, bound, network)
+        _, origin, spacing = self._grid_frame(resolution, bound)
+        if close:
+            grid = torch.nn.functional.pad(grid[None], (1, 1, 1, 1, 1, 1))[0]
+            origin = (origin - spacing).astype(np.float32)
+        torch.cuda.synchronize(self.device)
+        t1 = time.perf_counter()
+        v, n, f = marching_tetrahedra(grid, threshold, origin, spacing)
+        torch.cuda.synchronize(self.device)
+        t2 = time.perf_counter()
+        rgb = self.vertex_colors(v, n, network) if colors else None
+        torch.cuda.synchronize(self.device)
+        t3 = time.perf_counter()
+        return {"vertices": v, "normals": n, "colors": rgb, "faces": f,
+                "seconds": {"grid": t1 - t0, "isosurface": t2 - t1, "colors": t3 - t2}}
+
     # ---- metrics (nerf.py:306-330) ------------------------------------------------------------
     def update_and_return_metrics(self, images, coarse_images, fine_images, coarse_loss, fine_loss):
         """coarse_loss / fine_loss: floats, or ONE device tensor [2] (then `fine_loss` is None) that is read back
