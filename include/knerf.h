@@ -104,6 +104,25 @@ int knerf_generate_rays(const float* c2w_host, int H, int W, float focal, float 
                         int n_samples, const float* u, uint64_t seed, float* o, float* d, float* t,
                         void* stream);
 
+/* ---- random ray batches drawn across all training views (NeRF's N_rand; no counterpart in the reference) ----------
+ * images[n_img, H, W, C] (C >= 3; rgb in channels 0..2, e.g. ImageLoader's RGBA fp32) and c2w[n_img, 4, 4] (DEVICE):
+ * the prepared training views.  Pixel id p = (img*H + y)*W + x over P = n_img*H*W pixels.  Epoch `epoch` of key
+ * `perm_seed` visits every pixel once, in the order of a bijection pi of [0, P) computed in the kernel (no buffer):
+ * a 4-round balanced Feistel network on the smallest even bit width b >= 2 with 2^b >= P, cycle-walked until the
+ * value is < P.  Round r maps (L, R) -> (R, L ^ (mix(R ^ k_r) & mask)), mix = the splitmix64 finaliser,
+ * k_r = mix(mix(perm_seed) ^ (epoch*0x9E3779B97F4A7C15 + 0xD1B54A32D192ED03)) + r*0x9E3779B97F4A7C15, and the
+ * output is (L << b/2) | R.  Any window of any epoch is computed independently, so data-parallel ranks take disjoint
+ * windows of the same epoch without communicating.
+ * This call writes rays first .. first+R-1 of that order: pixel p_j = pi(first + j) gives o[j,3], d[j,3] and
+ * t[j, n_samples] -- the same bits knerf_generate_rays writes for pixel p_j of its view given the same uniforms --
+ * and target[j,3] = images[p_j, 0..2]; pixel[j] = p_j (int64, may be NULL).  u: [R*n_samples] uniforms or NULL (then
+ * Philox(seed) at counter j*n_samples + k, the batch-local convention of knerf_generate_rays).
+ * KNERF_ERR_INVALID: null pointer, n_img/H/W/n_samples <= 0, C < 3, first < 0, first + R > P.                  */
+int knerf_generate_ray_batch(const float* images, int n_img, int H, int W, int C, const float* c2w, float focal,
+                             float near_, float far_, int n_samples, uint64_t perm_seed, uint64_t epoch,
+                             int64_t first, int64_t R, const float* u, uint64_t seed, float* o, float* d, float* t,
+                             float* target, int64_t* pixel, void* stream);
+
 /* tf.random.uniform stand-in: n floats, multiples of 2^-24 in [0,1), Philox4x32-10(seed, offset) */
 int knerf_uniform(float* out, int64_t n, uint64_t seed, uint64_t offset, void* stream);
 

@@ -45,6 +45,8 @@ SIGNATURES = {
     "knerf_launch_count": (_U64, []),
     "knerf_device_supports_bf16": (_I, []),
     "knerf_generate_rays": (_I, [_P, _I, _I, _F, _F, _F, _I, _P, _U64, _P, _P, _P, _P]),
+    "knerf_generate_ray_batch": (_I, [_P, _I, _I, _I, _I, _P, _F, _F, _F, _I, _U64, _U64, _L, _L, _P, _U64,
+                                      _P, _P, _P, _P, _P, _P]),
     "knerf_uniform": (_I, [_P, _L, _U64, _U64, _P]),
     "knerf_positional_encoding": (_I, [_P, _L, _I, _I, _P, _I, _P]),
     "knerf_encode_position_and_directions": (_I, [_P, _P, _P, _L, _I, _I, _I, _P, _I, _P, _I, _P]),

@@ -46,3 +46,27 @@ class RaysGenerator:
             _lib.call("knerf_generate_rays", c2w.ctypes.data, H, W, self.focal_length, self.near, self.far, N,
                       _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t), _lib.stream())
         return o, d, t
+
+
+def generate_ray_batch(images, poses, focal, near, far, n_sample, perm_seed, epoch, first, n_rays, u=None, seed=None,
+                       with_pixel=False):
+    """`knerf_generate_ray_batch`: rays first .. first+n_rays-1 of epoch `epoch` of the permutation keyed by
+    `perm_seed` over every pixel of the view cache `images` [n_img, H, W, C] (CUDA fp32, C >= 3) with poses
+    [n_img, 4, 4].  Returns (target[n,3], o[n,3], d[n,3], t[n,N]) (+ pixel[n] int64, id (img*H + y)*W + x, when
+    `with_pixel`).  The jitter comes from Philox(seed), a new seed per call unless given, or from `u` [n, N]."""
+    n_img, H, W, C = images.shape
+    device = images.device
+    N = int(n_sample)
+    with torch.cuda.device(device):
+        mk = lambda *s: torch.empty(s, dtype=torch.float32, device=device)  # noqa: E731
+        target, o, d, t = mk(n_rays, 3), mk(n_rays, 3), mk(n_rays, 3), mk(n_rays, N)
+        pixel = torch.empty(n_rays, dtype=torch.int64, device=device) if with_pixel else None
+        if u is not None:
+            u = _lib.dev(u, device).reshape(n_rays, N)
+        if seed is None:
+            seed = next(_seed_counter)
+        _lib.call("knerf_generate_ray_batch", _lib.ptr(images), n_img, H, W, C, _lib.ptr(poses), float(focal),
+                  float(near), float(far), N, int(perm_seed) & 0xFFFFFFFFFFFFFFFF, int(epoch) & 0xFFFFFFFFFFFFFFFF,
+                  int(first), int(n_rays), _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t),
+                  _lib.ptr(target), None if pixel is None else pixel.data_ptr(), _lib.stream())
+    return (target, o, d, t, pixel) if with_pixel else (target, o, d, t)

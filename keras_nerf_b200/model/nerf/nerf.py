@@ -180,6 +180,14 @@ class NeRF:
     # ---- compile (nerf.py:78-173) -------------------------------------------------------------
     def compile(self, optimizer, loss, batch_size, image_height, image_width, ray_chunks, white_background=False,
                 is_training=True, **kwargs):
+        """nerf.py:78-173.  Keyword extensions: `fuse_chunks` (below) and `ray_batch`.
+
+        ray_batch=N > 0: the training step takes N rays drawn across all views (data.loader.RayBatchDataset), so
+        train_step((targets[N,3], (o[N,3], d[N,3], t[N,Nc]))) / accumulate_gradients take a flat ray batch, while
+        batch_size / image_height / image_width keep describing what predict_and_render_images, test_step and the
+        monitor render.  `ray_chunks` must divide N (checked like it is against the number of rays of an image batch)
+        and `fuse_chunks` applies to the N rays.  The logs keep their keys: the PSNR is that of the batch MSE and the
+        SSIM is NaN (a ray batch has no 11x11 window)."""
         self.run_eagerly = bool(kwargs.get("run_eagerly", False))
         self.optimizer, self.loss = optimizer, loss
         # The fused kernels implement the loss of the reference scripts: MeanSquaredError (train_single.py:127) or
@@ -200,18 +208,27 @@ class NeRF:
         assert self.num_rays % self.ray_chunks == 0, \
             f'ray_chunks {self.ray_chunks} must be a divisor of the number of rays {self.num_rays}'   # nerf.py:100
         self.sequential_chunks = self.num_rays // self.ray_chunks
+        self.ray_batch = int(kwargs.get("ray_batch", 0) or 0)
+        if self.ray_batch:
+            # the training step's own chunking; rendering keeps the chunks of the image batch
+            self._train_rays = self.ray_batch
+            train_rc = min(ray_chunks, self.ray_batch)
+            assert self.ray_batch % train_rc == 0, \
+                f'ray_chunks {train_rc} must be a divisor of the number of rays {self.ray_batch}'
+        else:
+            self._train_rays, train_rc = self.num_rays, self.ray_chunks
         # `ray_chunks` exists in the reference to bound TensorFlow's activation memory (train.py:46, 1024 by default); the
         # chunks of a step are independent and their gradients are summed, so executing k of them in one call gives the
         # same step (up to the fp32 summation order; with random fine-sample draws, other draws of the same
         # distribution) with fewer, larger launches -- 0.82 -> 1.22 M rays/s on a 160,000-ray step between 1,000- and
         # 32,000-ray calls.  Off unless asked for: fuse_chunks="auto" (calls of up to 32,768 rays) or an int k.
         fuse = kwargs.get("fuse_chunks", None)
-        k, nch = 1, self.sequential_chunks
+        k, nch = 1, self._train_rays // train_rc
         if fuse in ("auto", True):
-            k = max(j for j in range(1, nch + 1) if nch % j == 0 and (j == 1 or j * self.ray_chunks <= 32768))
+            k = max(j for j in range(1, nch + 1) if nch % j == 0 and (j == 1 or j * train_rc <= 32768))
         elif isinstance(fuse, int) and not isinstance(fuse, bool) and fuse > 1:
             k = max(j for j in range(1, min(fuse, nch) + 1) if nch % j == 0)
-        self._train_ray_chunks, self._train_chunks = self.ray_chunks * k, nch // k
+        self._train_ray_chunks, self._train_chunks = train_rc * k, nch // k
         self.device = self.device or _lib.default_device()
         self.nerf_utils = NeRFUtils(self.batch_size, self.image_height, self.image_width, self.ray_chunks,
                                     self.pos_emb_xyz, self.pos_emb_dir, self.white_background, device=self.device,
@@ -273,6 +290,11 @@ class NeRF:
         lib = _lib.load()
         rows = (self._train_ray_chunks if self.is_training else self.ray_chunks) * (self.n_coarse + self.n_fine)
         need = lib.knerf_workspace_bytes(C.byref(self.cfg), rows, self._prec_train, int(self.is_training))
+        if self.ray_batch and self.is_training and need >= 0:
+            # the training chunk of a ray batch can be smaller than the render chunk
+            render = lib.knerf_workspace_bytes(C.byref(self.cfg), self.ray_chunks * (self.n_coarse + self.n_fine),
+                                               self._prec_train, 0)
+            need = max(need, render) if render >= 0 else render
         if need < 0:
             raise _lib.KnerfError("knerf_workspace_bytes: " + lib.knerf_last_error().decode())
         self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
@@ -297,9 +319,9 @@ class NeRF:
         self.fine_ssim_metric = Mean(name="fine_ssim")
 
     # ---- helpers ------------------------------------------------------------------------------
-    def _flat_rays(self, rays):
+    def _flat_rays(self, rays, n=None):
         o, d, t = (_lib.dev(r, self.device) for r in rays)
-        n = self.num_rays
+        n = self.num_rays if n is None else n
         return o.reshape(n, 3), d.reshape(n, 3), t.reshape(n, self.n_coarse)
 
     def _u(self, u_fine, n):
@@ -534,11 +556,12 @@ class NeRF:
     def accumulate_gradients(self, images, rays, u_fine=None, seed=None, want_images=True, reduce=True):
         """The chunk loop of train_step (nerf.py:351-421): fills the two gradient accumulators and the loss
         accumulators; returns (coarse_images, fine_images) [B,H,W,3] (or None).  With a multi-rank strategy and
-        reduce=True the accumulators hold the cross-replica SUM when the enqueued work completes."""
+        reduce=True the accumulators hold the cross-replica SUM when the enqueued work completes.  Compiled with
+        `ray_batch`: images are targets [N,3] of a flat ray batch and the returned images are [N,3]."""
         images = _lib.dev(images, self.device)[..., :3]                           # nerf.py:335
-        n = self.num_rays
+        n = self._train_rays
         target = images.reshape(n, 3).contiguous()
-        o, d, t = self._flat_rays(rays)
+        o, d, t = self._flat_rays(rays, n)
         u = self._u(u_fine, n)
         ci = torch.empty((n, 3), dtype=torch.float32, device=self.device) if want_images else None
         fi = torch.empty((n, 3), dtype=torch.float32, device=self.device) if want_images else None
@@ -568,6 +591,8 @@ class NeRF:
         B, H, W = self.batch_size, self.image_height, self.image_width
         if not want_images:
             return None, None
+        if self.ray_batch:
+            return ci, fi
         return ci.view(B, H, W, 3), fi.view(B, H, W, 3)
 
     def apply_gradients(self):
@@ -603,6 +628,8 @@ class NeRF:
                 logging.warning('Fine Gradient is zero')
         self.apply_gradients()
         imgs = _lib.dev(images, self.device)[..., :3]
+        if self.ray_batch:      # one [1, 1, N] "image": the PSNR of the batch MSE, no SSIM window
+            imgs, ci, fi = (x.reshape(1, 1, self.ray_batch, 3) for x in (imgs, ci, fi))
         return self.update_and_return_metrics(imgs, ci, fi, losses, None)   # losses + metrics: one host read
 
     def test_step(self, inputs, u_fine=None, seed=None):

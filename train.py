@@ -3,7 +3,11 @@
 Multi-GPU: launch with `torchrun --nproc-per-node N train.py ...` -- one process per GPU replaces
 tf.distribute.MirroredStrategy (train.py:75): the loader batches `batch_size x N` views exactly like the
 reference's global batch (train.py:84-87) and each rank trains on its own `batch_size` views; the accumulated MLP
-gradients are SUM-all-reduced over NCCL before the two Adam steps."""
+gradients are SUM-all-reduced over NCCL before the two Adam steps.
+
+--ray_batch N trains on N random rays per replica and step, drawn across all training views (an epoch visits every
+pixel once; data.loader.RayBatchDataset) instead of --batch_size whole views; validation and the monitor still
+render --batch_size whole views.  Under torchrun the ranks take disjoint windows of the same epoch order."""
 import argparse
 import logging
 import os
@@ -72,26 +76,32 @@ def main(argv=None, multi_gpu=True):
                              "'off', or a count.  The chunks of a step are independent, so the step is the same")
     parser.add_argument('--records', type=str, default='fp8', choices=['fp8', 'bf16'],
                         help='bf16 mode: format of the activation / gradient records kept for the weight gradients')
+    parser.add_argument('--ray_batch', type=int, default=0,
+                        help='train on this many random rays per replica and step, drawn across all training views '
+                             '(0: --batch_size whole views per step, the reference\'s pipeline)')
     args = parser.parse_args(argv)
     logging.basicConfig(level=logging.DEBUG if args.verbose else logging.INFO,
                         format='%(asctime)s | %(name)s | %(levelname)s | %(message)s')
     logging.info(args)
 
-    strategy, replicas = None, 1
+    strategy, replicas, rank = None, 1, 0
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         from keras_nerf_b200.distributed import RayShardedStrategy
         strategy = RayShardedStrategy()
-        replicas = strategy.num_replicas_in_sync
+        replicas, rank = strategy.num_replicas_in_sync, strategy.rank
     print('Number of devices: {}'.format(replicas))
 
     loader = DatasetLoader(args.data_dir, args.white_bg)
     datasets = loader.load_dataset(batch_size=args.batch_size * replicas, image_width=args.img_wh,
                                    image_height=args.img_wh, near=args.near, far=args.far,
-                                   n_sample=args.num_coarse_samples)
+                                   n_sample=args.num_coarse_samples, ray_batch=args.ray_batch, rank=rank,
+                                   world=replicas)
     if strategy is not None:
-        for ds in datasets:
+        # a ray-batch train split is already this rank's share
+        split = 1 if args.ray_batch else 0
+        for ds in datasets[split:]:
             ds._rng.seed(42)                                 # every rank walks the same shuffled order
-        datasets = [ReplicaBatches(ds, strategy, args.batch_size) for ds in datasets]
+        datasets = datasets[:split] + [ReplicaBatches(ds, strategy, args.batch_size) for ds in datasets[split:]]
     train_dataset, val_dataset, test_dataset = datasets
 
     last_model_path = os.path.join(args.log_dir, args.name, "model")
@@ -109,9 +119,11 @@ def main(argv=None, multi_gpu=True):
                                update_freq=args.log_freq, verbose=args.verbose)
     last_epoch = monitor.last_epoch
     logging.info("Last epoch: {}".format(last_epoch))
+    if args.ray_batch:
+        train_dataset.epoch = last_epoch                     # continue the permutation sequence, do not replay epoch 0
     nerf.compile(optimizer='adam', loss='mean_squared_error', batch_size=args.batch_size, image_width=args.img_wh,
                  image_height=args.img_wh, ray_chunks=args.ray_chunks, run_eagerly=args.eagerly,
-                 white_background=args.white_bg,
+                 white_background=args.white_bg, ray_batch=args.ray_batch,
                  fuse_chunks=None if args.fuse_chunks == 'off' else
                  ('auto' if args.fuse_chunks == 'auto' else int(args.fuse_chunks)))
     if strategy is not None:
