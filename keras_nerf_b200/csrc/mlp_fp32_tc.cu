@@ -66,14 +66,12 @@ __device__ __forceinline__ float4 load_a4(const float* __restrict__ A, int lda, 
 
 // ---- weight operand blobs -------------------------------------------------------------------------------------
 // B[n][k] (n < N outputs, k < K reduction) = src[k * ld + n] (TRANS = false: a Keras kernel [in,out] used forward) or
-// src[n * ld + k] (TRANS = true: the same kernel used by dgrad).  The GEMM kernel works on column blocks of NU outputs
-// (NU = N for N <= 128, N / 2 above); blob: [N / NU blocks][K16 steps][3 splits][2 chunks][NU][8] bf16, zero beyond K, so
-// that one (block, step) stage is ONE contiguous bulk copy.  One thread per 16-byte vector (all three splits).
-__host__ __device__ inline int tcx_nu(int N) { return N; }   // column block of a work unit: all of N (tcx_gemm_kernel)
+// src[n * ld + k] (TRANS = true: the same kernel used by dgrad).  Blob: [K16 steps][3 splits][2 chunks][N][8] bf16, zero
+// beyond K, so that one step's stage is ONE contiguous bulk copy.  One thread per 16-byte vector (all three splits).
 
 __global__ void __launch_bounds__(256) tcx_pack_kernel(const float* __restrict__ src, int ld, int N, int K, int trans,
                                                        uint8_t* __restrict__ blob) {
-  const int ksteps = (K + 15) / 16, NU = tcx_nu(N);
+  const int ksteps = (K + 15) / 16;
   const int total = ksteps * 2 * N;
   for (int v = blockIdx.x * blockDim.x + threadIdx.x; v < total; v += gridDim.x * blockDim.x) {
     const int n = v % N, c = (v / N) & 1, ks = v / (2 * N);
@@ -85,11 +83,10 @@ __global__ void __launch_bounds__(256) tcx_pack_kernel(const float* __restrict__
     }
     uint4 p1, p2, p3;
     split3x8(x, p1, p2, p3);
-    const int nb = n / NU, nl = n - nb * NU;
-    uint8_t* base = blob + ((size_t)nb * ksteps + ks) * 96 * NU + (size_t)(c * NU + nl) * 16;
+    uint8_t* base = blob + (size_t)ks * 96 * N + (size_t)(c * N + n) * 16;
     *reinterpret_cast<uint4*>(base) = p1;
-    *reinterpret_cast<uint4*>(base + 32 * NU) = p2;
-    *reinterpret_cast<uint4*>(base + 64 * NU) = p3;
+    *reinterpret_cast<uint4*>(base + 32 * N) = p2;
+    *reinterpret_cast<uint4*>(base + 64 * N) = p3;
   }
 }
 
@@ -109,12 +106,12 @@ constexpr int kGThreads = 480;          // warps 0-7 split A, 8 and 14 = MMA iss
                                         // 10-13 = epilogue
 constexpr int kGStages = 4;
 struct GemmSmem {
-  // per stage: A [2 tiles][3 splits][2 chunks][128 rows][8] = 24 KB, B [3][2][NU <= 256][8] = 24 KB
+  // per stage: A [2 tiles][3 splits][2 chunks][128 rows][8] = 24 KB, B [3][2][N <= 256][8] = 24 KB
   uint8_t a[kGStages][2 * 3 * 4096];
   uint8_t b[kGStages][3 * 8192];
   float bias[256];                      // staged once: a scalar global load per column and row sat on the epilogue's
                                         // critical path (ncu: 37 % of all stall samples on the dependent FADDs)
-  uint64_t full[kGStages], a_ready[kGStages], empty[kGStages], acc_ready[2], acc_free[2];
+  uint64_t full[kGStages], a_ready[kGStages], empty[kGStages], acc_ready, acc_free;
   uint32_t tmem_base;
 };
 
@@ -129,14 +126,14 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   GemmSmem& sm = *reinterpret_cast<GemmSmem*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int N = g.N, NU = tcx_nu(N), nblocks = N / NU;
+  const int N = g.N;
   const int ks1 = (g.K1 + 15) / 16, ks2 = (g.K2 + 15) / 16, ksteps = ks1 + ks2;
-  const int64_t n_units = ((g.M + 255) / 256) * nblocks;      // unit = row block * nblocks + column block
+  const int64_t n_units = (g.M + 255) / 256;                  // unit = 256-row block
   const int64_t first = blockIdx.x, stride = gridDim.x;
   if (tid == 0) {
     // empty / acc_ready: one tcgen05.commit from EACH of the two issuing threads
     for (int i = 0; i < kGStages; ++i) { mbar_init(&sm.full[i], 1); mbar_init(&sm.a_ready[i], 8); mbar_init(&sm.empty[i], 2); }
-    for (int i = 0; i < 2; ++i) { mbar_init(&sm.acc_ready[i], 2); mbar_init(&sm.acc_free[i], 4); }
+    mbar_init(&sm.acc_ready, 2); mbar_init(&sm.acc_free, 4);
     fence_mbar_init();
   }
   if (warp == 8) tmem_alloc<512>(&sm.tmem_base);
@@ -145,19 +142,17 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = sm.tmem_base;
-  const uint32_t stage_bytes = 96u * (uint32_t)NU;
+  const uint32_t stage_bytes = 96u * (uint32_t)N;
 
   if (warp == 9) {
     // ---- weight-operand producer: one bulk copy per (unit, K = 16 step) ----
     if (lane == 0) {
       uint32_t it = 0;
       for (int64_t u = first; u < n_units; u += stride) {
-        const int nb = (int)(u % nblocks);
         for (int kt = 0; kt < ksteps; ++kt, ++it) {
           const uint32_t s = it % kGStages;
           if (it >= (uint32_t)kGStages) mbar_wait(&sm.empty[s], ((it / kGStages) - 1) & 1);
-          const uint8_t* src = (kt < ks1) ? g.B1 + ((size_t)nb * ks1 + kt) * stage_bytes
-                                          : g.B2 + ((size_t)nb * ks2 + (kt - ks1)) * stage_bytes;
+          const uint8_t* src = (kt < ks1) ? g.B1 + (size_t)kt * stage_bytes : g.B2 + (size_t)(kt - ks1) * stage_bytes;
           mbar_arrive_expect_tx(&sm.full[s], stage_bytes);
           tma_load_1d(sm.b[s], src, stage_bytes, &sm.full[s]);
         }
@@ -170,12 +165,11 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
     //      fp32 summation order -- every output bit -- is fixed ----
     if (lane == 0) {
       const int tile = warp == 8 ? 0 : 1;
-      const uint32_t idesc = umma_idesc_bf16(128, NU, 0, 0);
+      const uint32_t idesc = umma_idesc_bf16(128, N, 0, 0);
       uint32_t it = 0, un = 0;
       for (int64_t u = first; u < n_units; u += stride, ++un) {
-        const uint32_t slot = 0;
         if (un >= 1) {   // the epilogue warps have drained the previous unit (the accumulators fill the TMEM)
-          mbar_wait(&sm.acc_free[slot], (un - 1) & 1);
+          mbar_wait(&sm.acc_free, (un - 1) & 1);
           tc_fence_after();
         }
         for (int kt = 0; kt < ksteps; ++kt, ++it) {
@@ -187,12 +181,12 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
 #pragma unroll
           for (int p = 0; p < 6; ++p) {
             const uint64_t da = umma_smem_desc(a0 + tile * 12288 + kProdA[p] * 4096, 2048, 128);
-            const uint64_t db = umma_smem_desc(b0 + kProdB[p] * 32 * NU, 16 * NU, 128);
+            const uint64_t db = umma_smem_desc(b0 + kProdB[p] * 32 * N, 16 * N, 128);
             umma_bf16(tmem + tile * 256, da, db, idesc, (kt > 0 || p > 0) ? 1u : 0u);
           }
           umma_commit(&sm.empty[s]);
         }
-        umma_commit(&sm.acc_ready[slot]);
+        umma_commit(&sm.acc_ready);
       }
     }
   } else if (warp < 8) {
@@ -210,8 +204,7 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
     auto fetch = [&](int64_t gi, float4 (&x)[4]) {
       const int64_t un = gi / ksteps;
       const int kt = (int)(gi - un * ksteps);
-      const int64_t rb = (first + un * stride) / nblocks;
-      const int64_t grow = rb * 256 + tile * 128 + row0;
+      const int64_t grow = (first + un * stride) * 256 + tile * 128 + row0;
       const bool second = kt >= ks1;
       const float* A = second ? g.A2 : g.A1;
       const int lda = second ? g.lda2 : g.lda1, K = second ? g.K2 : g.K1, k0 = (second ? kt - ks1 : kt) * 16 + qk * 4;
@@ -248,24 +241,20 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
       }
     }
   } else {
-    // ---- epilogue warps 10..13: TMEM lane quadrant = warp & 3; both tiles, all NU columns of the unit ----
+    // ---- epilogue warps 10..13: TMEM lane quadrant = warp & 3; both tiles, all N columns of the unit ----
     const int q = warp & 3;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     uint32_t un = 0;
     for (int64_t u = first; u < n_units; u += stride, ++un) {
-      const uint32_t slot = 0;
-      const int64_t rb = u / nblocks;
-      const int cb = (int)(u % nblocks) * NU;
-      mbar_wait(&sm.acc_ready[slot], un & 1);
+      mbar_wait(&sm.acc_ready, un & 1);
       tc_fence_after();
 #pragma unroll 1
       for (int tl = 0; tl < 2; ++tl) {
-        const int64_t orow = rb * 256 + tl * 128 + q * 32 + lane;
+        const int64_t orow = u * 256 + tl * 128 + q * 32 + lane;
         const bool live = orow < g.M;
-        for (int c0 = 0; c0 < NU; c0 += 32) {
-          const int col = cb + c0;
+        for (int col = 0; col < N; col += 32) {
           uint32_t v[32];
-          tmem_ld32_issue(tmem + lane_base + tl * 256 + c0, v);   // warp-collective: outside the row guard
+          tmem_ld32_issue(tmem + lane_base + tl * 256 + col, v);   // warp-collective: outside the row guard
           // the ReLU' mask row (dgrad) is fetched while the TMEM load is in flight
           float4 mk[8];
           if (g.epi == 3 && live) {
@@ -292,7 +281,7 @@ __global__ void __launch_bounds__(kGThreads, 1) tcx_gemm_kernel(XGemmArgs g) {
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(&sm.acc_free[slot]);
+      if (lane == 0) mbar_arrive(&sm.acc_free);
     }
   }
   tc_fence_before();
@@ -486,8 +475,7 @@ int launch_gemm_tc(const GemmArgs& g, const void* blob1, const void* blob2, cuda
   if (x.A2 == nullptr) x.K2 = 0;
   const size_t smem = sizeof(GemmSmem);
   KN_CUDA(cudaFuncSetAttribute(tcx_gemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int64_t n_units = cdiv(g.M, 256) * (g.N / tcx_nu(g.N));
-  tcx_gemm_kernel<<<(unsigned)std::min<int64_t>(n_units, kNumSMs), kGThreads, smem, st>>>(x);
+  tcx_gemm_kernel<<<(unsigned)std::min<int64_t>(cdiv(g.M, 256), kNumSMs), kGThreads, smem, st>>>(x);
   KN_LAUNCH_CHECK();
   return KNERF_OK;
 }

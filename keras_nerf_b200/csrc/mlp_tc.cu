@@ -6,7 +6,7 @@
 // 256-wide models of up to eight layers with at most one skip concat, L_xyz <= 10, L_dir <= 4 (csrc/api.cu tc_chain_map,
 // tc_layout.cuh TcParams); the Python shim runs other shapes in the fp32_tc mode.
 //
-// Forward kernel (persistent CTA pairs, 384 threads per CTA; roles in tc_roles.cuh / tc_roles2.cuh):
+// Forward kernel (persistent CTA pairs, 384 threads per CTA; roles in tc_roles.cuh):
 //   warp 0      TMA producer: streams this CTA's half of the pre-packed bf16 weight blob, K = 64 stages, 4-slot ring
 //   warps 1,11  MMA issuers (leader CTA): tcgen05.mma.cta_group::2 (M = 256, N = 256|16, K = 16), alternate items
 //   warps 2-9   compute:      PE prologue, TMEM -> register epilogues (ReLU, bf16 pack) that write the next layer's
@@ -23,7 +23,7 @@
 #include <cstdlib>
 #include <type_traits>
 
-#include "tc_roles2.cuh"
+#include "tc_roles.cuh"
 
 namespace knerf {
 using namespace tc;
@@ -360,7 +360,7 @@ __device__ __noinline__ void epi_hidden(uint32_t tacc, uint8_t* __restrict__ hs,
 }
 
 // ---- the fused forward kernel ----------------------------------------------------------------------------
-// Launched as clusters of 2: the CTA pair shares every weight stage through cta_group::2 MMAs (tc_roles2.cuh); a
+// Launched as clusters of 2: the CTA pair shares every weight stage through cta_group::2 MMAs (tc_roles.cuh); a
 // work unit is four tiles (two per CTA).
 template <bool TRAIN, bool REC8>
 __global__ void __launch_bounds__(kThreads, 1)
@@ -378,16 +378,16 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
   const int64_t n_pairs = (n_tiles + 3) / 4;   // work units: four tiles per CTA pair
   const uint32_t cta = cluster_ctarank();
   const int64_t first = blockIdx.x >> 1, stride = gridDim.x >> 1;
-  const uint32_t tmem = chain2_setup(sm, tid, warp, cta);
+  const uint32_t tmem = chain_setup(sm, tid, warp, cta);
   auto tile_of = [&](int64_t unit, int tl) -> int64_t { return unit * 4 + tl * 2 + (int64_t)cta; };
 
   if (warp == 0) {
-    if (lane == 0) producer2_role<Prog>(sm, packed + kFwdPairOff, cta, n_pairs, first, stride);
+    if (lane == 0) producer_role<Prog>(sm, packed + kFwdPairOff, cta, n_pairs, first, stride);
   } else if (warp == 1) {
-    if (lane == 0 && cta == 0) mma2_role<Prog>(sm, tmem, 0u, ordered != 0, n_pairs, first, stride);
+    if (lane == 0 && cta == 0) mma_role<Prog>(sm, tmem, 0u, ordered != 0, n_pairs, first, stride);
     else if (lane == 0) relay_role<Prog>(sm, n_pairs, first, stride);   // peer CTA: its warp 1 is otherwise idle
   } else if (warp == 11) {
-    if (lane == 0 && cta == 0) mma2_role<Prog>(sm, tmem, 1u, ordered != 0, n_pairs, first, stride);
+    if (lane == 0 && cta == 0) mma_role<Prog>(sm, tmem, 1u, ordered != 0, n_pairs, first, stride);
   } else if (warp == 10) {
     // ============== record store (training): the operand tiles h0..h7 -> HBM, bulk copies ======================
     if constexpr (TRAIN && !REC8) {
@@ -404,26 +404,11 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
     uint32_t acc_par[2] = {0, 0};
 
-    uint32_t st_pending = 0, st_par = 0;      // training: bit tl = hs[tl] is being stored / parity of st_done[tl]
-    // this thread's (warp's) part of the next A operand is in smem; `record`: the tile is also a saved record
-    auto a_ready_arrive = [&](int tl, bool record) {
-      a_ready_arrive2(sm, tl, lane);
-      if (TRAIN && !REC8 && record) {   // (fp8 records leave from the epilogue's registers)
-        st_ready_arrive(&sm.st_ready[tl], lane);
-        st_pending |= 1u << tl;
-      }
-    };
-    auto hs_writable = [&](int tl) {          // the bulk store of the previous contents of hs[tl] has read them
-      if (TRAIN && ((st_pending >> tl) & 1)) {
-        mbar_wait(&sm.st_done[tl], (st_par >> tl) & 1);
-        st_par ^= 1u << tl;
-        st_pending &= ~(1u << tl);
-      }
-    };
+    ChainHandshake<TRAIN && !REC8> hk;
     auto prologue = [&](int64_t pair, int tl, const float (&p)[3]) {
       const int64_t tile = tile_of(pair, tl);
       pe_xyz<REC8>(sm.xs[tl], (TRAIN && tile < n_tiles) ? rec + tile * kRB + kOffXS : nullptr, r, h, p[0], p[1], p[2]);
-      a_ready_arrive(tl, false);
+      hk.arrive(sm, tl, lane, false);
     };
 
     KN_PROF_DECL();
@@ -456,7 +441,7 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
             // hidden layers: 128 of the 256 columns per thread
             float dirv[3];
             if (s == 5) load_dir(dirv, d, g, M, S);   // fetched now, used after the epilogue: the L2 latency hides behind it
-            hs_writable(tl);
+            hk.wait_writable(sm, tl);
             epi_hidden<TRAIN, REC8>(tmem + lane_base + tl * 256, sm.hs[tl], h, r,
                                     save ? rec_t + kOffMask + s * kMaskLayerBytes : nullptr,
                                     (REC8 && save) ? rec_t + kRec8H0 + s * kH8Bytes : nullptr);
@@ -464,7 +449,7 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
               // xs[tl] is dead after layer 5 (skip concat consumed): it now carries PE(dir) for the last step
               pe_dir<REC8>(sm.xs[tl], save ? rec_t + kOffDS : nullptr, r, h, dirv[0], dirv[1], dirv[2]);
             }
-            a_ready_arrive(tl, true);
+            hk.arrive(sm, tl, lane, true);
           } else {
             // columns 0..2 (+ 4..6): the rgb pre-activations, 3 (+ 7): sigma's (heads folded into the step, biases
             // included; mlp.py:40, 43-48).  One half-row thread per row finishes it; the other starts the next tile.
@@ -490,7 +475,7 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
     KN_PROF_END(t_c, 5);
     if (tid == 64) { KN_PROF_FLUSH(); }
   }
-  chain2_teardown(tmem, warp);
+  chain_teardown(tmem, warp);
 }
 
 }  // namespace
@@ -498,18 +483,7 @@ tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ 
 bool tc_path_compiled() { return true; }
 
 // diagnostic (-DKNERF_TC_TIMING builds only): copy and clear the forward kernel's per-CTA cycle counters
-int tc_debug_timing(unsigned long long* host_out, int n) {
-#ifdef KNERF_TC_TIMING
-  static unsigned long long zeros[160 * 40];
-  if (n > 160 * 40) n = 160 * 40;
-  if (cudaMemcpyFromSymbol(host_out, g_tc_prof, (size_t)n * 8) != cudaSuccess) return -1;
-  if (cudaMemcpyToSymbol(g_tc_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
-  return n;
-#else
-  (void)host_out; (void)n;
-  return 0;
-#endif
-}
+int tc_debug_timing(unsigned long long* host_out, int n) { return KN_PROF_READ(g_tc_prof, host_out, n); }
 
 int64_t tc_packed_weight_bytes(const Model& m) { return is_flagship(m) ? kPackedBytes : -1; }
 
@@ -559,35 +533,14 @@ int tc_forward(const Model& m, const float* params, const void* packed, const fl
                    (reinterpret_cast<uintptr_t>(ws) & 15) == 0,
                "tc_forward: rgbsigma / packed / workspace must be 16-byte aligned");
   KN_CHECK_ARG(M < (int64_t(1) << 31), "tc_forward: at most 2^31 - 1 samples per call");
-  const int64_t n_tiles = cdiv(M, kTileM);
-  cudaLaunchConfig_t cfg{};
-  cudaLaunchAttribute attr[1];
-  cfg.blockDim = dim3(kThreads);
-  cfg.stream = st;
-  cfg.gridDim = dim3((unsigned)(2 * std::min<int64_t>(cdiv(n_tiles, 4), kNumSMs / 2)));
-  cfg.dynamicSmemBytes = sizeof(ChainSmem);
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  // MMA issue order (tc_roles2.cuh): bit-reproducible when training, free-running at inference unless the call
+  // MMA issue order (tc_roles.cuh): bit-reproducible when training, free-running at inference unless the call
   // carries KNERF_TC_ORDERED
   const int ordered = (training || ordered_issue) ? 1 : 0;
-  const uint8_t* pk = (const uint8_t*)packed;
-  float4* out = (float4*)rgbsigma;
-  uint8_t* rec = training ? (uint8_t*)ws + kXBytes : nullptr;
-  if (training && rec8) {
-    KN_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes));
-    KN_CUDA(cudaLaunchKernelEx(&cfg, tc_mlp_fwd_kernel<true, true>, pk, o, d, t, M, S, out, rec, ordered));
-  } else if (training) {
-    KN_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes));
-    KN_CUDA(cudaLaunchKernelEx(&cfg, tc_mlp_fwd_kernel<true, false>, pk, o, d, t, M, S, out, rec, ordered));
-  } else {
-    KN_CUDA(cudaFuncSetAttribute(tc_mlp_fwd_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes));
-    KN_CUDA(cudaLaunchKernelEx(&cfg, tc_mlp_fwd_kernel<false, false>, pk, o, d, t, M, S, out, rec, ordered));
-  }
-  KN_LAUNCH_CHECK();
-  return KNERF_OK;
+  auto kernel = !training ? &tc_mlp_fwd_kernel<false, false>
+                : rec8    ? &tc_mlp_fwd_kernel<true, true>
+                          : &tc_mlp_fwd_kernel<true, false>;
+  return launch_chain(kernel, cdiv(M, kTileM), st, (const uint8_t*)packed, o, d, t, M, S, (float4*)rgbsigma,
+                      training ? (uint8_t*)ws + kXBytes : nullptr, ordered);
 }
 
 }  // namespace knerf

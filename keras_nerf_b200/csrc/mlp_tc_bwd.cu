@@ -17,7 +17,7 @@
 #include <algorithm>
 #include <cstdlib>
 #include <vector>
-#include "tc_roles2.cuh"
+#include "tc_roles.cuh"
 
 namespace knerf {
 using namespace tc;
@@ -90,7 +90,7 @@ __global__ void __launch_bounds__(256) dpre_amax_kernel(const float4* __restrict
   if ((threadIdx.x & 31) == 0 && m > 0.f) atomicMax(amax_bits, __float_as_uint(m));
 }
 
-// clusters of 2, cta_group::2 MMAs (tc_roles2.cuh); a work unit is four tiles (two per CTA)
+// clusters of 2, cta_group::2 MMAs (tc_roles.cuh); a work unit is four tiles (two per CTA)
 template <bool REC8>
 __global__ void __launch_bounds__(kThreads, 1)
 tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict__ d_pre, int64_t M,
@@ -105,16 +105,16 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
   const int64_t n_pairs = (n_tiles + 3) / 4;   // work units: four tiles per CTA pair
   const uint32_t cta = cluster_ctarank();
   const int64_t first = blockIdx.x >> 1, stride = gridDim.x >> 1;
-  const uint32_t tmem = chain2_setup(sm, tid, warp, cta);
+  const uint32_t tmem = chain_setup(sm, tid, warp, cta);
   auto tile_of = [&](int64_t unit, int tl) -> int64_t { return unit * 4 + tl * 2 + (int64_t)cta; };
 
   if (warp == 0) {
-    if (lane == 0) producer2_role<BwdProg>(sm, packed + kBwdPairOff, cta, n_pairs, first, stride);
+    if (lane == 0) producer_role<BwdProg>(sm, packed + kBwdPairOff, cta, n_pairs, first, stride);
   } else if (warp == 1) {
-    if (lane == 0 && cta == 0) mma2_role<BwdProg>(sm, tmem, 0u, true, n_pairs, first, stride);
+    if (lane == 0 && cta == 0) mma_role<BwdProg>(sm, tmem, 0u, true, n_pairs, first, stride);
     else if (lane == 0) relay_role<BwdProg>(sm, n_pairs, first, stride);
   } else if (warp == 11) {
-    if (lane == 0 && cta == 0) mma2_role<BwdProg>(sm, tmem, 1u, true, n_pairs, first, stride);
+    if (lane == 0 && cta == 0) mma_role<BwdProg>(sm, tmem, 1u, true, n_pairs, first, stride);
   } else if (warp == 10) {
     // record store: the A operands dZ7..dZ1 of the chain (items 1..7) are also the dZ records of the weight-gradient
     // kernel (tc_roles.cuh store_role); item 0 = (d rgb_pre, d sigma_pre) only takes part in the hand-shake: the
@@ -127,21 +127,7 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
                  [](int item) { return (uint32_t)(item == 0 ? 0 : kHSBytes); });   // dG stays on chip (item 0)
     }
   } else {
-    uint32_t st_pending = 0, st_par = 0;      // bit tl = hs[tl] is being stored / parity of st_done[tl]
-    auto a_ready_arrive = [&](int tl) {   // this thread's (warp's) part of the next A operand (= dZ record) is in smem
-      a_ready_arrive2(sm, tl, lane);
-      if (!REC8) {
-        st_ready_arrive(&sm.st_ready[tl], lane);
-        st_pending |= 1u << tl;
-      }
-    };
-    auto hs_writable = [&](int tl) {          // the bulk store of the previous contents of hs[tl] has read them
-      if ((st_pending >> tl) & 1) {
-        mbar_wait(&sm.st_done[tl], (st_par >> tl) & 1);
-        st_par ^= 1u << tl;
-        st_pending &= ~(1u << tl);
-      }
-    };
+    ChainHandshake<!REC8> hk;   // (every A operand of the chain is also a dZ record)
     const int q = warp & 3, h = (warp - 2) >> 2;
     const int r = q * 32 + lane;
     const uint32_t lane_base = (uint32_t)(q * 32) << 16;
@@ -170,20 +156,22 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
             make_uint4(pack_e5m2x4(dq.x, dq.y, dq.z, dq.w), 0u, 0u, 0u);
       if (h == 0) {   // bias gradients of the two heads: db_rgb = sum d(rgb_pre), db_sigma = sum d(sigma_pre)
         const float s0 = warp_sum(dp.x), s1 = warp_sum(dp.y), s2 = warp_sum(dp.z), s3 = warp_sum(dp.w);
+        // sum d(rgb_pre) of THIS call for tc_finish_kernel, over the values the weight-gradient kernel's heads task
+        // multiplies: the fp32 d_pre with fp8 records, the bf16 operand (kDzP) with bf16 records (dq = dp there)
+        const float r0 = REC8 ? s0 : warp_sum(bf16_lo(pk.x)), r1 = REC8 ? s1 : warp_sum(bf16_hi(pk.x)),
+                    r2 = REC8 ? s2 : warp_sum(bf16_lo(pk.y));
         if (lane == 0) {
           atomicAdd(grads + P.b_off[11], s0); atomicAdd(grads + P.b_off[11] + 1, s1);
           atomicAdd(grads + P.b_off[11] + 2, s2); atomicAdd(grads + P.b_off[8], s3);
-          if (REC8) {   // sum d(rgb_pre) of THIS call for tc_finish_kernel (the bf16 path sums its operand copy instead)
-            atomicAdd(xbuf + kXOffS, s0); atomicAdd(xbuf + kXOffS + 1, s1); atomicAdd(xbuf + kXOffS + 2, s2);
-          }
+          atomicAdd(xbuf + kXOffS, r0); atomicAdd(xbuf + kXOffS + 1, r1); atomicAdd(xbuf + kXOffS + 2, r2);
         }
       }
-      hs_writable(tl);
+      hk.wait_writable(sm, tl);
       // chunk 0 of the row (h = 0), zeros in chunk 1 (h = 0) and chunks 2, 3 (h = 1): the step reads K = 32, and a
       // stale NaN pattern times a zero weight would not be zero
       *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h) * kChunkA + r * 16) = pk;
       *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h + 1) * kChunkA + r * 16) = make_uint4(0u, 0u, 0u, 0u);
-      a_ready_arrive(tl);
+      hk.arrive(sm, tl, lane, true);
       KN_PROF_END(t_p, 15 + tl * 16);
     };
 
@@ -214,14 +202,14 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
           KN_PROF_BEGIN(t_e);
           acc_par[tl] ^= 1;
           tc_fence_after();
-          if (b + 1 < BwdProg::kSteps) hs_writable(tl);
+          if (b + 1 < BwdProg::kSteps) hk.wait_writable(sm, tl);
           const uint32_t tacc = tmem + lane_base + tl * 256;
           const uint4 mbv = make_uint4(mb[0], mb[1], mb[2], mb[3]);
           uint8_t* out8 = (REC8 && active) ? out : nullptr;
           if (b + 1 < BwdProg::kSteps) epi_dgrad<2, REC8>(tacc, sm.hs[tl], h, r, mbv, out8);
           else epi_dgrad<3, REC8>(tacc, active ? out : nullptr, h, r, mbv, out8);
           if (b + 1 < BwdProg::kSteps) {
-            a_ready_arrive(tl);
+            hk.arrive(sm, tl, lane, true);
             KN_PROF_END(t_e, 6 + tl * 16 + b);
           } else {
             tc_fence_before();
@@ -236,7 +224,7 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
     KN_PROF_END(t_c, 5);
     if (tid == 64) { KN_PROF_FLUSH(); }
   }
-  chain2_teardown(tmem, warp);
+  chain_teardown(tmem, warp);
 }
 
 // =============================================================================================================
@@ -264,7 +252,7 @@ constexpr int kWBlocks = 4;           // TMEM accumulator blocks of 128 columns:
 // are the bias gradient of that layer
 struct WUnit { int src, off, bytes, bias_layer, bias_col0, off2, bytes2; };
 // accumulator group: A = unit a (+ a_sub bytes), B = unit b (+ b_sub bytes)
-struct WGroup { int a, b, col, N, layer, row_base, row_limit, col_base, mode, free_a, free_b, a_sub, b_sub, issuer; };
+struct WGroup { int a, b, col, N, layer, row_base, row_limit, col_base, mode, a_sub, b_sub, issuer; };
 // last_grp[x][k]: the last group of issuer x that reads unit k (the one after which x releases the slot), -1 = none;
 // last_in_blk[x][b]: the last group of issuer x in TMEM block b (its last tile's MMAs end the block's accumulation);
 // a group covers the blocks blk_first(g) .. blk_last(g)
@@ -272,10 +260,13 @@ struct WTask {
   int n_units; WUnit u[kWMaxUnits]; int n_groups; WGroup g[kWMaxUnits]; int cost;
   int8_t last_grp[2][kWMaxUnits]; int8_t last_in_blk[2][kWBlocks];
 };
-// mode 0: dW[layer][(row_base+row), col_base+col]
-//      1: A = h7, B = the packed d_pre operand: column 3 = the sigma kernel's gradient, columns 0..2 = Y = h7^T d(rgb_pre)
-//         into the fp32 scratch
-//      4: A = PE(dir): columns 0..2 = Yd = PE(dir)^T d(rgb_pre) into the scratch     (tc_finish_kernel uses Y, Yd)
+// WGroup::mode, where the flush puts the accumulator:
+enum : int {
+  kFlushKernel = 0,   // dW[layer][(row_base+row), col_base+col] of a hidden layer
+  kFlushHeads = 1,    // A = h7, B = the packed d_pre operand: column 3 = the sigma kernel's gradient, columns 0..2 =
+                      // Y = h7^T d(rgb_pre) into the fp32 scratch
+  kFlushDir = 4,      // A = PE(dir): columns 0..2 = Yd = PE(dir)^T d(rgb_pre) into the scratch (tc_finish_kernel uses Y, Yd)
+};
 
 struct WTaskTable { WTask t[kNumTasks]; };
 // One accumulator group as its issuer runs it, built once per work item: units a / b, rel = release unit a (bit 0) /
@@ -296,7 +287,7 @@ static void fit_tasks_to_model(WTaskTable& T, const TcParams& P) {
     for (int gi = 0; gi < t.n_groups; ++gi) {
       WGroup& g = t.g[gi];
       const int l = g.layer;
-      if (g.mode == 0 && l >= 0 && l < 8) {
+      if (g.mode == kFlushKernel && l >= 0 && l < 8) {
         if (l == 5 && g.row_base == 256) {            // encoding rows of the concat layer
           g.row_base = P.U;
           if (!P.x5) g.row_limit = 0;
@@ -304,7 +295,7 @@ static void fit_tasks_to_model(WTaskTable& T, const TcParams& P) {
           g.row_limit = std::max(0, std::min(g.row_limit, P.U - g.row_base));
         }
         if (P.w_off[l] < 0) g.row_limit = 0;
-      } else if (g.mode == 1) {                       // Y = h7^T d(rgb_pre) and the sigma kernel: rows of h7
+      } else if (g.mode == kFlushHeads) {             // Y = h7^T d(rgb_pre) and the sigma kernel: rows of h7
         g.row_limit = std::max(0, std::min(g.row_limit, P.U - g.row_base));
       }
     }
@@ -351,10 +342,10 @@ static WTaskTable build_task_table(int dx, int dd) {
     t.u[0] = {0, a_off, kWUnitBytes, -1, 0}; t.u[1] = {1, b_off, kWUnitBytes, layer, 0};
     t.u[2] = {1, b_off + kWUnitBytes, kWUnitBytes, layer, 128}; t.u[3] = {0, a_off + kWUnitBytes, kWUnitBytes, -1, 0};
     t.n_groups = 4;
-    t.g[0] = {0, 1, 0, 128, layer, row_base, 128, 0, 0, 0, 0};
-    t.g[1] = {0, 2, 128, 128, layer, row_base, 128, 128, 0, 1, 0};
-    t.g[2] = {3, 1, 256, 128, layer, row_base + 128, 128, 0, 0, 0, 1};
-    t.g[3] = {3, 2, 384, 128, layer, row_base + 128, 128, 128, 0, 1, 1};
+    t.g[0] = {0, 1, 0, 128, layer, row_base, 128, 0, kFlushKernel, 0, 0};
+    t.g[1] = {0, 2, 128, 128, layer, row_base, 128, 128, kFlushKernel, 0, 0};
+    t.g[2] = {3, 1, 256, 128, layer, row_base + 128, 128, 0, kFlushKernel, 0, 0};
+    t.g[3] = {3, 2, 384, 128, layer, row_base + 128, 128, 128, kFlushKernel, 0, 0};
     t.cost = 128;
   };
   auto xpart = [&](int layer, int b_off, int row_base) {           // A: PE(xyz) (63 valid rows), B: two halves
@@ -366,8 +357,8 @@ static WTaskTable build_task_table(int dx, int dd) {
     t.u[0] = {0, kRecXS, kXSBytes, -1, 0}; t.u[1] = {1, b_off, kWUnitBytes, bl, 0};
     t.u[2] = {1, b_off + kWUnitBytes, kWUnitBytes, bl, 128};
     t.n_groups = 2;
-    t.g[0] = {0, 1, 0, 128, layer, row_base, dx, 0, 0, 0, 1};
-    t.g[1] = {0, 2, 128, 128, layer, row_base, dx, 128, 0, 1, 1};
+    t.g[0] = {0, 1, 0, 128, layer, row_base, dx, 0, kFlushKernel, 0, 0};
+    t.g[1] = {0, 2, 128, 128, layer, row_base, dx, 128, kFlushKernel, 0, 0};
     t.cost = 76;    // costs = measured time per tile of a CTA working alone on the task (x 128 / the `big` tasks'):
                     // 3,700 / 6,300 / 8,400 cycles -- the kernel is bound by its CTAs' per-tile time, so equal item
                     // TIMES (not bytes) remove the tail
@@ -379,9 +370,10 @@ static WTaskTable build_task_table(int dx, int dd) {
      // gradient that contains it factors through three columns:  h7^T dG = (h7^T d(rgb_pre)) Wc^T,
      // PE(dir)^T dG = (PE(dir)^T d(rgb_pre)) Wc^T,  sum dG = (sum d(rgb_pre)) Wc^T.  The task therefore reads h7, PE(dir)
      // and the packed (d rgb_pre, d sigma_pre) operand only -- N = 16 MMAs -- and leaves Y = h7^T d(rgb_pre) [256 x 3]
-     // (+ the sigma kernel's gradient, column 3 of the same accumulator), Yd = PE(dir)^T d(rgb_pre) [27 x 3] and
-     // s3 = sum d(rgb_pre) in the scratch; tc_finish_kernel expands them into dW / db of features, rgb_features and
-     // rgb.  Neither dG nor the rgb_features activations travel through HBM (64 KB per tile less than round 1).
+     // (+ the sigma kernel's gradient, column 3 of the same accumulator) and Yd = PE(dir)^T d(rgb_pre) [27 x 3] in the
+     // scratch, next to s3 = sum d(rgb_pre) from the dgrad prologue; tc_finish_kernel expands them into dW / db of
+     // features, rgb_features and rgb.  Neither dG nor the rgb_features activations travel through HBM (64 KB per
+     // tile less than round 1).
     WTask& t = T.t[n++];
     const int h7 = kRecH0 + 7 * kHSBytes;
     t.n_units = 3;
@@ -390,9 +382,9 @@ static WTaskTable build_task_table(int dx, int dd) {
                                                                 // at +8192, the packed (d rgb_pre, d sigma_pre) operand
     t.u[2] = {0, h7 + kWUnitBytes, kWUnitBytes, -1, 0, 0, 0};   // h7 features 128..255
     t.n_groups = 3;
-    t.g[0] = {0, 1, 0, 16, 8, 0, 128, 0, 1, 0, 0, 0, 8192};     // Y rows 0..127 (columns 0..2), sigma kernel (column 3)
-    t.g[1] = {2, 1, 32, 16, 8, 128, 128, 0, 1, 0, 0, 0, 8192};  // rows 128..255
-    t.g[2] = {1, 1, 64, 16, -1, 0, dd, 0, 4, 0, 0, 0, 8192};    // Yd: A and B share the unit
+    t.g[0] = {0, 1, 0, 16, 8, 0, 128, 0, kFlushHeads, 0, 8192};     // Y rows 0..127 (columns 0..2), sigma kernel (column 3)
+    t.g[1] = {2, 1, 32, 16, 8, 128, 128, 0, kFlushHeads, 0, 8192};  // rows 128..255
+    t.g[2] = {1, 1, 64, 16, -1, 0, dd, 0, kFlushDir, 0, 8192};      // Yd: A and B share the unit
     t.g[0].issuer = 0; t.g[1].issuer = 1; t.g[2].issuer = 0;
     t.cost = kHeadsCost;
   }
@@ -414,8 +406,8 @@ static WTaskTable build_task_table8(int dx, int dd) {
     // halves of the outputs are one operand), and each issuer issues half as many MMAs as with 128 x 128 groups -- the
     // kernel is bound by MMA issue (profiles/r03_wgrad.md)
     t.n_groups = 2;
-    t.g[0] = {0, 1, 0, 256, layer, row_base, 128, 0, 0, 0, 0, 0, 0};
-    t.g[1] = {0, 1, 256, 256, layer, row_base + 128, 128, 0, 0, 0, 0, kHalf, 0};
+    t.g[0] = {0, 1, 0, 256, layer, row_base, 128, 0, kFlushKernel, 0, 0};
+    t.g[1] = {0, 1, 256, 256, layer, row_base + 128, 128, 0, kFlushKernel, kHalf, 0};
     t.cost = 128;
   };
   auto xpart = [&](int layer, int b_off, int row_base) {
@@ -424,8 +416,8 @@ static WTaskTable build_task_table8(int dx, int dd) {
     const int bl = (layer == 0) ? 0 : -1;
     t.u[0] = {0, kRec8XS, 8192, -1, 0, 0, 0}; t.u[1] = {1, b_off, kH8Bytes, bl, 0, 0, 0};
     t.n_groups = 2;
-    t.g[0] = {0, 1, 0, 128, layer, row_base, dx, 0, 0, 0, 0, 0, 0};
-    t.g[1] = {0, 1, 128, 128, layer, row_base, dx, 128, 0, 0, 0, 0, kHalf};
+    t.g[0] = {0, 1, 0, 128, layer, row_base, dx, 0, kFlushKernel, 0, 0};
+    t.g[1] = {0, 1, 128, 128, layer, row_base, dx, 128, kFlushKernel, 0, kHalf};
     t.cost = kXpartCost8;
   };
   xpart(0, kDz8Z0, 0);
@@ -437,9 +429,9 @@ static WTaskTable build_task_table8(int dx, int dd) {
     t.u[0] = {0, kRec8H0 + 7 * kH8Bytes, kH8Bytes, -1, 0, 0, 0};   // h7
     t.u[1] = {0, kRec8DS, 4096, -1, 0, kDz8P, 2048};               // PE(dir) and, at +4096, the packed d_pre operand
     t.n_groups = 3;
-    t.g[0] = {0, 1, 0, 16, 8, 0, 128, 0, 1, 0, 0, 0, 4096};
-    t.g[1] = {0, 1, 32, 16, 8, 128, 128, 0, 1, 0, 0, kHalf, 4096};
-    t.g[2] = {1, 1, 64, 16, -1, 0, dd, 0, 4, 0, 0, 0, 4096};
+    t.g[0] = {0, 1, 0, 16, 8, 0, 128, 0, kFlushHeads, 0, 4096};
+    t.g[1] = {0, 1, 32, 16, 8, 128, 128, 0, kFlushHeads, kHalf, 4096};
+    t.g[2] = {1, 1, 64, 16, -1, 0, dd, 0, kFlushDir, 0, 4096};
     t.g[0].issuer = 0; t.g[1].issuer = 1; t.g[2].issuer = 0;
     t.cost = kHeadsCost8;
   }
@@ -746,8 +738,7 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
       __syncwarp();
       if (lane == 0) mbar_arrive(&sm.q_empty[j % kWQueue]);
       if (item < 0) break;
-      const int task = L.task[item];
-      const WTask& t = T.t[task];
+      const WTask& t = T.t[L.task[item]];
       const int64_t lo = L.range[item].x, hi = L.range[item].y;
       // While the tensor core works through the item, these warps take the bias gradients: column sums (over
       // samples) of every dZ unit passing through shared memory.  Thread (fc, fsub) owns 8 columns of chunk fc
@@ -758,7 +749,6 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
       for (int u = 0; u < 2; ++u)
 #pragma unroll
         for (int e = 0; e < 8; ++e) bacc[u][e] = 0.f;
-      float pacc[3] = {0.f, 0.f, 0.f};          // this thread's row of the packed d_pre operand, summed over the tiles
       for (int64_t tile = lo; tile < hi; ++tile) {
         int nb = 0;
         for (int k = 0; k < t.n_units; ++k, ++uit) {
@@ -786,10 +776,6 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
               }
             }
             ++nb;
-          }
-          if (!REC8 && t.u[k].bytes2 != 0) {   // the d_pre operand at +8192: [2 chunks][128 rows][8], chunk 0 = (r, g, b, sigma, 0..)
-            const uint2 v = *reinterpret_cast<const uint2*>(sm.slot[slot] + 8192 + ftid * 16);   // one row per thread: this
-            pacc[0] += bf16_lo(v.x); pacc[1] += bf16_hi(v.x); pacc[2] += bf16_lo(v.y);           // sits on the slot-release path
           }
 #ifdef KNERF_TC_TIMING
           const long long kn_sum_end = clock64();
@@ -832,13 +818,6 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
           ++nb;
         }
       }
-      if (!REC8 && task == kNumTasks - 1) {   // heads task: sum d(rgb_pre) of this call for tc_finish_kernel
-#pragma unroll
-        for (int e = 0; e < 3; ++e) {
-          const float sres = warp_sum(pacc[e]);
-          if (lane == 0) atomicAdd(xbuf + kXOffS + e, sres);
-        }
-      }
       KN_WG_ADD(7, 1);
       KN_WG_ADD(8, hi - lo);
       for (int b = 0; b < kWBlocks; ++b) {
@@ -857,7 +836,7 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
               for (int i = 0; i < 32; ++i) v[i] *= inv_scale;
             }
             if (row < g.row_limit) {
-              if (g.mode == 0) {   // kernel [fan_in, U] of a hidden layer: columns >= U belong to the padding
+              if (g.mode == kFlushKernel) {   // kernel [fan_in, U] of a hidden layer: columns >= U belong to the padding
                 float* dst = grads + P.w_off[g.layer] + (int64_t)(g.row_base + row) * P.U + g.col_base + c0;
                 const int nv = P.U - (g.col_base + c0);
                 if (nv >= 32 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0) {
@@ -868,7 +847,7 @@ tc_wgrad_kernel(const uint8_t* __restrict__ rec, const uint8_t* __restrict__ dz,
                   for (int i = 0; i < 32; ++i)
                     if (i < nv) atomicAdd(dst + i, v[i]);
                 }
-              } else if (g.mode == 1) {
+              } else if (g.mode == kFlushHeads) {
                 atomicAdd(grads + P.w_off[8] + g.row_base + row, v[3]);
                 float* dst = xbuf + kXOffY + (g.row_base + row) * 4;
                 atomicAdd(dst, v[0]); atomicAdd(dst + 1, v[1]); atomicAdd(dst + 2, v[2]);
@@ -996,33 +975,11 @@ __global__ void __launch_bounds__(256) tc_finish_kernel(const float* __restrict_
 }  // namespace
 
 // diagnostic (-DKNERF_TC_TIMING builds only): copy and clear the weight-gradient kernel's per-CTA counters
-int tc_debug_wgrad_timing(unsigned long long* host_out, int n) {
-#ifdef KNERF_TC_TIMING
-  static unsigned long long zeros[160 * kWProf];
-  if (n > 160 * kWProf) n = 160 * kWProf;
-  if (cudaMemcpyFromSymbol(host_out, g_wg_prof, (size_t)n * 8) != cudaSuccess) return -1;
-  if (cudaMemcpyToSymbol(g_wg_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
-  return n;
-#else
-  (void)host_out; (void)n;
-  return 0;
-#endif
-}
+int tc_debug_wgrad_timing(unsigned long long* host_out, int n) { return KN_PROF_READ(g_wg_prof, host_out, n); }
 
 // diagnostic (-DKNERF_TC_TIMING builds only): copy and clear the dgrad kernel's per-CTA cycle counters (the slots of
 // tc_roles.cuh; this translation unit has its own g_tc_prof, so the forward's counters do not mix in)
-int tc_debug_dgrad_timing(unsigned long long* host_out, int n) {
-#ifdef KNERF_TC_TIMING
-  static unsigned long long zeros[160 * 40];
-  if (n > 160 * 40) n = 160 * 40;
-  if (cudaMemcpyFromSymbol(host_out, g_tc_prof, (size_t)n * 8) != cudaSuccess) return -1;
-  if (cudaMemcpyToSymbol(g_tc_prof, zeros, sizeof(zeros)) != cudaSuccess) return -1;
-  return n;
-#else
-  (void)host_out; (void)n;
-  return 0;
-#endif
-}
+int tc_debug_dgrad_timing(unsigned long long* host_out, int n) { return KN_PROF_READ(g_tc_prof, host_out, n); }
 
 // parts: which of the backward kernels to launch (bit 0 dgrad, bit 1 wgrad + finish; KNERF_BWD_*_ONLY)
 int tc_backward(const Model& m, const float* params, const void* packed, const float* d_pre, int64_t R, int S,
@@ -1040,34 +997,18 @@ int tc_backward(const Model& m, const float* params, const void* packed, const f
   uint8_t* dz = rec + n_tiles * (int64_t)(rec8 ? kRec8Bytes : kRecBytes);
   const TcParams P = tc_make_params(m);
   // the fp32 scratch (rank-3 factors, sum d(rgb_pre), max|d_pre|) starts from zero in every call -- except that a
-  // weight-gradient-only call (KNERF_BWD_WGRAD_ONLY) over fp8 records keeps what the dgrad-only call before it left
-  // there: sum d(rgb_pre) and the scale of the gradient records
-  KN_CUDA(cudaMemsetAsync(xbuf, 0, ((rec8 && parts == 2) ? kXOffS : kXFloats) * sizeof(float), st));
+  // weight-gradient-only call (KNERF_BWD_WGRAD_ONLY) keeps what the dgrad-only call before it left there: sum d(rgb_pre)
+  // and (fp8 records) the scale of the gradient records
+  KN_CUDA(cudaMemsetAsync(xbuf, 0, (parts == 2 ? kXOffS : kXFloats) * sizeof(float), st));
 
   if (parts & 1) {
-    cudaLaunchConfig_t cfg{};
-    cudaLaunchAttribute attr[1];
-    cfg.blockDim = dim3(kThreads);
-    cfg.stream = st;
-    cfg.gridDim = dim3((unsigned)(2 * std::min<int64_t>(cdiv(n_tiles, 4), kNumSMs / 2)));
-    cfg.dynamicSmemBytes = sizeof(ChainSmem);
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    const uint8_t* pk = (const uint8_t*)packed;
     const float4* dp = (const float4*)d_pre;
-    const uint8_t* rec_c = rec;
     if (rec8) {
       dpre_amax_kernel<<<kNumSMs * 4, 256, 0, st>>>(dp, M, reinterpret_cast<uint32_t*>(xbuf) + kXOffAmax);
       KN_LAUNCH_CHECK();
-      KN_CUDA(cudaFuncSetAttribute(tc_mlp_dgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes));
-      KN_CUDA(cudaLaunchKernelEx(&cfg, tc_mlp_dgrad_kernel<true>, pk, dp, M, rec_c, dz, grads, P, xbuf));
-    } else {
-      KN_CUDA(cudaFuncSetAttribute(tc_mlp_dgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)cfg.dynamicSmemBytes));
-      KN_CUDA(cudaLaunchKernelEx(&cfg, tc_mlp_dgrad_kernel<false>, pk, dp, M, rec_c, dz, grads, P, xbuf));
     }
-    KN_LAUNCH_CHECK();
+    KN_TRY(launch_chain(rec8 ? &tc_mlp_dgrad_kernel<true> : &tc_mlp_dgrad_kernel<false>, n_tiles, st,
+                        (const uint8_t*)packed, dp, M, (const uint8_t*)rec, dz, grads, P, xbuf));
   }
   if (parts & 2) {
     // the task table (~3 KB) and the item list (~9 KB) are passed by value as __grid_constant__ parameters
@@ -1078,13 +1019,9 @@ int tc_backward(const Model& m, const float* params, const void* packed, const f
     const int n_items = build_items(h_table, n_tiles, h_items);
     if (n_items < 0) return fail(KNERF_ERR_UNSUPPORTED, "tc_backward: more than %d weight-gradient items", kWMaxItems);
     const size_t smem = sizeof(WSmem);
-    if (rec8) {
-      KN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      tc_wgrad_kernel<true><<<kNumSMs, kWThreads, smem, st>>>(rec, dz, grads, xbuf, P, h_table, h_items, n_items);
-    } else {
-      KN_CUDA(cudaFuncSetAttribute(tc_wgrad_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      tc_wgrad_kernel<false><<<kNumSMs, kWThreads, smem, st>>>(rec, dz, grads, xbuf, P, h_table, h_items, n_items);
-    }
+    auto wgrad = rec8 ? &tc_wgrad_kernel<true> : &tc_wgrad_kernel<false>;
+    KN_CUDA(cudaFuncSetAttribute(wgrad, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    wgrad<<<kNumSMs, kWThreads, smem, st>>>(rec, dz, grads, xbuf, P, h_table, h_items, n_items);
     KN_LAUNCH_CHECK();
     tc_finish_prep_kernel<<<6, 256, 0, st>>>(params, P, xbuf);
     KN_LAUNCH_CHECK();

@@ -74,8 +74,8 @@ struct BwdProg {
 //   step s: [stage 0: cta0 piece | cta1 piece][stage 1: ...] ... [bias stage: cta0 | cta1]
 //   piece = [k/8 chunks][N/2 rows][8]   (k = 64, or the 32-wide tail of the direction encoding, or 16 for the bias)
 constexpr int kPairK = 64;
-constexpr int kNumStages2 = 4;
-constexpr int kStageBytes2 = 128 * kPairK * 2;     // 16 KB ring slot (N/2 <= 128 rows)
+constexpr int kNumStages = 4;
+constexpr int kStageBytes = 128 * kPairK * 2;     // 16 KB ring slot (N/2 <= 128 rows)
 template <class Prog>
 struct PairLayout {
   __host__ __device__ static constexpr int ktot(int s) { return (Prog::nk_h(s) + Prog::nk_x(s)) * kKStage; }
@@ -169,7 +169,7 @@ constexpr int kDz8Top = 6;                         // max|d_pre| * scale lies in
 // fp32 scratch at the head of the training workspace (zeroed by every backward call): the weight-gradient kernel's
 // work-item counter (a uint32), Y = h7^T d(rgb_pre) [256 x 4], Yd = PE(dir)^T d(rgb_pre) [32 x 4] and sum d(rgb_pre) [4]
 // -- the rank-3 factors of every gradient that contains d(rgb_features) (tc_finish_kernel).  The counter lies below
-// kXOffS: a weight-gradient-only call over fp8 records zeroes only [0, kXOffS).
+// kXOffS: a weight-gradient-only call zeroes only [0, kXOffS).
 constexpr int kXOffQueue = 0;
 constexpr int kXOffY = 4;
 constexpr int kXOffYd = kXOffY + 256 * 4;
@@ -194,8 +194,8 @@ __host__ __device__ inline float dz8_scale(uint32_t amax_bits, bool inverse) {
 struct ChainSmem {
   uint8_t hs[2][kHSBytes];
   uint8_t xs[2][kXSBytes];
-  uint8_t stage[kNumStages2][kStageBytes2];
-  uint64_t full[kNumStages2], empty[kNumStages2], a_ready[2], acc_ready[2], st_ready[2], st_done[2];
+  uint8_t stage[kNumStages][kStageBytes];
+  uint64_t full[kNumStages], empty[kNumStages], a_ready[2], acc_ready[2], st_ready[2], st_done[2];
   uint32_t tmem_base;
   uint32_t items_issued;      // ordered mode: ring items whose MMAs have been issued (the two issuers take turns)
   uint32_t first_issued[2];   // unordered mode, per tile slot: GEMM steps whose first (accumulate = 0) MMA is issued

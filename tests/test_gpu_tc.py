@@ -253,7 +253,7 @@ def test_umma_selftest_2cta(N, K):
 @pytest.mark.parametrize("records", RECORDS)
 @pytest.mark.parametrize("R,S", [(37, 192), (300, 64), (1031, 192)])
 def test_tc_training_kernels_are_bit_reproducible(R, S, records):
-    """The chain kernels have TWO MMA-issuing threads (tc_roles2.cuh).  When training they hand over in ring order,
+    """The chain kernels have TWO MMA-issuing threads (tc_roles.cuh).  When training they hand over in ring order,
     so the fp32 accumulation order is fixed: forward output, activation / ReLU' records and the dZ records are
     bit-identical run after run; weight gradients differ only by the order of the fp32 atomics.  At inference the
     issuers run free by default (last-bit differences allowed) and the per-call option KNERF_TC_ORDERED restores the
