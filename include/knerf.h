@@ -123,6 +123,29 @@ int knerf_generate_ray_batch(const float* images, int n_img, int H, int W, int C
                              int64_t first, int64_t R, const float* u, uint64_t seed, float* o, float* d, float* t,
                              float* target, int64_t* pixel, void* stream);
 
+/* ---- forward-facing scenes: rays in normalized device coordinates (vanilla NeRF's ndc_rays; LLFF datasets) --------
+ * The same arguments and ray ids as knerf_generate_rays / knerf_generate_ray_batch, without near/far.  Per ray:
+ *  1. the world ray as knerf_generate_rays computes it: origin c2w[:3,3], unit direction w;
+ *  2. ndc_rays(H, W, focal, near = 1, o, w): tau = -(1 + o_z) / w_z, o' = o + tau*w (per component: tau*w_i, then
+ *     o_i + that), rx = o'_x/o'_z, ry = o'_y/o'_z, q = 2/o'_z, sx = (-2*focal)/W, sy = (-2*focal)/H;
+ *     o_ndc = (sx*rx, sy*ry, 1 + q),  d_ndc = (sx*(w_x/w_z - rx), sy*(w_y/w_z - ry), -q);
+ *  3. o = o_ndc, d = d_ndc / |d_ndc| (|.| = sqrt((x*x + y*y) + z*z));
+ *  4. t[k] = |d_ndc| * s_k, with s_k the stratified depth knerf_generate_rays computes for near = 0, far = 1 (the
+ *     same linspace end points, interval, jitter, clamp, and the same u indexing or Philox counters).
+ * Every operation is rounded on its own (no fused multiply-add), in the order written.  So o + d*t is
+ * o_ndc + s*d_ndc up to rounding, and the compositing step's delta t is vanilla's delta s * |d_ndc|.  The view
+ * direction the MLP sees is normalize(d_ndc), not the world direction: NDC maps lines to lines, so at a sample point
+ * one determines the other (a reparametrisation of the same input).  The batch variant gives every pixel the bits
+ * the whole-view variant gives it.
+ * Rays with w_z >= 0 in the given frame have no NDC image: their outputs are unspecified (callers refuse such views).
+ * KNERF_ERR_INVALID as for the non-NDC functions, before any device work.                                          */
+int knerf_generate_rays_ndc(const float* c2w_host, int H, int W, float focal, int n_samples, const float* u,
+                            uint64_t seed, float* o, float* d, float* t, void* stream);
+int knerf_generate_ray_batch_ndc(const float* images, int n_img, int H, int W, int C, const float* c2w, float focal,
+                                 int n_samples, uint64_t perm_seed, uint64_t epoch, int64_t first, int64_t R,
+                                 const float* u, uint64_t seed, float* o, float* d, float* t, float* target,
+                                 int64_t* pixel, void* stream);
+
 /* tf.random.uniform stand-in: n floats, multiples of 2^-24 in [0,1), Philox4x32-10(seed, offset) */
 int knerf_uniform(float* out, int64_t n, uint64_t seed, uint64_t offset, void* stream);
 

@@ -2,6 +2,8 @@
 // HBM-write-bound: 24 + 4*N bytes per ray out (+ 4*N in when the uniforms are supplied).
 // Random ray batches over all training views (knerf_generate_ray_batch): the same per-ray arithmetic, plus the target
 // rgb, 24 + 4*N + 12 bytes out and one scattered 16-byte read per ray.
+// Forward-facing scenes (knerf_generate_rays_ndc, knerf_generate_ray_batch_ndc): the same kernels instantiated with
+// NDC = true map each world ray into normalized device coordinates (ndc_map) and scale its depths; same traffic.
 #include "common.cuh"
 
 namespace knerf {
@@ -45,9 +47,11 @@ struct Strata {
   }
 };
 
-template <int VEC>
+// NDC: sample k of ray r is written as scale[r] * s_k (scale = the warp's 32 NDC direction norms, in shared memory).
+template <int VEC, bool NDC = false>
 __device__ __forceinline__ void stream_samples(const Strata& s, uint32_t base, uint32_t n, uint32_t lane,
-                                               const float* __restrict__ u, uint64_t seed, float* __restrict__ t) {
+                                               const float* __restrict__ u, uint64_t seed, float* __restrict__ t,
+                                               const float* scale = nullptr) {
   const int N = s.N;
   const uint32_t per_ray = (uint32_t)(N / VEC);
   const uint32_t units = n * per_ray;
@@ -85,6 +89,11 @@ __device__ __forceinline__ void stream_samples(const Strata& s, uint32_t base, u
       const float noise = __fsub_rn(__fmul_rn(uu[k], s.interval), s.half_iv);   // rays.py:122-123
       out[k] = fminf(fmaxf(__fadd_rn(lin, noise), s.near_), s.far_);            // rays.py:126-127
     }
+    if (NDC) {
+      const float sc = scale[r];
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) out[k] = __fmul_rn(sc, out[k]);
+    }
     if (VEC == 4) {
       *reinterpret_cast<float4*>(t + e0) = make_float4(out[0], out[1 % VEC], out[2 % VEC], out[3 % VEC]);
     } else {
@@ -93,10 +102,46 @@ __device__ __forceinline__ void stream_samples(const Strata& s, uint32_t base, u
   }
 }
 
+// Vanilla NeRF's ndc_rays(H, W, focal, near = 1, o, w) for a ray of origin o and direction w (w_z < 0): shift o to the
+// plane z = -1, o' = o + tau*w with tau = -(1 + o_z)/w_z, then
+//   o_ndc = (sx*o'_x/o'_z, sy*o'_y/o'_z, 1 + 2/o'_z),  d_ndc = (sx*(w_x/w_z - o'_x/o'_z), sy*(w_y/w_z - o'_y/o'_z), -2/o'_z)
+// with sx = -2f/W, sy = -2f/H.  Writes o_ndc and d_ndc/|d_ndc| and returns |d_ndc|.  Every operation is rounded on its
+// own (no contraction) in this order; tests/test_gpu_llff.py restates it in NumPy fp32 bit for bit.
+struct NdcMap {
+  float sx, sy;
+  __device__ __forceinline__ NdcMap(float focal, float Wf, float Hf) {
+    sx = __fdiv_rn(-2.0f * focal, Wf);
+    sy = __fdiv_rn(-2.0f * focal, Hf);
+  }
+  __device__ __forceinline__ float operator()(const float (&o)[3], const float (&w)[3], float (&o_ndc)[3],
+                                              float (&d_ndc)[3]) const {
+    const float tau = __fdiv_rn(-__fadd_rn(1.0f, o[2]), w[2]);
+    float op[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) op[i] = __fadd_rn(o[i], __fmul_rn(tau, w[i]));
+    const float rx = __fdiv_rn(op[0], op[2]), ry = __fdiv_rn(op[1], op[2]);
+    const float q = __fdiv_rn(2.0f, op[2]);
+    o_ndc[0] = __fmul_rn(sx, rx);
+    o_ndc[1] = __fmul_rn(sy, ry);
+    o_ndc[2] = __fadd_rn(1.0f, q);
+    float dn[3];
+    dn[0] = __fmul_rn(sx, __fsub_rn(__fdiv_rn(w[0], w[2]), rx));
+    dn[1] = __fmul_rn(sy, __fsub_rn(__fdiv_rn(w[1], w[2]), ry));
+    dn[2] = -q;
+    const float nrm = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(dn[0], dn[0]), __fmul_rn(dn[1], dn[1])),
+                                           __fmul_rn(dn[2], dn[2])));
+#pragma unroll
+    for (int i = 0; i < 3; ++i) d_ndc[i] = __fdiv_rn(dn[i], nrm);
+    return nrm;
+  }
+};
+
 // One warp per 32 consecutive rays.  Phase 1: lane l computes origin and direction of ray base + l (every lane busy:
 // the two divisions, the normalisation and its three divisions cost the warp one pass per 32 rays instead of one per
 // ray).  Phase 2: stream_samples.  Index arithmetic is 32-bit.
-template <int VEC>
+// NDC (near_ = 0, far_ = 1): phase 1 writes the NDC ray and keeps |d_ndc| in the warp's slot of shared memory, which
+// phase 2 reads for the depth scale (no shuffles in its divergent loop).
+template <int VEC, bool NDC>
 __global__ void __launch_bounds__(256) rays_kernel(Pose pose, int H, int W, float focal, float near_,
                                                    float far_, int N, const float* __restrict__ u,
                                                    uint64_t seed, float* __restrict__ o,
@@ -104,6 +149,8 @@ __global__ void __launch_bounds__(256) rays_kernel(Pose pose, int H, int W, floa
   const uint32_t n_rays = (uint32_t)H * (uint32_t)W;
   const float Wf = (float)W, Hf = (float)H;
   const Strata strata(near_, far_, N);
+  __shared__ float ndc_norm[NDC ? 256 : 1];
+  const NdcMap ndc(focal, Wf, Hf);
   const uint32_t lane = threadIdx.x & 31;
   const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
   for (uint32_t base = warp * 32; base < n_rays; base += n_warps * 32) {
@@ -112,13 +159,30 @@ __global__ void __launch_bounds__(256) rays_kernel(Pose pose, int H, int W, floa
       const uint32_t y = ray / (uint32_t)W, x = ray - y * (uint32_t)W;
       float dir[3];
       camera_direction(pose, x, y, Wf, Hf, focal, dir);
+      if constexpr (NDC) {
+        float on[3], dn[3];
+        ndc_norm[threadIdx.x] = ndc(pose.t, dir, on, dn);
 #pragma unroll
-      for (int i = 0; i < 3; ++i) {
-        d[(size_t)ray * 3 + i] = dir[i];
-        o[(size_t)ray * 3 + i] = pose.t[i];                // rays.py:112-113
+        for (int i = 0; i < 3; ++i) {
+          d[(size_t)ray * 3 + i] = dn[i];
+          o[(size_t)ray * 3 + i] = on[i];
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          d[(size_t)ray * 3 + i] = dir[i];
+          o[(size_t)ray * 3 + i] = pose.t[i];                // rays.py:112-113
+        }
       }
     }
-    stream_samples<VEC>(strata, base, min(32u, n_rays - base), lane, u, seed, t);
+    if constexpr (NDC) {
+      __syncwarp();
+      stream_samples<VEC, true>(strata, base, min(32u, n_rays - base), lane, u, seed, t,
+                                ndc_norm + (threadIdx.x & ~31u));
+      __syncwarp();                                          // the slot is rewritten by the next pass
+    } else {
+      stream_samples<VEC>(strata, base, min(32u, n_rays - base), lane, u, seed, t);
+    }
   }
 }
 
@@ -159,8 +223,8 @@ struct EpochPerm {
 
 // One warp per 32 consecutive batch rays.  Phase 1: lane l finds the pixel of ray base + l, reads its pose and its
 // rgb (one scattered 16-byte load when C == 4) and writes o, d, target (and pixel).  Phase 2: stream_samples with
-// batch-local counters, exactly as rays_kernel.
-template <int VEC>
+// batch-local counters, exactly as rays_kernel (NDC as there).
+template <int VEC, bool NDC>
 __global__ void __launch_bounds__(256) ray_batch_kernel(const float* __restrict__ images, int H, int W, int C,
                                                         bool rgba16, const float* __restrict__ c2w, float focal,
                                                         float near_, float far_, int N, EpochPerm perm,
@@ -171,6 +235,8 @@ __global__ void __launch_bounds__(256) ray_batch_kernel(const float* __restrict_
   const uint64_t HW = (uint64_t)H * (uint64_t)W;
   const float Wf = (float)W, Hf = (float)H;
   const Strata strata(near_, far_, N);
+  __shared__ float ndc_norm[NDC ? 256 : 1];
+  const NdcMap ndc(focal, Wf, Hf);
   const uint32_t lane = threadIdx.x & 31;
   const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
   for (uint32_t base = warp * 32; base < n_rays; base += n_warps * 32) {
@@ -199,15 +265,33 @@ __global__ void __launch_bounds__(256) ray_batch_kernel(const float* __restrict_
 #pragma unroll
         for (int i = 0; i < 3; ++i) rgb[i] = __ldg(px + i);
       }
+      if constexpr (NDC) {
+        float on[3], dn[3];
+        ndc_norm[threadIdx.x] = ndc(pose.t, dir, on, dn);
 #pragma unroll
-      for (int i = 0; i < 3; ++i) {
-        d[(size_t)ray * 3 + i] = dir[i];
-        o[(size_t)ray * 3 + i] = pose.t[i];
-        target[(size_t)ray * 3 + i] = rgb[i];
+        for (int i = 0; i < 3; ++i) {
+          d[(size_t)ray * 3 + i] = dn[i];
+          o[(size_t)ray * 3 + i] = on[i];
+          target[(size_t)ray * 3 + i] = rgb[i];
+        }
+      } else {
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+          d[(size_t)ray * 3 + i] = dir[i];
+          o[(size_t)ray * 3 + i] = pose.t[i];
+          target[(size_t)ray * 3 + i] = rgb[i];
+        }
       }
       if (pixel != nullptr) pixel[ray] = (int64_t)p;
     }
-    stream_samples<VEC>(strata, base, min(32u, n_rays - base), lane, u, seed, t);
+    if constexpr (NDC) {
+      __syncwarp();
+      stream_samples<VEC, true>(strata, base, min(32u, n_rays - base), lane, u, seed, t,
+                                ndc_norm + (threadIdx.x & ~31u));
+      __syncwarp();
+    } else {
+      stream_samples<VEC>(strata, base, min(32u, n_rays - base), lane, u, seed, t);
+    }
   }
 }
 
@@ -230,12 +314,16 @@ __global__ void __launch_bounds__(256) uniform_kernel(float* __restrict__ out, i
 
 using namespace knerf;
 
-extern "C" int knerf_generate_rays(const float* c2w_host, int H, int W, float focal, float near_,
-                                   float far_, int n_samples, const float* u, uint64_t seed, float* o,
-                                   float* d, float* t, void* stream) {
-  KN_CHECK_ARG(c2w_host && o && d && t, "knerf_generate_rays: null pointer");
-  KN_CHECK_ARG(H > 0 && W > 0 && n_samples > 0 && focal > 0.f, "knerf_generate_rays: bad shape H=%d W=%d N=%d focal=%g",
-               H, W, n_samples, (double)focal);
+namespace {
+
+// The argument checks and launch of knerf_generate_rays and knerf_generate_rays_ndc (`fn` names the entry point in the
+// messages); the NDC instantiation stratifies [0, 1] and scales each ray's depths by |d_ndc| in the kernel.
+template <bool NDC>
+int launch_rays(const char* fn, const float* c2w_host, int H, int W, float focal, float near_, float far_,
+                int n_samples, const float* u, uint64_t seed, float* o, float* d, float* t, void* stream) {
+  KN_CHECK_ARG(c2w_host && o && d && t, "%s: null pointer", fn);
+  KN_CHECK_ARG(H > 0 && W > 0 && n_samples > 0 && focal > 0.f, "%s: bad shape H=%d W=%d N=%d focal=%g", fn, H, W,
+               n_samples, (double)focal);
   Pose p;
   for (int i = 0; i < 3; ++i) {
     for (int j = 0; j < 3; ++j) p.r[i][j] = c2w_host[i * 4 + j];   // rays.py:99
@@ -245,32 +333,31 @@ extern "C" int knerf_generate_rays(const float* c2w_host, int H, int W, float fo
   const bool vec = (n_samples % 4 == 0) && ((reinterpret_cast<uintptr_t>(t) & 15) == 0) &&
                    (u == nullptr || (reinterpret_cast<uintptr_t>(u) & 15) == 0);
   KN_CHECK_ARG((int64_t)H * W < (int64_t)1 << 31 && (int64_t)n_samples * 32 < (int64_t)1 << 31,
-               "knerf_generate_rays: image too large (%d x %d)", H, W);
+               "%s: image too large (%d x %d)", fn, H, W);
   const int grid = (int)std::min<int64_t>(cdiv((int64_t)H * W, 256), (int64_t)kNumSMs * 16);
   if (vec)
-    rays_kernel<4><<<grid, 256, 0, st>>>(p, H, W, focal, near_, far_, n_samples, u, seed, o, d, t);
+    rays_kernel<4, NDC><<<grid, 256, 0, st>>>(p, H, W, focal, near_, far_, n_samples, u, seed, o, d, t);
   else
-    rays_kernel<1><<<grid, 256, 0, st>>>(p, H, W, focal, near_, far_, n_samples, u, seed, o, d, t);
+    rays_kernel<1, NDC><<<grid, 256, 0, st>>>(p, H, W, focal, near_, far_, n_samples, u, seed, o, d, t);
   KN_LAUNCH_CHECK();
   return KNERF_OK;
 }
 
-extern "C" int knerf_generate_ray_batch(const float* images, int n_img, int H, int W, int C, const float* c2w,
-                                        float focal, float near_, float far_, int n_samples, uint64_t perm_seed,
-                                        uint64_t epoch, int64_t first, int64_t R, const float* u, uint64_t seed,
-                                        float* o, float* d, float* t, float* target, int64_t* pixel, void* stream) {
-  KN_CHECK_ARG(images && c2w && o && d && t && target, "knerf_generate_ray_batch: null pointer");
+template <bool NDC>
+int launch_ray_batch(const char* fn, const float* images, int n_img, int H, int W, int C, const float* c2w,
+                     float focal, float near_, float far_, int n_samples, uint64_t perm_seed, uint64_t epoch,
+                     int64_t first, int64_t R, const float* u, uint64_t seed, float* o, float* d, float* t,
+                     float* target, int64_t* pixel, void* stream) {
+  KN_CHECK_ARG(images && c2w && o && d && t && target, "%s: null pointer", fn);
   KN_CHECK_ARG(n_img > 0 && H > 0 && W > 0 && n_samples > 0 && focal > 0.f,
-               "knerf_generate_ray_batch: bad shape n_img=%d H=%d W=%d N=%d focal=%g", n_img, H, W, n_samples,
-               (double)focal);
-  KN_CHECK_ARG(C >= 3, "knerf_generate_ray_batch: C=%d channels, need >= 3", C);
+               "%s: bad shape n_img=%d H=%d W=%d N=%d focal=%g", fn, n_img, H, W, n_samples, (double)focal);
+  KN_CHECK_ARG(C >= 3, "%s: C=%d channels, need >= 3", fn, C);
   KN_CHECK_ARG((int64_t)H * W < (int64_t)1 << 31 && (int64_t)n_samples * 32 < (int64_t)1 << 31,
-               "knerf_generate_ray_batch: image too large (%d x %d)", H, W);
+               "%s: image too large (%d x %d)", fn, H, W);
   const int64_t P = (int64_t)n_img * H * W;
-  KN_CHECK_ARG(first >= 0 && R >= 0 && first <= P - R,
-               "knerf_generate_ray_batch: window [%lld, %lld + %lld) outside [0, %lld)", (long long)first,
-               (long long)first, (long long)R, (long long)P);
-  KN_CHECK_ARG(R < (int64_t)1 << 31, "knerf_generate_ray_batch: R=%lld rays per call, need < 2^31", (long long)R);
+  KN_CHECK_ARG(first >= 0 && R >= 0 && first <= P - R, "%s: window [%lld, %lld + %lld) outside [0, %lld)", fn,
+               (long long)first, (long long)first, (long long)R, (long long)P);
+  KN_CHECK_ARG(R < (int64_t)1 << 31, "%s: R=%lld rays per call, need < 2^31", fn, (long long)R);
   if (R == 0) return KNERF_OK;
   EpochPerm perm;
   perm.P = (uint64_t)P;
@@ -285,13 +372,44 @@ extern "C" int knerf_generate_ray_batch(const float* images, int n_img, int H, i
   const bool rgba16 = C == 4 && (reinterpret_cast<uintptr_t>(images) & 15) == 0;
   const int grid = (int)std::min<int64_t>(cdiv(R, 256), (int64_t)kNumSMs * 16);
   if (vec)
-    ray_batch_kernel<4><<<grid, 256, 0, st>>>(images, H, W, C, rgba16, c2w, focal, near_, far_, n_samples, perm,
-                                              first, (uint32_t)R, u, seed, o, d, t, target, pixel);
+    ray_batch_kernel<4, NDC><<<grid, 256, 0, st>>>(images, H, W, C, rgba16, c2w, focal, near_, far_, n_samples,
+                                                   perm, first, (uint32_t)R, u, seed, o, d, t, target, pixel);
   else
-    ray_batch_kernel<1><<<grid, 256, 0, st>>>(images, H, W, C, rgba16, c2w, focal, near_, far_, n_samples, perm,
-                                              first, (uint32_t)R, u, seed, o, d, t, target, pixel);
+    ray_batch_kernel<1, NDC><<<grid, 256, 0, st>>>(images, H, W, C, rgba16, c2w, focal, near_, far_, n_samples,
+                                                   perm, first, (uint32_t)R, u, seed, o, d, t, target, pixel);
   KN_LAUNCH_CHECK();
   return KNERF_OK;
+}
+
+}  // namespace
+
+extern "C" int knerf_generate_rays(const float* c2w_host, int H, int W, float focal, float near_,
+                                   float far_, int n_samples, const float* u, uint64_t seed, float* o,
+                                   float* d, float* t, void* stream) {
+  return launch_rays<false>("knerf_generate_rays", c2w_host, H, W, focal, near_, far_, n_samples, u, seed, o, d, t,
+                            stream);
+}
+
+extern "C" int knerf_generate_rays_ndc(const float* c2w_host, int H, int W, float focal, int n_samples,
+                                       const float* u, uint64_t seed, float* o, float* d, float* t, void* stream) {
+  return launch_rays<true>("knerf_generate_rays_ndc", c2w_host, H, W, focal, 0.0f, 1.0f, n_samples, u, seed, o, d,
+                           t, stream);
+}
+
+extern "C" int knerf_generate_ray_batch(const float* images, int n_img, int H, int W, int C, const float* c2w,
+                                        float focal, float near_, float far_, int n_samples, uint64_t perm_seed,
+                                        uint64_t epoch, int64_t first, int64_t R, const float* u, uint64_t seed,
+                                        float* o, float* d, float* t, float* target, int64_t* pixel, void* stream) {
+  return launch_ray_batch<false>("knerf_generate_ray_batch", images, n_img, H, W, C, c2w, focal, near_, far_,
+                                 n_samples, perm_seed, epoch, first, R, u, seed, o, d, t, target, pixel, stream);
+}
+
+extern "C" int knerf_generate_ray_batch_ndc(const float* images, int n_img, int H, int W, int C, const float* c2w,
+                                            float focal, int n_samples, uint64_t perm_seed, uint64_t epoch,
+                                            int64_t first, int64_t R, const float* u, uint64_t seed, float* o,
+                                            float* d, float* t, float* target, int64_t* pixel, void* stream) {
+  return launch_ray_batch<true>("knerf_generate_ray_batch_ndc", images, n_img, H, W, C, c2w, focal, 0.0f, 1.0f,
+                                n_samples, perm_seed, epoch, first, R, u, seed, o, d, t, target, pixel, stream);
 }
 
 extern "C" int knerf_uniform(float* out, int64_t n, uint64_t seed, uint64_t offset, void* stream) {

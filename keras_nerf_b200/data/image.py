@@ -24,13 +24,39 @@ def decode_image_rgba(source) -> np.ndarray:
         return np.array(im.convert("RGBA"), dtype=np.uint8)   # a writable copy
 
 
+def as_rgba_uint8(image) -> torch.Tensor:
+    """path / encoded bytes / decoded [H,W,3|4] uint8 array or tensor -> [H,W,4] uint8 tensor (opaque alpha added)"""
+    if torch.is_tensor(image) or isinstance(image, np.ndarray):
+        rgba = torch.as_tensor(image)
+        if rgba.dtype != torch.uint8 or rgba.dim() != 3 or rgba.shape[-1] not in (3, 4):
+            raise ValueError("decoded images must be [H,W,3|4] uint8")
+        if rgba.shape[-1] == 3:                         # decode_image(channels=4) gives opaque alpha
+            rgba = torch.cat([rgba, torch.full_like(rgba[..., :1], 255)], dim=-1)
+        return rgba
+    return torch.from_numpy(decode_image_rgba(image))
+
+
+def prepare_image(image, out_h: int, out_w: int, white_background: bool = False, device=None) -> torch.Tensor:
+    """`knerf_image_prepare` on one image: -> float32 CUDA tensor [out_h, out_w, 4] (antialiased bilinear resize,
+    rgb composited on the background, alpha).  `image` as `as_rgba_uint8` takes it."""
+    device = device or _lib.default_device()
+    rgba = as_rgba_uint8(image).contiguous().to(device, non_blocking=True)
+    in_h, in_w = int(rgba.shape[0]), int(rgba.shape[1])
+    with torch.cuda.device(device):
+        out = torch.empty((int(out_h), int(out_w), 4), dtype=torch.float32, device=device)
+        _lib.call("knerf_image_prepare", _lib.ptr(rgba, torch.uint8), in_h, in_w, int(out_h), int(out_w),
+                  int(white_background), _lib.ptr(out), _lib.stream())
+    return out
+
+
 class ImageLoader:
     """Same constructor and call signature as keras_nerf/data/image.py:4-35.
 
     `__call__(image_path)` -> float32 CUDA tensor [image_width, image_height, 4] (rgb composited on the
     background, alpha), i.e. the reference's axis order: it hands (image_width, image_height) to
     tf.image.resize as (height, width) (image.py:22-23); identical for the square images of nerf_synthetic.
-    Also accepts encoded bytes or an already decoded [H,W,3|4] uint8 array / tensor.
+    Also accepts encoded bytes or an already decoded [H,W,3|4] uint8 array / tensor.  `prepare_image` takes
+    (out_h, out_w) in the usual order.
     """
 
     def __init__(self, image_width: int, image_height: int, white_background: bool = False, device=None, **kwargs):
@@ -40,20 +66,5 @@ class ImageLoader:
         self.device = torch.device(device) if device is not None else None
 
     def __call__(self, image_path) -> torch.Tensor:
-        device = self.device or _lib.default_device()
-        if torch.is_tensor(image_path) or isinstance(image_path, np.ndarray):
-            rgba = torch.as_tensor(image_path)
-            if rgba.dtype != torch.uint8 or rgba.dim() != 3 or rgba.shape[-1] not in (3, 4):
-                raise ValueError("decoded images must be [H,W,3|4] uint8")
-            if rgba.shape[-1] == 3:                         # decode_image(channels=4) gives opaque alpha
-                rgba = torch.cat([rgba, torch.full_like(rgba[..., :1], 255)], dim=-1)
-        else:
-            rgba = torch.from_numpy(decode_image_rgba(image_path))
-        rgba = rgba.contiguous().to(device, non_blocking=True)
-        in_h, in_w = int(rgba.shape[0]), int(rgba.shape[1])
-        out_h, out_w = self.image_width, self.image_height   # (sic) image.py:22-23
-        with torch.cuda.device(device):
-            out = torch.empty((out_h, out_w, 4), dtype=torch.float32, device=device)
-            _lib.call("knerf_image_prepare", _lib.ptr(rgba, torch.uint8), in_h, in_w, out_h, out_w,
-                      int(self.white_background), _lib.ptr(out), _lib.stream())
-        return out
+        # (sic) image.py:22-23: out_h, out_w = image_width, image_height
+        return prepare_image(image_path, self.image_width, self.image_height, self.white_background, self.device)

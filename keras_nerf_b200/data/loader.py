@@ -112,10 +112,11 @@ class RayBatchDataset:
 
     `images` [n_img, H, W, C] (CUDA fp32, C >= 3) is the prepared view cache (n*H*W*16 bytes for RGBA: 256 MB for 100
     views of 400 x 400), `poses` [n_img, 4, 4].  `epoch` is the epoch the next pass walks; each pass advances it, and a
-    resumed run sets it to the first epoch it trains."""
+    resumed run sets it to the first epoch it trains.  `ndc=True` draws the rays of forward-facing scenes in
+    normalized device coordinates (`generate_ray_batch(..., ndc=True)`; near and far unused)."""
 
     def __init__(self, images, poses, focal, near, far, n_sample, ray_batch, rank=0, world=1, perm_seed=None,
-                 epoch=0, limit=None):
+                 epoch=0, limit=None, ndc=False):
         self.images = torch.as_tensor(images).contiguous()        # the kernel refuses anything but CUDA fp32
         self.poses = torch.as_tensor(poses, dtype=torch.float32, device=self.images.device).reshape(-1, 4, 4)
         self.poses = self.poses.contiguous()
@@ -131,6 +132,7 @@ class RayBatchDataset:
         self.perm_seed = permutation_seed() if perm_seed is None else int(perm_seed)
         self.epoch = int(epoch)
         self.limit = limit
+        self.ndc = bool(ndc)
 
     def window(self, step):
         """first position of this rank's batch `step` in the epoch's order"""
@@ -140,7 +142,7 @@ class RayBatchDataset:
         """batch `step` of epoch `epoch` of this rank: (targets, (o, d, t)) (+ pixel ids when `with_pixel`)"""
         out = generate_ray_batch(self.images, self.poses, self.focal, self.near, self.far, self.n_sample,
                                  self.perm_seed, epoch, self.window(step), self.ray_batch, u=u, seed=seed,
-                                 with_pixel=with_pixel)
+                                 with_pixel=with_pixel, ndc=self.ndc)
         return (out[0], tuple(out[1:4])) + ((out[4],) if with_pixel else ())
 
     def _batches(self, epoch):
@@ -159,7 +161,8 @@ class RayBatchDataset:
     def take(self, count):
         """the first `count` batches of each pass; the view cache is shared, the epoch counter is the copy's own"""
         return RayBatchDataset(self.images, self.poses, self.focal, self.near, self.far, self.n_sample,
-                               self.ray_batch, self.rank, self.world, self.perm_seed, self.epoch, limit=count)
+                               self.ray_batch, self.rank, self.world, self.perm_seed, self.epoch, limit=count,
+                               ndc=self.ndc)
 
 
 class DatasetLoader:

@@ -17,10 +17,14 @@ class RaysGenerator:
     `__call__(camera_params)` -> (ray_origin[H,W,3], ray_direction[H,W,3], sample_points[H,W,N]) as CUDA
     tensors.  The reference draws fresh `tf.random.uniform` jitter on every call; here the draws come
     from the library's Philox stream (a new seed per call) unless `u` [H,W,N] is passed explicitly.
+
+    `ndc=True` (forward-facing scenes, vanilla NeRF's `ndc_rays` with near plane 1): `knerf_generate_rays_ndc` writes
+    the rays in normalized device coordinates, o = o_ndc, d = normalize(d_ndc), t = |d_ndc| * s with s stratified on
+    [0, 1]; `near` and `far` are not used.
     """
 
     def __init__(self, focal_length: float, image_width: int, image_height: int, near: float, far: float,
-                 n_sample: int, device=None, **kwargs):
+                 n_sample: int, device=None, ndc: bool = False, **kwargs):
         self.focal_length = float(focal_length)
         self.image_width = int(image_width)
         self.image_height = int(image_height)
@@ -28,6 +32,7 @@ class RaysGenerator:
         self.far = float(far)
         self.n_sample = int(n_sample)
         self.device = torch.device(device) if device is not None else None
+        self.ndc = bool(ndc)
 
     def __call__(self, camera_params, u=None, seed=None):
         device = self.device or _lib.default_device()
@@ -43,17 +48,22 @@ class RaysGenerator:
                 u = _lib.dev(u, device).reshape(H, W, N)
             if seed is None:
                 seed = next(_seed_counter)
-            _lib.call("knerf_generate_rays", c2w.ctypes.data, H, W, self.focal_length, self.near, self.far, N,
-                      _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t), _lib.stream())
+            if self.ndc:
+                _lib.call("knerf_generate_rays_ndc", c2w.ctypes.data, H, W, self.focal_length, N, _lib.ptr(u),
+                          int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t), _lib.stream())
+            else:
+                _lib.call("knerf_generate_rays", c2w.ctypes.data, H, W, self.focal_length, self.near, self.far, N,
+                          _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t), _lib.stream())
         return o, d, t
 
 
 def generate_ray_batch(images, poses, focal, near, far, n_sample, perm_seed, epoch, first, n_rays, u=None, seed=None,
-                       with_pixel=False):
+                       with_pixel=False, ndc=False):
     """`knerf_generate_ray_batch`: rays first .. first+n_rays-1 of epoch `epoch` of the permutation keyed by
     `perm_seed` over every pixel of the view cache `images` [n_img, H, W, C] (CUDA fp32, C >= 3) with poses
     [n_img, 4, 4].  Returns (target[n,3], o[n,3], d[n,3], t[n,N]) (+ pixel[n] int64, id (img*H + y)*W + x, when
-    `with_pixel`).  The jitter comes from Philox(seed), a new seed per call unless given, or from `u` [n, N]."""
+    `with_pixel`).  The jitter comes from Philox(seed), a new seed per call unless given, or from `u` [n, N].
+    `ndc=True`: `knerf_generate_ray_batch_ndc`, the rays of RaysGenerator(..., ndc=True); near and far are not used."""
     n_img, H, W, C = images.shape
     device = images.device
     N = int(n_sample)
@@ -65,8 +75,12 @@ def generate_ray_batch(images, poses, focal, near, far, n_sample, perm_seed, epo
             u = _lib.dev(u, device).reshape(n_rays, N)
         if seed is None:
             seed = next(_seed_counter)
-        _lib.call("knerf_generate_ray_batch", _lib.ptr(images), n_img, H, W, C, _lib.ptr(poses), float(focal),
-                  float(near), float(far), N, int(perm_seed) & 0xFFFFFFFFFFFFFFFF, int(epoch) & 0xFFFFFFFFFFFFFFFF,
-                  int(first), int(n_rays), _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t),
-                  _lib.ptr(target), None if pixel is None else pixel.data_ptr(), _lib.stream())
+        head = (_lib.ptr(images), n_img, H, W, C, _lib.ptr(poses), float(focal))
+        tail = (N, int(perm_seed) & 0xFFFFFFFFFFFFFFFF, int(epoch) & 0xFFFFFFFFFFFFFFFF, int(first), int(n_rays),
+                _lib.ptr(u), int(seed), _lib.ptr(o), _lib.ptr(d), _lib.ptr(t), _lib.ptr(target),
+                None if pixel is None else pixel.data_ptr(), _lib.stream())
+        if ndc:
+            _lib.call("knerf_generate_ray_batch_ndc", *head, *tail)
+        else:
+            _lib.call("knerf_generate_ray_batch", *head, float(near), float(far), *tail)
     return (target, o, d, t, pixel) if with_pixel else (target, o, d, t)

@@ -101,3 +101,90 @@ def write_nerf_synthetic_like(data_dir: str, image_wh: int = 64, n_train: int = 
         with open(os.path.join(data_dir, f"transforms_{subset}.json"), "w") as f:
             json.dump({"camera_angle_x": LEGO_FOV, "frames": frames}, f)
     return data_dir
+
+
+# ---- a forward-facing scene in LLFF layout (data.llff) ----------------------------------------------------------------
+# Three spheres 1.9 to 7.7 units in front of the cameras and a textured back plane at depth 50: a depth ratio of about
+# 26, the situation NDC is for.  (centre, radius, albedo)
+LLFF_SPHERES = (((0.35, 0.15, -2.5), 0.6, (0.9, 0.35, 0.2)),
+                ((-0.9, -0.4, -4.2), 0.9, (0.25, 0.7, 0.35)),
+                ((1.2, 0.9, -6.5), 1.2, (0.3, 0.4, 0.9)))
+LLFF_PLANE_Z = -50.0
+
+
+def llff_like_poses(n_views: int, seed: int = 0) -> torch.Tensor:
+    """[n_views, 3, 4] camera-to-world matrices ([right, up, back] axes, cameras looking along -z) on a small planar
+    spiral of radius <= 0.3 at z = 0, each turned by up to 3 degrees about x and y"""
+    import math
+    g = torch.Generator().manual_seed(seed)
+    out = torch.zeros((n_views, 3, 4), dtype=torch.float64)
+    for k in range(n_views):
+        a = 2.0 * math.pi * 1.5 * k / max(n_views, 1)
+        r = 0.3 * (0.4 + 0.6 * (k + 1) / n_views)
+        yaw, pitch = (torch.rand(2, generator=g, dtype=torch.float64) * 2 - 1) * math.radians(3.0)
+        cy, sy, cp, sp = math.cos(yaw), math.sin(yaw), math.cos(pitch), math.sin(pitch)
+        ry = torch.tensor([[cy, 0, sy], [0, 1, 0], [-sy, 0, cy]], dtype=torch.float64)
+        rx = torch.tensor([[1, 0, 0], [0, cp, -sp], [0, sp, cp]], dtype=torch.float64)
+        out[k, :, :3] = ry @ rx
+        out[k, :, 3] = torch.tensor([r * math.cos(a), r * math.sin(a), 0.0], dtype=torch.float64)
+    return out
+
+
+def render_llff_like(c2w: torch.Tensor, H: int, W: int, focal: float) -> tuple:
+    """host ray trace of the forward-facing scene for one [3, 4] pose with the camera model of knerf_generate_rays
+    -> (rgb [H, W, 3] in [0, 1], camera-space depth [H, W])"""
+    ys, xs = torch.meshgrid(torch.arange(H, dtype=torch.float64), torch.arange(W, dtype=torch.float64), indexing="ij")
+    cam = torch.stack([(xs - W * 0.5) / focal, -(ys - H * 0.5) / focal, -torch.ones_like(xs)], -1)
+    c2w = c2w.to(torch.float64)
+    d = torch.nn.functional.normalize(cam @ c2w[:, :3].T, dim=-1)
+    o = c2w[:, 3].expand_as(d)
+    light = torch.nn.functional.normalize(torch.tensor([0.5, 0.8, 0.6], dtype=torch.float64), dim=0)
+    t_hit = (LLFF_PLANE_Z - o[..., 2]) / d[..., 2]                          # every ray of the frame looks down -z
+    p = o + d * t_hit[..., None]
+    # back plane: smooth colour waves (period about 6 units) and a checker of period 8
+    check = ((torch.floor(p[..., 0] / 4) + torch.floor(p[..., 1] / 4)) % 2)
+    rgb = torch.stack([0.5 + 0.3 * torch.sin(p[..., 0] * 1.05), 0.5 + 0.3 * torch.sin(p[..., 1] * 0.9 + 1.0),
+                       0.45 + 0.25 * torch.cos((p[..., 0] + p[..., 1]) * 0.7)], -1) * (0.75 + 0.25 * check[..., None])
+    for centre, radius, albedo in LLFF_SPHERES:
+        c = torch.tensor(centre, dtype=torch.float64)
+        oc = o - c
+        b = (oc * d).sum(-1)
+        disc = b * b - ((oc * oc).sum(-1) - radius * radius)
+        t = -b - torch.sqrt(disc.clamp_min(0))
+        hit = (disc > 0) & (t > 0) & (t < t_hit)
+        n = torch.nn.functional.normalize(oc + d * t[..., None], dim=-1)
+        stripes = 0.8 + 0.2 * torch.sin((n[..., 1] * 9.0))
+        shade = (0.35 + 0.65 * (n @ light).clamp_min(0)) * stripes
+        col = torch.tensor(albedo, dtype=torch.float64) * shade[..., None]
+        rgb = torch.where(hit[..., None], col, rgb)
+        t_hit = torch.where(hit, t, t_hit)
+    depth = t_hit * (d @ -c2w[:, 2])                                        # along the camera's viewing axis
+    return rgb.clamp(0, 1), depth
+
+
+def write_llff_like(data_dir: str, H: int = 48, W: int = 64, n_views: int = 20, factors=(), seed: int = 0) -> str:
+    """An LLFF-layout directory of the forward-facing analytic scene: `poses_bounds.npy` ([n_views, 17] in LLFF's own
+    [down, right, back] axis order, hwf = (H, W, focal), bounds = the view's nearest and farthest visible depth) and
+    `images/` PNGs of H x W, plus `images_{f}/` at (H // f, W // f) for every f in `factors`, rendered with focal / f.
+    Poses from `llff_like_poses(n_views, seed)`.  Host-only (torch CPU + Pillow)."""
+    import os
+
+    import numpy as np
+    from PIL import Image
+
+    focal = 0.9 * W
+    poses = llff_like_poses(n_views, seed)
+    rows = []
+    for f in (1,) + tuple(factors):
+        folder = os.path.join(data_dir, "images" if f == 1 else f"images_{f}")
+        os.makedirs(folder, exist_ok=True)
+        for k in range(n_views):
+            rgb, depth = render_llff_like(poses[k], H // f, W // f, focal / f)
+            png = (rgb.numpy() * 255.0 + 0.5).astype(np.uint8)
+            Image.fromarray(png, mode="RGB").save(os.path.join(folder, f"view_{k:03d}.png"))
+            if f == 1:
+                c2w = poses[k].numpy()
+                m = np.stack([-c2w[:, 1], c2w[:, 0], c2w[:, 2], c2w[:, 3], np.array([H, W, focal])], 1)
+                rows.append(np.concatenate([m.reshape(-1), [float(depth.min()), float(depth.max())]]))
+    np.save(os.path.join(data_dir, "poses_bounds.npy"), np.stack(rows).astype(np.float32))
+    return data_dir

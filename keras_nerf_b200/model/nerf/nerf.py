@@ -180,14 +180,18 @@ class NeRF:
     # ---- compile (nerf.py:78-173) -------------------------------------------------------------
     def compile(self, optimizer, loss, batch_size, image_height, image_width, ray_chunks, white_background=False,
                 is_training=True, **kwargs):
-        """nerf.py:78-173.  Keyword extensions: `fuse_chunks` (below) and `ray_batch`.
+        """nerf.py:78-173.  Keyword extensions: `fuse_chunks` (below), `ray_batch` and `train_ray_chunks`.
 
         ray_batch=N > 0: the training step takes N rays drawn across all views (data.loader.RayBatchDataset), so
         train_step((targets[N,3], (o[N,3], d[N,3], t[N,Nc]))) / accumulate_gradients take a flat ray batch, while
         batch_size / image_height / image_width keep describing what predict_and_render_images, test_step and the
         monitor render.  `ray_chunks` must divide N (checked like it is against the number of rays of an image batch)
         and `fuse_chunks` applies to the N rays.  The logs keep their keys: the PSNR is that of the batch MSE and the
-        SSIM is NaN (a ray batch has no 11x11 window)."""
+        SSIM is NaN (a ray batch has no 11x11 window).
+
+        train_ray_chunks=c (with ray_batch): the training step's chunk, which must divide N, while `ray_chunks` stays
+        the render chunk, which must divide the image batch's rays.  Default `ray_chunks` for both.  Image sizes and
+        ray batches that share no large divisor (an LLFF view of 378 x 504 and N = 4096 share 16) need the two apart."""
         self.run_eagerly = bool(kwargs.get("run_eagerly", False))
         self.optimizer, self.loss = optimizer, loss
         # The fused kernels implement the loss of the reference scripts: MeanSquaredError (train_single.py:127) or
@@ -212,7 +216,7 @@ class NeRF:
         if self.ray_batch:
             # the training step's own chunking; rendering keeps the chunks of the image batch
             self._train_rays = self.ray_batch
-            train_rc = min(ray_chunks, self.ray_batch)
+            train_rc = min(int(kwargs.get("train_ray_chunks") or ray_chunks), self.ray_batch)
             assert self.ray_batch % train_rc == 0, \
                 f'ray_chunks {train_rc} must be a divisor of the number of rays {self.ray_batch}'
         else:

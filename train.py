@@ -7,7 +7,11 @@ gradients are SUM-all-reduced over NCCL before the two Adam steps.
 
 --ray_batch N trains on N random rays per replica and step, drawn across all training views (an epoch visits every
 pixel once; data.loader.RayBatchDataset) instead of --batch_size whole views; validation and the monitor still
-render --batch_size whole views.  Under torchrun the ranks take disjoint windows of the same epoch order."""
+render --batch_size whole views.  Under torchrun the ranks take disjoint windows of the same epoch order.
+
+--dataset_type llff trains on a forward-facing LLFF scene (poses_bounds.npy + images/, data.llff.LLFFDatasetLoader):
+H, W and focal come from the dataset (--factor downsamples), every --llffhold-th view is held out, and the rays are in
+normalized device coordinates unless --no_ndc.  --img_wh, --near and --far are ignored then."""
 import argparse
 import logging
 import os
@@ -79,6 +83,12 @@ def main(argv=None, multi_gpu=True):
     parser.add_argument('--ray_batch', type=int, default=0,
                         help='train on this many random rays per replica and step, drawn across all training views '
                              '(0: --batch_size whole views per step, the reference\'s pipeline)')
+    parser.add_argument('--dataset_type', type=str, default='blender', choices=['blender', 'llff'],
+                        help="'blender': a nerf_synthetic directory (transforms_*.json); 'llff': a forward-facing "
+                             "scene (poses_bounds.npy + images/)")
+    parser.add_argument('--factor', type=int, default=8, help='llff: image downsampling factor')
+    parser.add_argument('--llffhold', type=int, default=8, help='llff: hold out every N-th view for val / test')
+    parser.add_argument('--no_ndc', action='store_true', help='llff: sample in world space between the bounds')
     args = parser.parse_args(argv)
     logging.basicConfig(level=logging.DEBUG if args.verbose else logging.INFO,
                         format='%(asctime)s | %(name)s | %(levelname)s | %(message)s')
@@ -91,11 +101,30 @@ def main(argv=None, multi_gpu=True):
         replicas, rank = strategy.num_replicas_in_sync, strategy.rank
     print('Number of devices: {}'.format(replicas))
 
-    loader = DatasetLoader(args.data_dir, args.white_bg)
-    datasets = loader.load_dataset(batch_size=args.batch_size * replicas, image_width=args.img_wh,
-                                   image_height=args.img_wh, near=args.near, far=args.far,
-                                   n_sample=args.num_coarse_samples, ray_batch=args.ray_batch, rank=rank,
-                                   world=replicas)
+    image_height = image_width = args.img_wh
+    train_ray_chunks = None                                  # the training step's chunk: --ray_chunks
+    if args.dataset_type == 'llff':
+        from keras_nerf_b200.data.llff import LLFFDatasetLoader, ray_chunks_for
+        loader = LLFFDatasetLoader(args.data_dir, factor=args.factor, llffhold=args.llffhold, ndc=not args.no_ndc)
+        image_height, image_width = loader.H, loader.W
+        logging.info(f"LLFF scene: {loader.H} x {loader.W}, focal {loader.focal:.3f}, "
+                     + ("NDC rays" if loader.ndc else f"near {loader.near:.4f}, far {loader.far:.4f}")
+                     + "; --img_wh, --near and --far are ignored")
+        datasets = loader.load_dataset(batch_size=args.batch_size * replicas, n_sample=args.num_coarse_samples,
+                                       ray_batch=args.ray_batch, rank=rank, world=replicas)
+        # the render chunk must divide the views' rays and the training chunk the ray batch: chosen apart, each as
+        # close to --ray_chunks as its size allows
+        render_chunks, train_ray_chunks = ray_chunks_for(args.batch_size * loader.H * loader.W, args.ray_batch,
+                                                         args.ray_chunks)
+        logging.info(f"ray chunks: {render_chunks} to render the {loader.H} x {loader.W} views, {train_ray_chunks} "
+                     f"per training chunk (--ray_chunks {args.ray_chunks})")
+        args.ray_chunks = render_chunks
+    else:
+        loader = DatasetLoader(args.data_dir, args.white_bg)
+        datasets = loader.load_dataset(batch_size=args.batch_size * replicas, image_width=args.img_wh,
+                                       image_height=args.img_wh, near=args.near, far=args.far,
+                                       n_sample=args.num_coarse_samples, ray_batch=args.ray_batch, rank=rank,
+                                       world=replicas)
     if strategy is not None:
         # a ray-batch train split is already this rank's share
         split = 1 if args.ray_batch else 0
@@ -121,9 +150,9 @@ def main(argv=None, multi_gpu=True):
     logging.info("Last epoch: {}".format(last_epoch))
     if args.ray_batch:
         train_dataset.epoch = last_epoch                     # continue the permutation sequence, do not replay epoch 0
-    nerf.compile(optimizer='adam', loss='mean_squared_error', batch_size=args.batch_size, image_width=args.img_wh,
-                 image_height=args.img_wh, ray_chunks=args.ray_chunks, run_eagerly=args.eagerly,
-                 white_background=args.white_bg, ray_batch=args.ray_batch,
+    nerf.compile(optimizer='adam', loss='mean_squared_error', batch_size=args.batch_size, image_width=image_width,
+                 image_height=image_height, ray_chunks=args.ray_chunks, run_eagerly=args.eagerly,
+                 white_background=args.white_bg, ray_batch=args.ray_batch, train_ray_chunks=train_ray_chunks,
                  fuse_chunks=None if args.fuse_chunks == 'off' else
                  ('auto' if args.fuse_chunks == 'auto' else int(args.fuse_chunks)))
     if strategy is not None:
