@@ -7,7 +7,7 @@
 
 fwd: the forward kernel at inference (train=0) and training (train=1).  dgrad: forward, then three dgrad-only backward
 calls; the counters of the last one are read.  Counters are CTA means (tc_roles.cuh slots); `epilogue cycles per step`
-are per work unit (two tiles per CTA) and tile slot, `prologue` (dgrad) the same for the tile's first A operand."""
+are per work unit (two tiles per CTA) and tile slot, `prologue` the same for the tile's first A operand."""
 import ctypes as C
 import os
 import sys
@@ -57,8 +57,7 @@ def main():
               f"compute-wait-acc {m[4]/1e3:.0f}, compute-total {m[5]/1e3:.0f}")
         for tl in range(2):
             line = " ".join(f"{m[6 + tl * 16 + s] / units:.0f}" for s in range(steps))
-            if steps == 8:
-                line += f"; prologue {m[15 + tl * 16] / units:.0f}"
+            line += f"; prologue {m[15 + tl * 16] / units:.0f}"
             print(f"  epilogue cycles per step, tile slot {tl}: {line}")
         return True
 

@@ -370,115 +370,63 @@ __global__ void __launch_bounds__(kThreads, 1)
 tc_mlp_fwd_kernel(const uint8_t* __restrict__ packed, const float* __restrict__ o, const float* __restrict__ d,
                   const float* __restrict__ t, int64_t M, int S, float4* __restrict__ rgbsigma,
                   uint8_t* __restrict__ rec, int ordered) {
-  using Prog = FwdProg;
-  constexpr int kLast = Prog::kSteps - 1;
+  constexpr int kLast = FwdProg::kSteps - 1;
   constexpr int kRB = REC8 ? kRec8Bytes : kRecBytes, kOffXS = REC8 ? kRec8XS : kRecXS, kOffDS = REC8 ? kRec8DS : kRecDS,
                 kOffMask = REC8 ? kRec8Mask : kRecMask;
+  constexpr bool kStore = TRAIN && !REC8;   // bf16 records: the operand tiles h0..h7 -> HBM through the store warp
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   ChainSmem& sm = *reinterpret_cast<ChainSmem*>(smem_raw);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int64_t n_tiles = (M + kTileM - 1) / kTileM;
-  const int64_t n_pairs = (n_tiles + 3) / 4;   // work units: four tiles per CTA pair
-  const uint32_t cta = cluster_ctarank();
-  const int64_t first = blockIdx.x >> 1, stride = gridDim.x >> 1;
-  const uint32_t tmem = chain_setup(sm, tid, warp, cta);
-  auto tile_of = [&](int64_t unit, int tl) -> int64_t { return unit * 4 + tl * 2 + (int64_t)cta; };
+  const ChainWalk<FwdProg> walk((M + kTileM - 1) / kTileM);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int h = (warp - 2) >> 2, r = (warp & 3) * 32 + lane;   // compute warps: row r, column half h
+  ChainHandshake<kStore> hk;
+  float p[3];   // the sample of the slot's next tile: fetched early, encoded by the prologue
 
-  if (warp == 0) {
-    if (lane == 0) producer_role<Prog>(sm, packed + kFwdPairOff, cta, n_pairs, first, stride);
-  } else if (warp == 1) {
-    if (lane == 0 && cta == 0) mma_role<Prog>(sm, tmem, 0u, ordered != 0, n_pairs, first, stride);
-    else if (lane == 0) relay_role<Prog>(sm, n_pairs, first, stride);   // peer CTA: its warp 1 is otherwise idle
-  } else if (warp == 11) {
-    if (lane == 0 && cta == 0) mma_role<Prog>(sm, tmem, 1u, ordered != 0, n_pairs, first, stride);
-  } else if (warp == 10) {
-    // ============== record store (training): the operand tiles h0..h7 -> HBM, bulk copies ======================
-    if constexpr (TRAIN && !REC8) {
-      if (lane == 0) {
-        store_role(sm, 8, n_tiles, n_pairs, first, stride, tile_of,
-                   [&](int item, int64_t tile) { return rec + tile * kRecBytes + kRecH0 + item * kHSBytes; },
-                   [](int) { return (uint32_t)kHSBytes; });
+  auto prologue = [&](int64_t pair, int tl, bool first) {
+    const int64_t tile = walk.tile_of(pair, tl);
+    if (first) load_sample(p, o, d, t, tile * kTileM + r, M, S);
+    pe_xyz<REC8>(sm.xs[tl], (TRAIN && tile < walk.n_tiles) ? rec + tile * kRB + kOffXS : nullptr, r, h, p[0], p[1], p[2]);
+    hk.arrive(sm, tl, lane, false);
+  };
+  auto epilogue = [&](int64_t pair, int s, int tl, auto acc) {
+    const int64_t tile = walk.tile_of(pair, tl);
+    const int64_t g = tile * kTileM + r;
+    const bool valid = g < M;
+    const bool save = TRAIN && tile < walk.n_tiles;
+    uint8_t* rec_t = rec + tile * kRB;
+    const uint32_t tacc = acc();
+    if (s < kLast) {
+      // hidden layers: 128 of the 256 columns per thread
+      float dirv[3];
+      if (s == 5) load_dir(dirv, d, g, M, S);   // fetched now, used after the epilogue: the L2 latency hides behind it
+      hk.wait_writable(sm, tl);
+      epi_hidden<TRAIN, REC8>(tacc, sm.hs[tl], h, r, save ? rec_t + kOffMask + s * kMaskLayerBytes : nullptr,
+                              (REC8 && save) ? rec_t + kRec8H0 + s * kH8Bytes : nullptr);
+      if (s == 5) {
+        // xs[tl] is dead after layer 5 (skip concat consumed): it now carries PE(dir) for the last step
+        pe_dir<REC8>(sm.xs[tl], save ? rec_t + kOffDS : nullptr, r, h, dirv[0], dirv[1], dirv[2]);
+      }
+      hk.arrive(sm, tl, lane, true);
+    } else {
+      // columns 0..2 (+ 4..6): the rgb pre-activations, 3 (+ 7): sigma's (heads folded into the step, biases
+      // included; mlp.py:40, 43-48).  One half-row thread per row finishes it; the other starts the next tile.
+      const int64_t next = pair + walk.stride;   // the next tile of this slot: fetch its sample now, encode it afterwards
+      if (next < walk.n_pairs) load_sample(p, o, d, t, walk.tile_of(next, tl) * kTileM + r, M, S);
+      if (h == 0) {   // warp-uniform
+        float a[8];
+        tmem_ld8(tacc, a);
+        const float z[4] = {a[0] + a[4], a[1] + a[5], a[2] + a[6], a[3] + a[7]};
+        if (valid)
+          rgbsigma[g] = make_float4(1.f / (1.f + expf(-z[0])), 1.f / (1.f + expf(-z[1])), 1.f / (1.f + expf(-z[2])),
+                                    fmaxf(z[3], 0.f));
       }
     }
-  } else {
-    // =========================== compute warps ==========================
-    const int q = warp & 3, h = (warp - 2) >> 2;
-    const int r = q * 32 + lane;
-    const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    uint32_t acc_par[2] = {0, 0};
-
-    ChainHandshake<TRAIN && !REC8> hk;
-    auto prologue = [&](int64_t pair, int tl, const float (&p)[3]) {
-      const int64_t tile = tile_of(pair, tl);
-      pe_xyz<REC8>(sm.xs[tl], (TRAIN && tile < n_tiles) ? rec + tile * kRB + kOffXS : nullptr, r, h, p[0], p[1], p[2]);
-      hk.arrive(sm, tl, lane, false);
-    };
-
-    KN_PROF_DECL();
-    KN_PROF_BEGIN(t_c);
-    if (first < n_pairs) {
-#pragma unroll 1
-      for (int tl = 0; tl < 2; ++tl) {
-        float p0[3];
-        load_sample(p0, o, d, t, tile_of(first, tl) * kTileM + r, M, S);
-        prologue(first, tl, p0);
-      }
-    }
-    for (int64_t pair = first; pair < n_pairs; pair += stride) {
-      for (int s = 0; s < Prog::kSteps; ++s) {
-#pragma unroll 1
-        for (int tl = 0; tl < 2; ++tl) {
-          const int64_t tile = tile_of(pair, tl);
-          const int64_t g = tile * kTileM + r;
-          const bool valid = g < M;
-          const bool save = TRAIN && tile < n_tiles;
-          uint8_t* rec_t = rec + tile * kRB;
-          KN_PROF_BEGIN(t_w);
-          mbar_wait_cluster(&sm.acc_ready[tl], acc_par[tl]);
-          KN_PROF_END(t_w, 4);
-          KN_PROF_BEGIN(t_e);
-          acc_par[tl] ^= 1;
-          tc_fence_after();
-
-          if (s < kLast) {
-            // hidden layers: 128 of the 256 columns per thread
-            float dirv[3];
-            if (s == 5) load_dir(dirv, d, g, M, S);   // fetched now, used after the epilogue: the L2 latency hides behind it
-            hk.wait_writable(sm, tl);
-            epi_hidden<TRAIN, REC8>(tmem + lane_base + tl * 256, sm.hs[tl], h, r,
-                                    save ? rec_t + kOffMask + s * kMaskLayerBytes : nullptr,
-                                    (REC8 && save) ? rec_t + kRec8H0 + s * kH8Bytes : nullptr);
-            if (s == 5) {
-              // xs[tl] is dead after layer 5 (skip concat consumed): it now carries PE(dir) for the last step
-              pe_dir<REC8>(sm.xs[tl], save ? rec_t + kOffDS : nullptr, r, h, dirv[0], dirv[1], dirv[2]);
-            }
-            hk.arrive(sm, tl, lane, true);
-          } else {
-            // columns 0..2 (+ 4..6): the rgb pre-activations, 3 (+ 7): sigma's (heads folded into the step, biases
-            // included; mlp.py:40, 43-48).  One half-row thread per row finishes it; the other starts the next tile.
-            const int64_t next = pair + stride;
-            float nin[3] = {0.f, 0.f, 0.f};   // the next tile of this slot: fetch its sample now, encode it afterwards
-            if (next < n_pairs) load_sample(nin, o, d, t, tile_of(next, tl) * kTileM + r, M, S);
-            if (h == 0) {   // warp-uniform
-              float a[8];
-              tmem_ld8(tmem + lane_base + tl * 256, a);
-              const float z[4] = {a[0] + a[4], a[1] + a[5], a[2] + a[6], a[3] + a[7]};
-              if (valid)
-                rgbsigma[g] = make_float4(1.f / (1.f + expf(-z[0])), 1.f / (1.f + expf(-z[1])), 1.f / (1.f + expf(-z[2])),
-                                          fmaxf(z[3], 0.f));
-            }
-            tc_fence_before();
-            // this tile is finished: start the next pair's tile in the same slot right away
-            if (next < n_pairs) prologue(next, tl, nin);
-          }
-          KN_PROF_END(t_e, 6 + tl * 16 + s);
-        }
-      }
-    }
-    KN_PROF_END(t_c, 5);
-    if (tid == 64) { KN_PROF_FLUSH(); }
-  }
-  chain_teardown(tmem, warp);
+  };
+  // inference: the step loop fully unrolled, so that every epilogue branch on s resolves at compile time; the training
+  // variants, with the record stores in their epilogues, keep one copy of the loop body (instruction cache)
+  chain_body<kStore, TRAIN ? 1 : FwdProg::kSteps>(sm, walk, packed + kFwdPairOff, ordered != 0, prologue, epilogue,
+                     [&](int item, int64_t tile) { return rec + tile * kRecBytes + kRecH0 + item * kHSBytes; },
+                     [](int) { return (uint32_t)kHSBytes; });
 }
 
 }  // namespace

@@ -98,133 +98,81 @@ tc_mlp_dgrad_kernel(const uint8_t* __restrict__ packed, const float4* __restrict
                     float* __restrict__ xbuf) {
   constexpr int kRB = REC8 ? kRec8Bytes : kRecBytes, kOffMask = REC8 ? kRec8Mask : kRecMask,
                 kDB = REC8 ? kDz8Bytes : kDzBytes;
+  constexpr bool kStore = !REC8;   // every A operand of the chain is also a dZ record (fp8 records leave from the
+                                   // epilogue's registers)
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   ChainSmem& sm = *reinterpret_cast<ChainSmem*>(smem_raw);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int64_t n_tiles = (M + kTileM - 1) / kTileM;
-  const int64_t n_pairs = (n_tiles + 3) / 4;   // work units: four tiles per CTA pair
-  const uint32_t cta = cluster_ctarank();
-  const int64_t first = blockIdx.x >> 1, stride = gridDim.x >> 1;
-  const uint32_t tmem = chain_setup(sm, tid, warp, cta);
-  auto tile_of = [&](int64_t unit, int tl) -> int64_t { return unit * 4 + tl * 2 + (int64_t)cta; };
+  const ChainWalk<BwdProg> walk((M + kTileM - 1) / kTileM);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int h = (warp - 2) >> 2, r = (warp & 3) * 32 + lane;   // compute warps: row r, column half h
+  ChainHandshake<kStore> hk;
+  // fp8 records: one power-of-two scale per call, from max|d_pre| (written by dpre_amax_kernel before this launch)
+  const float scale = REC8 ? dz8_scale(__ldg(reinterpret_cast<const uint32_t*>(xbuf) + kXOffAmax), false) : 1.f;
 
-  if (warp == 0) {
-    if (lane == 0) producer_role<BwdProg>(sm, packed + kBwdPairOff, cta, n_pairs, first, stride);
-  } else if (warp == 1) {
-    if (lane == 0 && cta == 0) mma_role<BwdProg>(sm, tmem, 0u, true, n_pairs, first, stride);
-    else if (lane == 0) relay_role<BwdProg>(sm, n_pairs, first, stride);
-  } else if (warp == 11) {
-    if (lane == 0 && cta == 0) mma_role<BwdProg>(sm, tmem, 1u, true, n_pairs, first, stride);
-  } else if (warp == 10) {
-    // record store: the A operands dZ7..dZ1 of the chain (items 1..7) are also the dZ records of the weight-gradient
-    // kernel (tc_roles.cuh store_role); item 0 = (d rgb_pre, d sigma_pre) only takes part in the hand-shake: the
-    // prologue writes its record (kDzP)
-    if (!REC8 && lane == 0) {   // (fp8 records leave from the epilogue's registers)
-      store_role(sm, 8, n_tiles, n_pairs, first, stride, tile_of,
-                 [&](int item, int64_t tile) {
-                   return dz + tile * kDzBytes + (item == 0 ? kDzG : kDzZ0 + (8 - item) * kHSBytes);
-                 },
-                 [](int item) { return (uint32_t)(item == 0 ? 0 : kHSBytes); });   // dG stays on chip (item 0)
-    }
-  } else {
-    ChainHandshake<!REC8> hk;   // (every A operand of the chain is also a dZ record)
-    const int q = warp & 3, h = (warp - 2) >> 2;
-    const int r = q * 32 + lane;
-    const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-    uint32_t acc_par[2] = {0, 0};
-    // fp8 records: one power-of-two scale per call, from max|d_pre| (written by dpre_amax_kernel before this launch)
-    const float scale = REC8 ? dz8_scale(__ldg(reinterpret_cast<const uint32_t*>(xbuf) + kXOffAmax), false) : 1.f;
-
-    KN_PROF_DECL();
-    // tile start: (d rgb_pre, d sigma_pre, 0 ...) is the first A operand (K = 32, tc_layout.cuh BwdProg)
-    auto prologue = [&](int64_t pair, int tl) {
-      KN_PROF_BEGIN(t_p);
-      const int64_t tile = tile_of(pair, tl);
-      const int64_t g = tile * kTileM + r;
-      const bool active = tile < n_tiles;
-      float4 dp = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (g < M) dp = d_pre[g];
-      // fp8 records: the whole chain runs on gradients times the record scale (a power of two: the same mantissas, so
-      // every dZ is the same number times 2^k), and the e5m2 records need no multiply in the epilogues
-      const float4 dq = REC8 ? make_float4(dp.x * scale, dp.y * scale, dp.z * scale, dp.w * scale) : dp;
-      uint8_t* dz_t = dz + tile * kDB;
-      const uint4 pk = (h == 0) ? make_uint4(pack_bf16x2(dq.x, dq.y), pack_bf16x2(dq.z, dq.w), 0u, 0u)
-                                : make_uint4(0u, 0u, 0u, 0u);
-      if (active && !REC8) *reinterpret_cast<uint4*>(dz_t + kDzP + h * kChunkA + r * 16) = pk;   // (dq = dp here)
-      if (active && REC8 && h == 0)   // one 16-column chunk: (d rgb_pre, d sigma_pre) * scale, then zeros
-        *reinterpret_cast<uint4*>(dz_t + kDz8P + r * 16) =
-            make_uint4(pack_e5m2x4(dq.x, dq.y, dq.z, dq.w), 0u, 0u, 0u);
-      if (h == 0) {   // bias gradients of the two heads: db_rgb = sum d(rgb_pre), db_sigma = sum d(sigma_pre)
-        const float s0 = warp_sum(dp.x), s1 = warp_sum(dp.y), s2 = warp_sum(dp.z), s3 = warp_sum(dp.w);
-        // sum d(rgb_pre) of THIS call for tc_finish_kernel, over the values the weight-gradient kernel's heads task
-        // multiplies: the fp32 d_pre with fp8 records, the bf16 operand (kDzP) with bf16 records (dq = dp there)
-        const float r0 = REC8 ? s0 : warp_sum(bf16_lo(pk.x)), r1 = REC8 ? s1 : warp_sum(bf16_hi(pk.x)),
-                    r2 = REC8 ? s2 : warp_sum(bf16_lo(pk.y));
-        if (lane == 0) {
-          atomicAdd(grads + P.b_off[11], s0); atomicAdd(grads + P.b_off[11] + 1, s1);
-          atomicAdd(grads + P.b_off[11] + 2, s2); atomicAdd(grads + P.b_off[8], s3);
-          atomicAdd(xbuf + kXOffS, r0); atomicAdd(xbuf + kXOffS + 1, r1); atomicAdd(xbuf + kXOffS + 2, r2);
-        }
-      }
-      hk.wait_writable(sm, tl);
-      // chunk 0 of the row (h = 0), zeros in chunk 1 (h = 0) and chunks 2, 3 (h = 1): the step reads K = 32, and a
-      // stale NaN pattern times a zero weight would not be zero
-      *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h) * kChunkA + r * 16) = pk;
-      *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h + 1) * kChunkA + r * 16) = make_uint4(0u, 0u, 0u, 0u);
-      hk.arrive(sm, tl, lane, true);
-      KN_PROF_END(t_p, 15 + tl * 16);
-    };
-
-    KN_PROF_BEGIN(t_c);
-    if (first < n_pairs) {
-#pragma unroll 1
-      for (int tl = 0; tl < 2; ++tl) prologue(first, tl);
-    }
-    for (int64_t pair = first; pair < n_pairs; pair += stride) {
-      for (int b = 0; b < BwdProg::kSteps; ++b) {
-        const int zi = 7 - b;                                  // index of the dZ this step produces
-#pragma unroll 1
-        for (int tl = 0; tl < 2; ++tl) {
-          const int64_t tile = tile_of(pair, tl);
-          const bool active = tile < n_tiles;
-          uint8_t* out = REC8 ? dz + tile * kDB + kDz8Z0 + zi * kH8Bytes : dz + tile * kDB + kDzZ0 + zi * kHSBytes;
-          const uint8_t* mask = rec + tile * kRB + kOffMask + zi * kMaskLayerBytes;
-          // the ReLU' bits (written by the forward, 1 bit per activation) do not depend on the accumulator: fetch
-          // this thread's 4 x 32 columns BEFORE waiting for the MMA so that the latency overlaps it
-          uint32_t mb[4] = {0u, 0u, 0u, 0u};
-          if (active) {
-            const uint4 mv = __ldg(reinterpret_cast<const uint4*>(mask + h * 2048 + r * 16));
-            mb[0] = mv.x; mb[1] = mv.y; mb[2] = mv.z; mb[3] = mv.w;
-          }
-          KN_PROF_BEGIN(t_w);
-          mbar_wait_cluster(&sm.acc_ready[tl], acc_par[tl]);
-          KN_PROF_END(t_w, 4);
-          KN_PROF_BEGIN(t_e);
-          acc_par[tl] ^= 1;
-          tc_fence_after();
-          if (b + 1 < BwdProg::kSteps) hk.wait_writable(sm, tl);
-          const uint32_t tacc = tmem + lane_base + tl * 256;
-          const uint4 mbv = make_uint4(mb[0], mb[1], mb[2], mb[3]);
-          uint8_t* out8 = (REC8 && active) ? out : nullptr;
-          if (b + 1 < BwdProg::kSteps) epi_dgrad<2, REC8>(tacc, sm.hs[tl], h, r, mbv, out8);
-          else epi_dgrad<3, REC8>(tacc, active ? out : nullptr, h, r, mbv, out8);
-          if (b + 1 < BwdProg::kSteps) {
-            hk.arrive(sm, tl, lane, true);
-            KN_PROF_END(t_e, 6 + tl * 16 + b);
-          } else {
-            tc_fence_before();
-            KN_PROF_END(t_e, 6 + tl * 16 + b);
-            // (bias gradients = column sums of the dZ tiles are taken by tc_wgrad_kernel, which has them in smem)
-            const int64_t next = pair + stride;
-            if (next < n_pairs) prologue(next, tl);
-          }
-        }
+  // tile start: (d rgb_pre, d sigma_pre, 0 ...) is the first A operand (K = 32, tc_layout.cuh BwdProg)
+  auto prologue = [&](int64_t pair, int tl, bool) {
+    const int64_t tile = walk.tile_of(pair, tl);
+    const int64_t g = tile * kTileM + r;
+    const bool active = tile < walk.n_tiles;
+    float4 dp = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (g < M) dp = d_pre[g];
+    // fp8 records: the whole chain runs on gradients times the record scale (a power of two: the same mantissas, so
+    // every dZ is the same number times 2^k), and the e5m2 records need no multiply in the epilogues
+    const float4 dq = REC8 ? make_float4(dp.x * scale, dp.y * scale, dp.z * scale, dp.w * scale) : dp;
+    uint8_t* dz_t = dz + tile * kDB;
+    const uint4 pk = (h == 0) ? make_uint4(pack_bf16x2(dq.x, dq.y), pack_bf16x2(dq.z, dq.w), 0u, 0u)
+                              : make_uint4(0u, 0u, 0u, 0u);
+    if (active && !REC8) *reinterpret_cast<uint4*>(dz_t + kDzP + h * kChunkA + r * 16) = pk;   // (dq = dp here)
+    if (active && REC8 && h == 0)   // one 16-column chunk: (d rgb_pre, d sigma_pre) * scale, then zeros
+      *reinterpret_cast<uint4*>(dz_t + kDz8P + r * 16) = make_uint4(pack_e5m2x4(dq.x, dq.y, dq.z, dq.w), 0u, 0u, 0u);
+    if (h == 0) {   // bias gradients of the two heads: db_rgb = sum d(rgb_pre), db_sigma = sum d(sigma_pre)
+      const float s0 = warp_sum(dp.x), s1 = warp_sum(dp.y), s2 = warp_sum(dp.z), s3 = warp_sum(dp.w);
+      // sum d(rgb_pre) of THIS call for tc_finish_kernel, over the values the weight-gradient kernel's heads task
+      // multiplies: the fp32 d_pre with fp8 records, the bf16 operand (kDzP) with bf16 records (dq = dp there)
+      const float r0 = REC8 ? s0 : warp_sum(bf16_lo(pk.x)), r1 = REC8 ? s1 : warp_sum(bf16_hi(pk.x)),
+                  r2 = REC8 ? s2 : warp_sum(bf16_lo(pk.y));
+      if (lane == 0) {
+        atomicAdd(grads + P.b_off[11], s0); atomicAdd(grads + P.b_off[11] + 1, s1);
+        atomicAdd(grads + P.b_off[11] + 2, s2); atomicAdd(grads + P.b_off[8], s3);
+        atomicAdd(xbuf + kXOffS, r0); atomicAdd(xbuf + kXOffS + 1, r1); atomicAdd(xbuf + kXOffS + 2, r2);
       }
     }
-    KN_PROF_END(t_c, 5);
-    if (tid == 64) { KN_PROF_FLUSH(); }
-  }
-  chain_teardown(tmem, warp);
+    hk.wait_writable(sm, tl);
+    // chunk 0 of the row (h = 0), zeros in chunk 1 (h = 0) and chunks 2, 3 (h = 1): the step reads K = 32, and a
+    // stale NaN pattern times a zero weight would not be zero
+    *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h) * kChunkA + r * 16) = pk;
+    *reinterpret_cast<uint4*>(sm.hs[tl] + (2 * h + 1) * kChunkA + r * 16) = make_uint4(0u, 0u, 0u, 0u);
+    hk.arrive(sm, tl, lane, true);
+  };
+  // (bias gradients = column sums of the dZ tiles are taken by tc_wgrad_kernel, which has them in smem)
+  auto epilogue = [&](int64_t pair, int b, int tl, auto acc) {
+    const int zi = 7 - b;                                  // index of the dZ this step produces
+    const int64_t tile = walk.tile_of(pair, tl);
+    const bool active = tile < walk.n_tiles;
+    uint8_t* out = REC8 ? dz + tile * kDB + kDz8Z0 + zi * kH8Bytes : dz + tile * kDB + kDzZ0 + zi * kHSBytes;
+    const uint8_t* mask = rec + tile * kRB + kOffMask + zi * kMaskLayerBytes;
+    // the ReLU' bits (written by the forward, 1 bit per activation) do not depend on the accumulator: fetch this
+    // thread's 4 x 32 columns BEFORE waiting for the MMA so that the latency overlaps it
+    uint32_t mb[4] = {0u, 0u, 0u, 0u};
+    if (active) {
+      const uint4 mv = __ldg(reinterpret_cast<const uint4*>(mask + h * 2048 + r * 16));
+      mb[0] = mv.x; mb[1] = mv.y; mb[2] = mv.z; mb[3] = mv.w;
+    }
+    const uint32_t tacc = acc();
+    if (b + 1 < BwdProg::kSteps) hk.wait_writable(sm, tl);
+    const uint4 mbv = make_uint4(mb[0], mb[1], mb[2], mb[3]);
+    uint8_t* out8 = (REC8 && active) ? out : nullptr;
+    if (b + 1 < BwdProg::kSteps) epi_dgrad<2, REC8>(tacc, sm.hs[tl], h, r, mbv, out8);
+    else epi_dgrad<3, REC8>(tacc, active ? out : nullptr, h, r, mbv, out8);
+    if (b + 1 < BwdProg::kSteps) hk.arrive(sm, tl, lane, true);
+  };
+  // record store: the A operands of the chain are also the dZ records of the weight-gradient kernel; item 0 =
+  // (d rgb_pre, d sigma_pre) only takes part in the hand-shake: the prologue writes its record (kDzP)
+  chain_body<kStore, 1>(sm, walk, packed + kBwdPairOff, true, prologue, epilogue,
+                     [&](int item, int64_t tile) {
+                       return dz + tile * kDzBytes + (item == 0 ? kDzG : kDzZ0 + (8 - item) * kHSBytes);
+                     },
+                     [](int item) { return (uint32_t)(item == 0 ? 0 : kHSBytes); });   // dG stays on chip (item 0)
 }
 
 // =============================================================================================================
